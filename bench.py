@@ -6,10 +6,14 @@ the current mask (README.md:54-68 loop; device counter RNG) and apply Env.step()
 Env._get_mask() to all B resident envs, auto-reset on done.  Workloads are BASELINE.json's
 configs; the default is configs[1] (LongestPath-v0 N=50 E=200 parenting=2, 65,536 envs per GPU).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 `--impl reference` times the CPU implementation of the same path (the C restatement of the
 reference in oracle/, OpenMP over envs, all host threads) on a bounded sample of the workload.
+
+`--dump-outputs DIR` writes what the last timed step of the headline workload returned to its caller
+(step_outputs) as DIR/<name>.npy; instances and actions are seeded, so two builds run with the same
+arguments can be compared array for array.
 """
 import argparse
 import json
@@ -160,6 +164,30 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["no samples"]}
         return {"sm_mhz": float(np.median(sm)), "sm_max_mhz": float(max(mx)), "reasons": sorted(reasons),
                 "samples": len(sm), "power_w_max": float(max(pw))}
+
+
+DUMP_BYTES = 63_000_000      # array bytes of --dump-outputs: with the .npy headers the files stay under 64 MB
+
+
+def step_outputs(env, budget=DUMP_BYTES):
+    """What a caller of the timed step (ge_step_sampled) receives for every env, as float arrays: the action drawn, reward,
+    the four flag fields, solution_cost and the packed valid-action mask expanded to [envs, A].  A batch whose arrays would
+    exceed `budget` bytes is cut to a fixed, seeded sample of envs; env_index says which."""
+    import torch
+    B, A = env.B, env.desc.A
+    per_env = 8 + 8 + 4 + 4 * 4 + 8 + 4 * A
+    idx = np.arange(B)
+    if B * per_env > budget:
+        idx = np.sort(np.random.default_rng(0).choice(B, budget // per_env, replace=False))
+    ti = torch.as_tensor(idx, device=env.reward.device)
+    flags = env.flags[ti].cpu().numpy()
+    bits = env.t["mask_bits"][ti].cpu().numpy()
+    mask = np.unpackbits(bits.view(np.uint8), axis=1, bitorder="little")[:, :A]
+    return {"env_index": idx.astype(np.float64), "action": env.actions_dev[ti].cpu().numpy().astype(np.float64),
+            "reward": env.reward[ti].cpu().numpy().astype(np.float32), "done": flags[:, 0].astype(np.float32),
+            "solved": flags[:, 1].view(np.int8).astype(np.float32), "status": flags[:, 2].astype(np.float32),
+            "has_mask": flags[:, 3].astype(np.float32), "solution_cost": env.solution_cost[ti].cpu().numpy().astype(np.float64),
+            "mask": mask.astype(np.float32)}
 
 
 def host_policy(rng, mask):
@@ -324,13 +352,14 @@ STREAM_CHUNKS = {"cfg2_longest_path": 8, "cfg1_shortest_path": 8, "perishable": 
                  "cfg5_multicast": 2, "cfg5_distcenter": 2}   # (profiles/r02_stream_sweep.jsonl)
 
 
-def measure_streaming(D, flush, wl, B, K, W, env, env0, args, per_launch_bytes):
+def measure_streaming(D, flush, wl, B, K, W, env, env0, args, per_launch_bytes, dump=False):
     """Streaming protocol: EXACTLY K steps inside ONE timed region (one CUDA event pair, barrier + synchronize on both sides),
     no flush kernels in it.  The steps rotate over R independent resident batches of B envs whose per-step traffic adds up to
     > 3x L2 (inputs larger than L2: every step finds its batch cold); a workload whose single batch already moves more than
     that per step uses R = 1.  One step of a batch = C sub-batch launches on C free-running stream chains (envs are
     independent: step t+1 of an env only has to follow step t of the same env), launched with GE_FLAG_PDL.
-    Returns None when the R batches do not fit in memory (then only the isolated protocol is reported)."""
+    Returns None when the R batches do not fit in memory (then only the isolated protocol is reported).
+    dump: also return step_outputs() of the batch that took the last timed step."""
     import torch
     from graphenvs_b200 import BatchedGraphEnv
     from graphenvs_b200.batch import SliceStreams
@@ -397,20 +426,22 @@ def measure_streaming(D, flush, wl, B, K, W, env, env0, args, per_launch_bytes):
     w1 = time.time()
     ms = a.elapsed_time(b)
     total_ms_max = D.reduce([ms], "max")[0]
+    outputs = step_outputs(envs[(K - 1) % R]) if dump else None
     for e in envs:
         e.enable_pdl(False)
     n_launch = K * (len(sl[0].bounds) if sl else 1)
     del graph, tail, sl, envs
     torch.cuda.empty_cache()
     return {"total_ms": total_ms_max, "ms_per_step": total_ms_max / K, "steps": K, "replicas": R, "chunks": C_, "pdl": not args.no_pdl,
-            "gpu_launches": n_launch, "wall": (w0, w1), "rotation_bytes": per_launch_bytes * R,
+            "gpu_launches": n_launch, "wall": (w0, w1), "rotation_bytes": per_launch_bytes * R, "outputs": outputs,
             "launch": "CUDA graph of %d steps replayed %d times%s, ONE event pair around all %d steps; step i runs on batch i %% %d; "
                       "each step = %d sub-batch launch(es) on %d stream chain(s)%s" % (G, q, (" + one graph of %d steps" % r) if r else "", K, R, C_, C_, ", programmatic dependent launch" if not args.no_pdl else "")}
 
 
-def measure_workload(D, flush, wl, B, K, W, args, host_side_policy, envs_total_note=None, sampler=None, seed_env0=None):
+def measure_workload(D, flush, wl, B, K, W, args, host_side_policy, envs_total_note=None, sampler=None, seed_env0=None, dump=False):
     """One workload on this rank's B envs: device-timed env-steps/s (value), the end-to-end C-ABI number (e2e), the
-    roofline of the step kernel, reset-time costs.  Every rank calls it with the same arguments (barriers inside)."""
+    roofline of the step kernel, reset-time costs.  Every rank calls it with the same arguments (barriers inside).
+    dump: the result also carries "outputs", step_outputs() of the last timed step of the protocol that gives `value`."""
     import torch
     from graphenvs_b200 import BatchedGraphEnv
     env_id, N, E, kw, _, survey_bytes, desc = WORKLOADS[wl]
@@ -486,6 +517,7 @@ def measure_workload(D, flush, wl, B, K, W, args, host_side_policy, envs_total_n
         kern_ms += [e[0 if fused else 1].elapsed_time(e[2]) for e in events]
     D.barrier()
     w1 = time.time()
+    outputs = step_outputs(env) if dump else None    # before the streaming protocol steps this batch further
     step_ms, kern_ms = np.array(step_ms), np.array(kern_ms)
     assert step_ms.size == K
     total_ms_max, kern_ms_mean = D.reduce([float(step_ms.sum()), float(kern_ms.mean())], "max")
@@ -507,7 +539,7 @@ def measure_workload(D, flush, wl, B, K, W, args, host_side_policy, envs_total_n
     stream = None
     if fused and not args.no_streaming:
         try:
-            stream = measure_streaming(D, flush, wl, B, K, W, env, env0, args, per_launch)
+            stream = measure_streaming(D, flush, wl, B, K, W, env, env0, args, per_launch, dump=dump)
         except torch.cuda.OutOfMemoryError:       # the R batches did not fit after all: the isolated protocol stands alone
             stream = None
             torch.cuda.empty_cache()
@@ -516,6 +548,7 @@ def measure_workload(D, flush, wl, B, K, W, args, host_side_policy, envs_total_n
     clocks = sampler.stop(w0, stream["wall"][1] if stream else w1) if sampler is not None else None
     if stream:
         value, ms_per_step, kern_ms_mean, launch_mode, n_launches = envs_all * K / (stream["total_ms"] * 1e-3), stream["ms_per_step"], stream["ms_per_step"], stream["launch"], stream["gpu_launches"]
+        outputs = stream["outputs"]
     else:
         value, ms_per_step, n_launches = iso_value, total_ms_max / K, isolated["gpu_launches"]
 
@@ -682,6 +715,8 @@ def measure_workload(D, flush, wl, B, K, W, args, host_side_policy, envs_total_n
         "episodes": float(stats[0]), "solved": float(stats[1]),
         "memory_gb_per_gpu": mem / 1e9,
     }
+    if dump:
+        res["outputs"] = outputs
     return res
 
 
@@ -798,7 +833,12 @@ def run_ours(args):
     flush = L2Flush(torch, D.dev, args.flush)
     sampler = ClockSampler(D.local) if rank == 0 else None
     t_all = time.time()
-    head = measure_workload(D, flush, wl, B, K, W, args, host_side_policy=not args.e2e_device_policy, sampler=sampler)
+    head = measure_workload(D, flush, wl, B, K, W, args, host_side_policy=not args.e2e_device_policy, sampler=sampler,
+                            dump=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:      # rank 0's envs
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in head.pop("outputs").items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if world == 1 and not args.no_cpu:
         head["cpu_baseline"] = cpu_rate(wl, args.cpu_seconds)
     head["cpu_reference_python"] = python_reference_entry(wl)
@@ -907,6 +947,9 @@ def main():
     ap.add_argument("--stream-chunks", type=int, default=0, help="sub-batch chains per step in the streaming protocol (0 = per-workload table)")
     ap.add_argument("--mode", default="fused", choices=["fused", "split"],
                     help="fused: ge_step_sampled (one launch per step); split: ge_sample_actions + ge_step")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline workload returned (step_outputs: float32 / float64, "
+                         "at most 64 MB, a seeded sample of envs beyond that) as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -8,6 +8,8 @@ import sys
 import types
 
 import numpy as np
+import pytest
+import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -61,6 +63,62 @@ def test_host_policy_picks_valid_actions():
     a = bench.host_policy(rng, mask)
     assert a.dtype == np.int32 and mask[np.arange(500), a].all()
     assert len(np.unique(a)) > 5
+
+
+def _fake_stepped_env(B, A, seed=0):
+    rng = np.random.default_rng(seed)
+    mask = rng.random((B, A)) < 0.3
+    AW = (A + 31) // 32
+    bits = np.packbits(np.pad(mask, ((0, 0), (0, 32 * AW - A))), axis=1, bitorder="little").view(np.int32)
+    flags = np.stack([rng.integers(0, 2, B), rng.integers(-1, 2, B) & 0xFF, rng.integers(0, 2, B), rng.integers(0, 2, B)], 1)
+    env = types.SimpleNamespace(B=B, desc=types.SimpleNamespace(A=A), t={"mask_bits": torch.from_numpy(bits)},
+                                flags=torch.from_numpy(flags.astype(np.uint8)), reward=torch.from_numpy(rng.random(B, dtype=np.float32)),
+                                solution_cost=torch.from_numpy(rng.random(B)), actions_dev=torch.from_numpy(rng.integers(0, A, B, dtype=np.int32)))
+    return env, mask, flags
+
+
+def test_step_outputs_are_float_arrays_of_what_the_caller_receives():
+    env, mask, flags = _fake_stepped_env(100, 40)
+    out = bench.step_outputs(env)
+    assert all(a.dtype in (np.float32, np.float64) and a.shape[0] == 100 for a in out.values())
+    np.testing.assert_array_equal(out["mask"], mask)
+    np.testing.assert_array_equal(out["solved"], flags[:, 1].astype(np.uint8).view(np.int8))
+    np.testing.assert_array_equal(out["action"], env.actions_dev.numpy())
+    np.testing.assert_array_equal(out["solution_cost"], env.solution_cost.numpy())
+    np.testing.assert_array_equal(out["env_index"], np.arange(100))
+
+
+def test_step_outputs_of_a_large_batch_are_a_fixed_sample_within_the_budget():
+    env, mask, _ = _fake_stepped_env(5000, 300)
+    full = bench.step_outputs(env)
+    budget = 200_000
+    out = bench.step_outputs(env, budget=budget)
+    assert 0 < sum(a.nbytes for a in out.values()) <= budget
+    idx = out["env_index"].astype(np.int64)
+    assert len(idx) < 5000 and np.all(np.diff(idx) > 0)
+    for name, a in out.items():
+        np.testing.assert_array_equal(a, full[name][idx])
+    again = bench.step_outputs(env, budget=budget)
+    for name, a in out.items():
+        np.testing.assert_array_equal(a, again[name])
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_identical_from_run_to_run(tmp_path):
+    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--only-headline", "--steps", "7", "--warmup", "3", "--no-cpu",
+           "--e2e-steps", "3", "--no-e2e-obs"]
+    runs = []
+    for name in ("a", "b"):
+        out = subprocess.check_output(cmd + ["--dump-outputs", str(tmp_path / name)]).decode().strip().splitlines()[-1]
+        assert json.loads(out)["steps"] == 7
+        runs.append({f[:-len(".npy")]: np.load(tmp_path / name / f) for f in os.listdir(tmp_path / name)})
+    a, b = runs
+    assert sorted(a) == sorted(("env_index", "action", "reward", "done", "solved", "status", "has_mask", "solution_cost", "mask"))
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= 64_000_000
+    for f in a:
+        assert a[f].dtype in (np.float32, np.float64)
+        np.testing.assert_array_equal(a[f], b[f], err_msg=f)
+    assert a["done"].any() and a["mask"].any()
 
 
 def test_reference_arm_prints_the_contract_line():
