@@ -3,7 +3,8 @@
 Public surface:
   make(id, **kwargs)                 gymnasium-shaped single env (reference ids and kwargs)
   make_batched(id, num_envs, ...)    batched vector env with the same per-env semantics
-  BatchedGraphEnv                    the engine class behind both
+  BatchedGraphEnv                    the engine class behind both (sample_logits: policy-driven action draw)
+  masked_log_prob(logits, mask_bits, actions)   differentiable masked log-prob + entropy for the update (policy.py)
   utils.vectorize_graph / devectorize_graph / get_env_info   (graph_envs/utils.py layout contract)
 """
 from .spec import ENV_SPECS, get_env_info, get_num_features  # noqa: F401
@@ -19,6 +20,9 @@ def __getattr__(attr):  # lazy: keeps `import graphenvs_b200` cheap and torch-fr
     if attr in ("make", "make_batched", "register_with_gymnasium", "registry"):
         from . import registration
         return getattr(registration, attr)
+    if attr == "masked_log_prob":
+        from .policy import masked_log_prob
+        return masked_log_prob
     if attr in ("Instance", "generate_instance"):
         from . import instances
         return getattr(instances, attr)

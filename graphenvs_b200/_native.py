@@ -97,7 +97,10 @@ class StepOut(C.Structure):
 EXPORTS = ["ge_abi_version", "ge_last_error", "ge_fill_layout", "ge_step_smem_bytes", "ge_build_adjacency",
            "ge_prepare", "ge_features", "ge_generate", "ge_generate_fallbacks", "ge_pool_refill", "ge_reset", "ge_step", "ge_step_sampled", "ge_sample_actions", "ge_obs_len",
            "ge_obs_flat", "ge_obs_graph", "ge_obs_nodes", "ge_step_kernel_name", "ge_batch_slice", "ge_step_host", "ge_step_host_pipelined", "ge_step_host_compact", "ge_progress_supported",
-           "ge_step_host_release", "ge_mask_mirror_supported", "ge_mask_bytes_current", "ge_mask_bytes", "ge_stats"]
+           "ge_step_host_release", "ge_mask_mirror_supported", "ge_mask_bytes_current", "ge_mask_bytes", "ge_stats",
+           "ge_sample_logits", "ge_masked_log_prob", "ge_masked_log_prob_backward"]
+
+LOGITS_F32, LOGITS_BF16 = 0, 1   # GE_LOGITS_*
 
 _lib = None
 
@@ -145,6 +148,9 @@ def lib():
     L.ge_mask_mirror_supported.argtypes = [BP]
     L.ge_mask_bytes_current.argtypes = [BP]
     L.ge_mask_bytes.argtypes = [BP, C.c_int, C.c_int, _P]
+    L.ge_sample_logits.argtypes = [BP, _P, C.c_int, C.c_int, C.c_uint64, C.c_uint32, _P, _P, _P, _P]
+    L.ge_masked_log_prob.argtypes = [_P, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P]
+    L.ge_masked_log_prob_backward.argtypes = [_P, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P]
     if L.ge_abi_version() != 3:
         raise NativeError("ABI version mismatch")
     _lib = L

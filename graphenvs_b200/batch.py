@@ -448,6 +448,32 @@ class BatchedGraphEnv:
         _native.check(self.lib.ge_sample_actions(C.byref(self.desc), int(seed), int(t), _ptr(out), self._stream()))
         return out
 
+    def sample_logits(self, logits, seed, t, greedy=False, out=None):
+        """Policy-driven action draw (ge_sample_logits): a categorical over the valid actions of the current packed mask.
+
+        logits: CUDA [B, A] float32 / bfloat16 on this batch's device (made contiguous).  greedy=False draws by Gumbel-max with
+        counter-based noise of (seed, global env id, t + env clock, action); greedy=True takes the argmax (lowest index on
+        ties).  Returns (actions int32[B], log_prob f32[B], entropy f32[B]); actions default to self.actions_dev, `out` =
+        (actions, log_prob, entropy) preallocated tensors.  Follow with step(actions) / step_async(actions).  Empty mask rows
+        give (-1, 0, 0).  The log_prob / entropy equal policy.masked_log_prob's on the same inputs bit for bit."""
+        from .policy import _DTYPES
+        if not isinstance(logits, torch.Tensor) or logits.device != self.device:
+            raise ValueError("sample_logits: logits must be a tensor on %s" % self.device)
+        if logits.dtype not in _DTYPES:
+            raise TypeError("sample_logits: logits must be float32 or bfloat16, got %s" % logits.dtype)
+        if tuple(logits.shape) != (self.B, self.desc.A):
+            raise ValueError("sample_logits: logits shape %s, expected (%d, %d)" % (tuple(logits.shape), self.B, self.desc.A))
+        logits = logits.detach().contiguous()
+        if out is None:
+            acts = self.actions_dev
+            lp = torch.empty((self.B,), dtype=torch.float32, device=self.device)
+            ent = torch.empty((self.B,), dtype=torch.float32, device=self.device)
+        else:
+            acts, lp, ent = out
+        _native.check(self.lib.ge_sample_logits(C.byref(self.desc), _ptr(logits), _DTYPES[logits.dtype], int(bool(greedy)), int(seed),
+                                                int(t), _ptr(acts), _ptr(lp), _ptr(ent), self._stream()))
+        return acts, lp, ent
+
     def host_io(self):
         """Pinned host mirror of the device output block: (block, reward, flags, solution_cost, mask_bits) views."""
         Bp, nbytes = self._io_layout

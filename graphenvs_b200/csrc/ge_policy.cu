@@ -1,0 +1,305 @@
+// ge_policy.cu -- masked categorical over policy logits (sm_100a): ge_sample_logits, ge_masked_log_prob and its backward.
+//
+// One device routine, masked_row(), is the whole reduction: for one row of logits it walks the packed valid-action mask
+// and reads ONLY the logits of set bits.  Lane l of the warp owns actions 32w + l; per nonzero mask word it loads its
+// logit iff its bit is set, so the warp's loads are coalesced and a 32-byte sector without a valid action is never
+// fetched (the frontier masks of Multicast / SteinerTree are sparse).  Mask words are read 32 at a time (one coalesced
+// 128-byte load, then broadcast by shuffle) and zero words are skipped warp-uniformly; U nonzero words are loaded before
+// any of them is accumulated, so their loads overlap.  Per lane it keeps online accumulators over the valid actions:
+//   mx = max l,  se = sum exp(l - mx),  st = sum exp(l - mx) * (l - mx),  and the best (score, index, l),
+// merged across the warp by a shuffle butterfly in a fixed order.  Then lse = mx + log(se) and H = log(se) - st / se
+// (= lse - sum p l without the cancellation of two large terms).  Every kernel calls the same routine with the same
+// arithmetic, so the sampler's log_prob / entropy equal the forward kernel's bit for bit; there are no atomics.
+#include <climits>
+#include <cstdio>
+#include <cuda_bf16.h>
+
+#include "ge_common.cuh"
+
+extern "C" int ge_set_error(int code, const char *fmt, ...);
+
+using namespace ge;
+
+namespace {
+
+constexpr int POL_WPB = 8;  // warps (= rows) per block
+constexpr int POL_U = 4;    // nonzero mask words whose logits are loaded together
+
+enum { MODE_STATS = 0, MODE_GREEDY = 1, MODE_GUMBEL = 2 };
+
+template <int DT>
+__device__ __forceinline__ float load_logit(const void *row, size_t i) {
+    if (DT == GE_LOGITS_BF16) {
+        const unsigned short u = __ldg(reinterpret_cast<const unsigned short *>(row) + i);
+        return __uint_as_float((uint32_t)u << 16);
+    }
+    return __ldg(reinterpret_cast<const float *>(row) + i);
+}
+template <int DT>
+__device__ __forceinline__ void store_grad(void *row, size_t i, float g) {
+    if (DT == GE_LOGITS_BF16) reinterpret_cast<__nv_bfloat16 *>(row)[i] = __float2bfloat16_rn(g);
+    else reinterpret_cast<float *>(row)[i] = g;
+}
+
+// Gumbel noise of action a (include/graphenvs_b200.h, ge_sample_logits): key = per-row 64-bit key.
+__device__ __forceinline__ float gumbel(uint64_t key, int a) {
+    const uint32_t h = mix32(key, (uint32_t)a, 0x85EBCA6Bu);
+    const float u = __fmul_rn((float)(h >> 8) + 0.5f, 5.9604644775390625e-8f);  // ((h >> 8) + 1/2) / 2^24, exact, in (0, 1)
+    return -logf(-logf(u));
+}
+__device__ __forceinline__ uint64_t row_key(uint64_t seed, uint32_t env, uint32_t t) {
+    return ((uint64_t)mix32(seed, env, t) << 32) | (uint64_t)mix32(seed ^ 0xD1B54A32D192ED03ull, env, t);
+}
+
+struct RowStats {
+    float mx, se, st;  // max valid logit, sum exp(l - mx), sum exp(l - mx) * (l - mx); se == 0 <=> no valid action
+    float bs, bl;      // best score and its logit
+    int bi;            // its action (INT_MAX = none)
+};
+
+__device__ __forceinline__ void acc_one(RowStats &r, float l) {
+    if (l > r.mx) {
+        if (r.se > 0.f) {
+            const float dm = __fsub_rn(r.mx, l);  // < 0
+            const float sc = expf(dm);
+            r.st = __fmul_rn(sc, __fmaf_rn(dm, r.se, r.st));
+            r.se = __fmaf_rn(r.se, sc, 1.f);
+        } else {
+            r.se = 1.f; r.st = 0.f;
+        }
+        r.mx = l;
+    } else {
+        const float dl = __fsub_rn(l, r.mx);
+        const float e = expf(dl);
+        r.se = __fadd_rn(r.se, e);
+        r.st = __fmaf_rn(e, dl, r.st);
+    }
+}
+
+__device__ __forceinline__ void merge(RowStats &r, const RowStats &o) {
+    if (o.se > 0.f) {
+        if (r.se > 0.f) {
+            const float M = fmaxf(r.mx, o.mx);
+            const float d1 = __fsub_rn(r.mx, M), d2 = __fsub_rn(o.mx, M);
+            const float a1 = expf(d1), a2 = expf(d2);
+            r.st = __fadd_rn(__fmul_rn(a1, __fmaf_rn(d1, r.se, r.st)), __fmul_rn(a2, __fmaf_rn(d2, o.se, o.st)));
+            r.se = __fadd_rn(__fmul_rn(r.se, a1), __fmul_rn(o.se, a2));
+            r.mx = M;
+        } else {
+            r.mx = o.mx; r.se = o.se; r.st = o.st;
+        }
+    }
+    if (o.bs > r.bs || (o.bs == r.bs && o.bi < r.bi)) { r.bs = o.bs; r.bi = o.bi; r.bl = o.bl; }
+}
+
+// The shared reduction over one row (see the file comment).  Warp-cooperative; the result is warp-uniform.
+template <int DT, int MODE>
+__device__ __forceinline__ RowStats masked_row(const void *row, const uint32_t *__restrict__ mrow, int A, int AW, uint64_t key, int lane) {
+    RowStats r;
+    r.mx = -INFINITY; r.se = 0.f; r.st = 0.f; r.bs = -INFINITY; r.bl = 0.f; r.bi = INT_MAX;
+    for (int w0 = 0; w0 < AW; w0 += 32) {
+        const int wl = w0 + lane;
+        const uint32_t mw = wl < AW ? (__ldg(mrow + wl) & tail_mask(A, wl)) : 0u;   // bits >= A are ignored
+        unsigned nz = __ballot_sync(GE_FULL, mw != 0u);
+        while (nz) {
+            float v[POL_U];
+            int idx[POL_U];
+            bool has[POL_U];
+#pragma unroll
+            for (int k = 0; k < POL_U; ++k) {
+                const int src = nz ? __ffs((int)nz) - 1 : 0;
+                const bool any = nz != 0u;
+                nz &= nz - 1u;
+                const uint32_t word = __shfl_sync(GE_FULL, mw, src);
+                idx[k] = ((w0 + src) << 5) + lane;
+                has[k] = any && ((word >> lane) & 1u);
+                v[k] = has[k] ? load_logit<DT>(row, (size_t)idx[k]) : 0.f;
+            }
+#pragma unroll
+            for (int k = 0; k < POL_U; ++k) {
+                if (!has[k]) continue;
+                acc_one(r, v[k]);
+                if (MODE != MODE_STATS) {
+                    const float s = MODE == MODE_GUMBEL ? __fadd_rn(v[k], gumbel(key, idx[k])) : v[k];
+                    if (s > r.bs) { r.bs = s; r.bi = idx[k]; r.bl = v[k]; }   // strictly greater: a lane visits its actions in order
+                }
+            }
+        }
+    }
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+        RowStats q;
+        q.mx = __shfl_xor_sync(GE_FULL, r.mx, o);
+        q.se = __shfl_xor_sync(GE_FULL, r.se, o);
+        q.st = __shfl_xor_sync(GE_FULL, r.st, o);
+        q.bs = __shfl_xor_sync(GE_FULL, r.bs, o);
+        q.bl = __shfl_xor_sync(GE_FULL, r.bl, o);
+        q.bi = __shfl_xor_sync(GE_FULL, r.bi, o);
+        if (lane & o) { RowStats t = q; merge(t, r); r = t; }   // lower lanes first: the same order on both sides
+        else merge(r, q);
+    }
+    r.mx = __shfl_sync(GE_FULL, r.mx, 0);
+    r.se = __shfl_sync(GE_FULL, r.se, 0);
+    r.st = __shfl_sync(GE_FULL, r.st, 0);
+    r.bl = __shfl_sync(GE_FULL, r.bl, 0);
+    r.bi = __shfl_sync(GE_FULL, r.bi, 0);
+    return r;
+}
+
+__device__ __forceinline__ float row_lse(const RowStats &r) { return r.se > 0.f ? __fadd_rn(r.mx, logf(r.se)) : -INFINITY; }
+__device__ __forceinline__ float row_entropy(const RowStats &r) { return r.se > 0.f ? __fsub_rn(logf(r.se), __fdiv_rn(r.st, r.se)) : 0.f; }
+
+template <int DT, int MODE>
+__global__ void __launch_bounds__(POL_WPB * 32) policy_sample_kernel(ge_batch d, const void *__restrict__ logits, uint64_t seed, uint32_t t,
+                                                                      int32_t *__restrict__ actions, float *__restrict__ log_prob,
+                                                                      float *__restrict__ entropy) {
+    pdl_launch_dependents();   // programmatic dependent launch (ge_common.cuh): nothing is touched before pdl_wait()
+    pdl_wait();
+    const int lane = threadIdx.x & 31;
+    const int b = blockIdx.x * POL_WPB + (threadIdx.x >> 5);
+    if (b >= d.B) return;
+    const size_t esz = DT == GE_LOGITS_BF16 ? 2 : 4;
+    const void *row = reinterpret_cast<const char *>(logits) + (size_t)b * d.A * esz;
+    uint64_t key = 0;
+    if (MODE == MODE_GUMBEL) key = row_key(seed, (uint32_t)(d.env_id0 + b), t + (d.env_steps ? d.env_steps[b] : 0u));
+    const RowStats r = masked_row<DT, MODE>(row, d.mask_bits + (size_t)b * d.AW, d.A, d.AW, key, lane);
+    if (lane == 0) {
+        const bool any = r.se > 0.f;
+        actions[b] = any ? r.bi : -1;
+        if (log_prob) log_prob[b] = any ? __fsub_rn(r.bl, row_lse(r)) : 0.f;
+        if (entropy) entropy[b] = row_entropy(r);
+    }
+}
+
+__device__ __forceinline__ bool valid_action(const uint32_t *mrow, int A, int a) {
+    return a >= 0 && a < A && ((__ldg(mrow + (a >> 5)) >> (a & 31)) & 1u);
+}
+
+template <int DT>
+__global__ void __launch_bounds__(POL_WPB * 32) policy_logprob_kernel(const void *__restrict__ logits, int B, int A, const uint32_t *__restrict__ mask_bits,
+                                                                       const int32_t *__restrict__ actions, float *__restrict__ log_prob,
+                                                                       float *__restrict__ entropy, float *__restrict__ lse) {
+    const int lane = threadIdx.x & 31;
+    const int b = blockIdx.x * POL_WPB + (threadIdx.x >> 5);
+    if (b >= B) return;
+    const int AW = (A + 31) >> 5;
+    const size_t esz = DT == GE_LOGITS_BF16 ? 2 : 4;
+    const void *row = reinterpret_cast<const char *>(logits) + (size_t)b * A * esz;
+    const uint32_t *mrow = mask_bits + (size_t)b * AW;
+    const RowStats r = masked_row<DT, MODE_STATS>(row, mrow, A, AW, 0, lane);
+    if (lane == 0) {
+        const int a = actions[b];
+        const float L = row_lse(r);
+        float lp = 0.f;
+        if (r.se > 0.f) lp = valid_action(mrow, A, a) ? __fsub_rn(load_logit<DT>(row, (size_t)a), L) : -INFINITY;
+        log_prob[b] = lp;
+        entropy[b] = row_entropy(r);
+        lse[b] = L;
+    }
+}
+
+// grad_logits[b, i] = g_lp (1[i = a] - p_i) - g_H p_i (log p_i + H) for valid i, 0 elsewhere; p_i = exp(l_i - lse).
+template <int DT>
+__global__ void __launch_bounds__(POL_WPB * 32) policy_logprob_bwd_kernel(const void *__restrict__ logits, int B, int A, const uint32_t *__restrict__ mask_bits,
+                                                                           const int32_t *__restrict__ actions, const float *__restrict__ lse,
+                                                                           const float *__restrict__ entropy, const float *__restrict__ g_lp,
+                                                                           const float *__restrict__ g_h, void *__restrict__ grad) {
+    const int lane = threadIdx.x & 31;
+    const int b = blockIdx.x * POL_WPB + (threadIdx.x >> 5);
+    if (b >= B) return;
+    const int AW = (A + 31) >> 5;
+    const size_t esz = DT == GE_LOGITS_BF16 ? 2 : 4;
+    const void *row = reinterpret_cast<const char *>(logits) + (size_t)b * A * esz;
+    void *grow = reinterpret_cast<char *>(grad) + (size_t)b * A * esz;
+    const uint32_t *mrow = mask_bits + (size_t)b * AW;
+    const int a0 = actions[b];
+    const int a = valid_action(mrow, A, a0) ? a0 : -1;   // an invalid action contributes no log_prob gradient
+    const float glp = (g_lp && a >= 0) ? g_lp[b] : 0.f;
+    const float gh = g_h ? g_h[b] : 0.f;
+    const float L = lse[b], H = entropy[b];
+    for (int w0 = 0; w0 < AW; w0 += 32) {
+        const int wl = w0 + lane;
+        const uint32_t mw = wl < AW ? (__ldg(mrow + wl) & tail_mask(A, wl)) : 0u;
+        const int nw = min(32, AW - w0);
+#pragma unroll 4
+        for (int k = 0; k < nw; ++k) {
+            const uint32_t word = __shfl_sync(GE_FULL, mw, k);
+            const int i = ((w0 + k) << 5) + lane;
+            if (i >= A) continue;
+            float g = 0.f;
+            if ((word >> lane) & 1u) {
+                const float lp = __fsub_rn(load_logit<DT>(row, (size_t)i), L);
+                const float p = expf(lp);
+                g = __fsub_rn(__fmul_rn(glp, __fsub_rn(i == a ? 1.f : 0.f, p)), __fmul_rn(__fmul_rn(gh, p), __fadd_rn(lp, H)));
+            }
+            store_grad<DT>(grow, (size_t)i, g);
+        }
+    }
+}
+
+int launched(const char *what) {
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? GE_OK : ge_set_error(GE_ERR_CUDA, "%s launch: %s", what, cudaGetErrorString(e));
+}
+
+int check_rows(const char *fn, const void *logits, int dtype, int B, int A, const uint32_t *mask_bits, const int32_t *actions) {
+    if (dtype != GE_LOGITS_F32 && dtype != GE_LOGITS_BF16) return ge_set_error(GE_ERR_ARG, "%s: unknown logits dtype %d", fn, dtype);
+    if (B <= 0 || A <= 0) return ge_set_error(GE_ERR_ARG, "%s: bad shape B=%d A=%d", fn, B, A);
+    if (!logits || !mask_bits || !actions) return ge_set_error(GE_ERR_ARG, "%s: null logits / mask_bits / actions", fn);
+    return GE_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int ge_sample_logits(const ge_batch *d, const void *logits, int dtype, int greedy, uint64_t seed, uint32_t t, int32_t *actions,
+                     float *log_prob, float *entropy, void *stream) {
+    GE_NVTX("ge_sample_logits");
+    if (!d) return ge_set_error(GE_ERR_ARG, "ge_sample_logits: null batch");
+    if (dtype != GE_LOGITS_F32 && dtype != GE_LOGITS_BF16) return ge_set_error(GE_ERR_ARG, "ge_sample_logits: unknown logits dtype %d", dtype);
+    if (d->B <= 0 || d->A <= 0 || d->AW != (d->A + 31) / 32) return ge_set_error(GE_ERR_ARG, "ge_sample_logits: bad shape B=%d A=%d AW=%d (call ge_fill_layout)", d->B, d->A, d->AW);
+    if (!logits || !actions || !d->mask_bits) return ge_set_error(GE_ERR_ARG, "ge_sample_logits: null logits / actions / mask_bits");
+    const dim3 grid((d->B + POL_WPB - 1) / POL_WPB), block(POL_WPB * 32);
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e;
+    if (dtype == GE_LOGITS_BF16)
+        e = greedy ? ge_launch_step(policy_sample_kernel<GE_LOGITS_BF16, MODE_GREEDY>, grid, block, 0, st, *d, logits, seed, t, actions, log_prob, entropy)
+                   : ge_launch_step(policy_sample_kernel<GE_LOGITS_BF16, MODE_GUMBEL>, grid, block, 0, st, *d, logits, seed, t, actions, log_prob, entropy);
+    else
+        e = greedy ? ge_launch_step(policy_sample_kernel<GE_LOGITS_F32, MODE_GREEDY>, grid, block, 0, st, *d, logits, seed, t, actions, log_prob, entropy)
+                   : ge_launch_step(policy_sample_kernel<GE_LOGITS_F32, MODE_GUMBEL>, grid, block, 0, st, *d, logits, seed, t, actions, log_prob, entropy);
+    if (e != cudaSuccess) { (void)cudaGetLastError(); return ge_set_error(GE_ERR_CUDA, "policy_sample_kernel launch: %s", cudaGetErrorString(e)); }
+    return GE_OK;
+}
+
+int ge_masked_log_prob(const void *logits, int dtype, int B, int A, const uint32_t *mask_bits, const int32_t *actions, float *log_prob,
+                       float *entropy, float *lse, void *stream) {
+    GE_NVTX("ge_masked_log_prob");
+    int rc = check_rows("ge_masked_log_prob", logits, dtype, B, A, mask_bits, actions);
+    if (rc) return rc;
+    if (!log_prob || !entropy || !lse) return ge_set_error(GE_ERR_ARG, "ge_masked_log_prob: null log_prob / entropy / lse");
+    const unsigned grid = (unsigned)((B + POL_WPB - 1) / POL_WPB);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == GE_LOGITS_BF16) policy_logprob_kernel<GE_LOGITS_BF16><<<grid, POL_WPB * 32, 0, st>>>(logits, B, A, mask_bits, actions, log_prob, entropy, lse);
+    else policy_logprob_kernel<GE_LOGITS_F32><<<grid, POL_WPB * 32, 0, st>>>(logits, B, A, mask_bits, actions, log_prob, entropy, lse);
+    return launched("policy_logprob_kernel");
+}
+
+int ge_masked_log_prob_backward(const void *logits, int dtype, int B, int A, const uint32_t *mask_bits, const int32_t *actions,
+                                const float *lse, const float *entropy, const float *grad_log_prob, const float *grad_entropy,
+                                void *grad_logits, void *stream) {
+    GE_NVTX("ge_masked_log_prob_backward");
+    int rc = check_rows("ge_masked_log_prob_backward", logits, dtype, B, A, mask_bits, actions);
+    if (rc) return rc;
+    if (!lse || !entropy || !grad_logits) return ge_set_error(GE_ERR_ARG, "ge_masked_log_prob_backward: null lse / entropy / grad_logits");
+    const unsigned grid = (unsigned)((B + POL_WPB - 1) / POL_WPB);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == GE_LOGITS_BF16)
+        policy_logprob_bwd_kernel<GE_LOGITS_BF16><<<grid, POL_WPB * 32, 0, st>>>(logits, B, A, mask_bits, actions, lse, entropy, grad_log_prob, grad_entropy, grad_logits);
+    else
+        policy_logprob_bwd_kernel<GE_LOGITS_F32><<<grid, POL_WPB * 32, 0, st>>>(logits, B, A, mask_bits, actions, lse, entropy, grad_log_prob, grad_entropy, grad_logits);
+    return launched("policy_logprob_bwd_kernel");
+}
+
+}  // extern "C"

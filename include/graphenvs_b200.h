@@ -31,6 +31,8 @@
  *                     distribution parity only (device RNG), see DESIGN.md
  *   ge_sample_actions README.md:54-68 "random valid action" loop (policy stand-in for benches)
  *   ge_step_sampled   the same loop body fused: action draw + Env.step() in one launch
+ *   ge_sample_logits  the policy side of a training loop: a masked categorical over policy logits (Gumbel-max / greedy),
+ *   ge_masked_log_prob (+ _backward)  its differentiable log-prob and entropy for the update (ge_policy.cu)
  */
 #ifndef GRAPHENVS_B200_H
 #define GRAPHENVS_B200_H
@@ -305,6 +307,47 @@ int ge_step_host_release(const ge_batch *batch);
 
 /* Reduces acc[4,B] to out[4] (device double[4]): episodes, solved, sum reward, sum final cost. */
 int ge_stats(const ge_batch *batch, double *out4, void *stream);
+
+/* ---- Rollout helpers: a categorical policy over the valid actions (csrc/ge_policy.cu) ----
+ *
+ * Logits are row-major [rows, A] on the device, float32 (GE_LOGITS_F32) or bfloat16 (GE_LOGITS_BF16, upcast to float32);
+ * all arithmetic is float32.  The mask of row b is the packed bitset of ceil(A/32) words at mask_bits + b * ceil(A/32)
+ * (the layout of ge_batch.mask_bits).  Per row, over the VALID actions V only:
+ *   lse = log sum_{i in V} exp(l_i),  p_i = exp(l_i - lse),  H = lse - sum_{i in V} p_i l_i  (entropy in nats).
+ * Edge semantics (all three calls):
+ *   - empty mask row: action -1, log_prob 0, entropy 0, lse -inf, zero gradient (ge_sample_actions also returns -1);
+ *   - mask bits at positions >= A are ignored, and no logit at index >= A is ever read;
+ *   - logits of invalid actions are never read (NaN / inf there change nothing); logits of valid actions must be finite;
+ *   - ge_masked_log_prob with an action outside [0, A) or on a clear bit (non-empty row): log_prob = -inf, the entropy is still
+ *     computed, and the backward pass gets no gradient from that row's log_prob term;
+ *   - deterministic: no atomics and a fixed reduction order, the same inputs give bit-identical outputs; for the same logits,
+ *     mask and action, ge_sample_logits' log_prob / entropy equal ge_masked_log_prob's bit for bit (PPO ratio exactly 1);
+ *   - rows are addressed with size_t offsets (rows * A may exceed 2^31 elements).
+ * Bad arguments (unknown dtype, rows or A <= 0, a NULL required pointer) return GE_ERR_ARG. */
+#define GE_LOGITS_F32 0
+#define GE_LOGITS_BF16 1
+/* Draws actions[b] for every env of `batch` from its current packed mask (batch->mask_bits) and the logits [B, A]:
+ * greedy != 0: argmax of l over the valid actions; otherwise Gumbel-max, argmax of l_a + g_a.  Ties go to the lowest action
+ * index (greedy equals torch.argmax of the masked logits).  log_prob / entropy [B] (float32, may be NULL) of the chosen action.
+ * Noise: a pure counter-based function of (seed, e, t', a), e = env_id0 + b (global env id), t' = t + env_steps[b] when
+ * env_steps is set (uint32 arithmetic), with mix32 = the splitmix of ge_sample_actions (csrc/ge_common.cuh):
+ *   key = (uint64) mix32(seed, e, t') << 32 | mix32(seed ^ 0xD1B54A32D192ED03, e, t')
+ *   h   = mix32(key, a, 0x85EBCA6B),   u = ((h >> 8) + 0.5) / 2^24  (exact in float32, in (0, 1))
+ *   g_a = -logf(-logf(u)),   score_a = l_a + g_a  (float32)
+ * So a rank slice draws what the single-GPU batch draws, and a captured CUDA graph with the env clock draws fresh actions on
+ * every replay.  With all logits equal the draw is uniform but NOT the action ge_sample_actions picks (different noise).
+ * Under GE_FLAG_PDL the launch may start under the previous step's tail; it touches nothing before that step completes, and
+ * every step kernel reads actions[b] only after its own wait, so sample -> step -> sample chains are safe. */
+int ge_sample_logits(const ge_batch *batch, const void *logits, int dtype, int greedy, uint64_t seed, uint32_t t,
+                     int32_t *actions, float *log_prob, float *entropy, void *stream);
+/* log_prob, entropy, lse [rows] of actions[rows] under the masked categorical (no ge_batch: masks from a rollout buffer). */
+int ge_masked_log_prob(const void *logits, int dtype, int rows, int A, const uint32_t *mask_bits, const int32_t *actions,
+                       float *log_prob, float *entropy, float *lse, void *stream);
+/* Dense grad_logits [rows, A] in the logits' dtype from lse / entropy of ge_masked_log_prob (no second reduction):
+ *   g_lp (1[i = a] - p_i) - g_H p_i (log p_i + H) for valid i, 0 elsewhere.  grad_log_prob / grad_entropy may be NULL (= 0). */
+int ge_masked_log_prob_backward(const void *logits, int dtype, int rows, int A, const uint32_t *mask_bits, const int32_t *actions,
+                                const float *lse, const float *entropy, const float *grad_log_prob, const float *grad_entropy,
+                                void *grad_logits, void *stream);
 
 #ifdef __cplusplus
 }
