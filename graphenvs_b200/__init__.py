@@ -3,7 +3,8 @@
 Public surface:
   make(id, **kwargs)                 gymnasium-shaped single env (reference ids and kwargs)
   make_batched(id, num_envs, ...)    batched vector env with the same per-env semantics
-  BatchedGraphEnv                    the engine class behind both (sample_logits: policy-driven action draw)
+  BatchedGraphEnv                    the engine class behind both (sample_logits: policy-driven action draw;
+                                     save_states / load_states / gather_instances / like: branching for search decoders)
   masked_log_prob(logits, mask_bits, actions)   differentiable masked log-prob + entropy for the update (policy.py)
   utils.vectorize_graph / devectorize_graph / get_env_info   (graph_envs/utils.py layout contract)
 """
@@ -14,9 +15,9 @@ __version__ = "0.1.0"
 
 
 def __getattr__(attr):  # lazy: keeps `import graphenvs_b200` cheap and torch-free until needed
-    if attr in ("BatchedGraphEnv",):
-        from .batch import BatchedGraphEnv
-        return BatchedGraphEnv
+    if attr in ("BatchedGraphEnv", "EnvStates", "STATE_DYNAMIC", "STATE_CLOCK", "STATE_STATS", "STATE_ALL"):
+        from . import batch
+        return getattr(batch, attr)
     if attr in ("make", "make_batched", "register_with_gymnasium", "registry"):
         from . import registration
         return getattr(registration, attr)

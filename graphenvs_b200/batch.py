@@ -16,10 +16,26 @@ from . import _native
 from .spec import ENV_SPECS, check_ctor_args
 
 PREP_HEURISTIC, PREP_MAXDIST, PREP_INRANGE, PREP_ALT_HEURISTIC, PREP_DC_EDGES = 1, 2, 4, 8, 16
+STATE_DYNAMIC, STATE_CLOCK, STATE_STATS, STATE_ALL = (_native.STATE_DYNAMIC, _native.STATE_CLOCK, _native.STATE_STATS,
+                                                      _native.STATE_ALL)
+# the state arrays of a record (include/graphenvs_b200.h, GE_STATE_*): dynamic, clock, stats
+_STATE_ARRAYS = ("head", "node_bits", "node_bits2", "edge_bits", "dist32", "bestkey", "cost", "counters", "done", "mask_bits",
+                 "mask_cnt", "env_steps", "acc", "traj")
 
 
 def _ptr(t):
     return None if t is None else C.c_void_p(t.data_ptr())
+
+
+class EnvStates:
+    """Saved per-env states (BatchedGraphEnv.save_states): `data` is a uint8 [n, record_bytes] device tensor of opaque records
+    (ge_state_save), `signature` the env id, shape and set of state arrays a batch must have to load them."""
+
+    def __init__(self, data, signature):
+        self.data, self.signature = data, signature
+
+    def __len__(self):
+        return self.data.shape[0]
 
 
 class BatchedGraphEnv:
@@ -145,6 +161,21 @@ class BatchedGraphEnv:
         self._out = _native.StepOut(_ptr(self.reward), _ptr(self.flags), _ptr(self.solution_cost))
         self._loaded = False
 
+    def like(self, num_envs, **overrides):
+        """A new batch of `num_envs` envs, nothing loaded yet, with this batch's env id, parameters and engine options (device,
+        byte_mask, auto_reset, structural_features, env_id0, keep_w64, force_warp, dc_rows, dc_transposed); `overrides` replace
+        any of them.  Fill it with gather_instances(), e.g. the wide batch of a multi-start decoder."""
+        P = {k: v for k, v in self.params.items() if k in dict(self.spec.defaults)}   # ctor kwargs only, not derived values
+        P.pop("structural_features", None)          # ShortestPath's ignored ctor kwarg (shortest_path.py:23) vs the engine's own flag
+        n_nodes, n_edges = self.params["n_nodes"], self.params["n_edges"]
+        d = self.desc
+        opts = dict(device=self.device, byte_mask="mask_bytes" in self.t, auto_reset=bool(d.flags & 1),
+                    structural_features=self.structural_features, env_id0=d.env_id0, keep_w64="w64" in self.t,
+                    force_warp=bool(d.flags & 8), dc_rows=self._dc_rows, dc_transposed="in_range_t" in self.t)
+        opts.update(P)
+        opts.update(overrides)
+        return BatchedGraphEnv(self.env_id, num_envs, n_nodes, n_edges, **opts)
+
     # ------------------------------------------------------------------ plumbing
     def _sync_desc(self):
         for name in ("row_ptr", "col", "w32", "w64", "adj_bits", "rev", "esrc", "bestkey", "wsort", "wcode", "dfa", "dc_edges", "dc_rows", "wmin", "wmat", "src", "dest", "target_bits", "node_cost", "node_xy",
@@ -163,8 +194,9 @@ class BatchedGraphEnv:
 
     def enable_pdl(self, on=True):
         """GE_FLAG_PDL (include/graphenvs_b200.h): step launches may start under the tail of the previous launch of the stream
-        and prefetch static instance data; valid while the preceding work in the stream is another step (not generate() /
-        finalize_graphs() / an InstancePool refill, which rewrite static arrays)."""
+        and prefetch static instance data; valid while the preceding work in the stream is another step or a save_states() /
+        load_states() (not generate() / finalize_graphs() / gather_instances() / an InstancePool refill, which rewrite static
+        arrays)."""
         self.desc.flags = (self.desc.flags | 16) if on else (self.desc.flags & ~16)
 
     def _stream(self):
@@ -632,6 +664,108 @@ class BatchedGraphEnv:
 
     def state_dict(self):
         return {k: v.clone() for k, v in self.t.items()}
+
+    # ------------------------------------------------------------------ branching (csrc/ge_state.cu)
+    def state_signature(self):
+        """What a batch must share with the one a record was saved from: env id, shape parameters and the set of state arrays."""
+        d = self.desc
+        present = tuple(k for k in _STATE_ARRAYS if (self.env_steps is not None if k == "env_steps" else k in self.t))
+        return (self.env_id, d.kind, d.N, d.M, d.parenting, d.n_dests, d.n_choices, d.n_targets, present)
+
+    def record_bytes(self):
+        """Bytes of one env's state record (ge_state_record_bytes)."""
+        n = self.lib.ge_state_record_bytes(C.byref(self.desc))
+        if n < 0:
+            _native.check(n)
+        return n
+
+    def _index(self, index, n, lo, hi, who):
+        """An env / record index as int32 on the device.  A device tensor is trusted (out-of-range entries are skipped by the
+        kernels); host data must have n entries (any number up to self.B when n is None), all in [lo, hi)."""
+        if isinstance(index, torch.Tensor) and index.is_cuda:
+            if index.device != self.device or index.dim() != 1 or (n is not None and index.numel() != n):
+                raise ValueError("%s: index must be a 1-D tensor of %s entries on %s" % (who, n if n is not None else "<= B", self.device))
+            return index.to(torch.int32).contiguous()
+        a = np.asarray(index.numpy() if isinstance(index, torch.Tensor) else index)
+        if a.ndim != 1 or (a.size and a.dtype.kind not in "iu") or (n is not None and a.shape[0] != n) or (n is None and a.shape[0] > self.B):
+            raise ValueError("%s: index must be a 1-D integer sequence of %s entries" % (who, n if n is not None else "<= %d" % self.B))
+        if a.size and (int(a.min()) < lo or int(a.max()) >= hi):
+            raise ValueError("%s: index entries must lie in [%d, %d)" % (who, lo, hi))
+        return torch.from_numpy(a.astype(np.int32)).to(self.device)
+
+    def save_states(self, index=None, out=None):
+        """EnvStates of envs `index` (all envs when None), one record each, every state array included (ge_state_save).
+        out: an EnvStates of this batch's signature with as many records, to write into."""
+        idx = None if index is None else self._index(index, None, 0, self.B, "save_states")
+        n = self.B if idx is None else idx.numel()
+        sig = self.state_signature()
+        if out is None:
+            out = EnvStates(torch.empty((n, self.record_bytes()), dtype=torch.uint8, device=self.device), sig)
+        elif not isinstance(out, EnvStates) or out.signature != sig or tuple(out.data.shape) != (n, self.record_bytes()):
+            raise ValueError("save_states: out must be EnvStates of this batch's signature with %d records" % n)
+        _native.check(self.lib.ge_state_save(C.byref(self.desc), _ptr(idx), n, _ptr(out.data), self._stream()))
+        return out
+
+    def load_states(self, states, index=None, what=STATE_ALL):
+        """Env b <- record index[b] of `states` (record b when index is None) -- ge_state_load.  what: STATE_DYNAMIC, plus
+        STATE_CLOCK (env_steps) and / or STATE_STATS (acc, traj).  A host index is validated (-1 = leave env b as it is); a
+        device index is trusted and its out-of-range entries leave their envs untouched.  An in-place fork within one batch is
+        env.load_states(env.save_states(), parents)."""
+        if not isinstance(states, EnvStates):
+            raise TypeError("load_states: states must be EnvStates (from save_states)")
+        if states.signature != self.state_signature():
+            raise ValueError("load_states: records saved from a batch of signature %s cannot be loaded into one of %s"
+                             % (states.signature, self.state_signature()))
+        data = states.data
+        if data.device != self.device or data.dtype != torch.uint8 or data.dim() != 2 or not data.is_contiguous():
+            raise ValueError("load_states: records must be a contiguous uint8 [n, record_bytes] tensor on %s" % self.device)
+        n = data.shape[0]
+        if index is None and n < self.B:
+            raise ValueError("load_states: %d records for %d envs (pass an index)" % (n, self.B))
+        idx = None if index is None else self._index(index, self.B, -1, n, "load_states")
+        if data.shape[1] != self.record_bytes():
+            raise ValueError("load_states: records of %d bytes, this batch's are %d" % (data.shape[1], self.record_bytes()))
+        _native.check(self.lib.ge_state_load(C.byref(self.desc), _ptr(data), n, _ptr(idx), int(what), self._stream()))
+
+    def gather_instances(self, src, index=None):
+        """Env b <- the instance (every static array) of src env index[b] (src env b when None) -- ge_gather_instances.
+        src: a loaded BatchedGraphEnv of the same env id and shape (e.g. this batch's like()).  A host index is validated
+        (-1 = leave env b as it is); a device index is trusted.  Writes no state: follow with reset() or load_states().
+        DistributionCenter: the batches must share the distance automaton; a batch without one takes src's when the gather
+        covers every env."""
+        if not isinstance(src, BatchedGraphEnv):
+            raise TypeError("gather_instances: src must be a BatchedGraphEnv")
+        if src is self:
+            raise ValueError("gather_instances: src must be another batch (no in-place gather)")
+        if src.env_id != self.env_id or not src._loaded:
+            raise ValueError("gather_instances: src must be a loaded %s batch" % self.env_id)
+        if index is None and src.B < self.B:
+            raise ValueError("gather_instances: src has %d envs, this batch %d (pass an index)" % (src.B, self.B))
+        idx = None if index is None else self._index(index, self.B, -1, src.B, "gather_instances")
+        if "dfa" in self.t or "dfa" in src.t:
+            if "dfa" in self.t and "dfa" in src.t:
+                if not torch.equal(self.t["dfa"], src.t["dfa"]):
+                    raise ValueError("gather_instances: the batches have different distance automata")
+            elif "dfa" in src.t and (idx is None or bool(((idx >= 0) & (idx < src.B)).all())):
+                self._take_automaton(src)
+            else:
+                raise ValueError("gather_instances: the distance automaton of src (%s) and of this batch (%s) differ; a batch "
+                                 "takes src's only when the gather covers every env" % ("dfa" in src.t, "dfa" in self.t))
+        _native.check(self.lib.ge_gather_instances(C.byref(self.desc), C.byref(src.desc), _ptr(idx), self._stream()))
+        self._loaded = True
+        self._features_loaded = "features" in self.t
+
+    def _take_automaton(self, src):
+        """DistributionCenter: src's distance automaton and room for the arrays derived from it (filled by the gather)."""
+        T, B, MP = self.t, self.B, self.desc.MP
+        T["dfa"] = src.t["dfa"].clone()
+        T["wcode"] = torch.zeros((B, MP), dtype=torch.uint8, device=self.device)
+        if "dc_edges" in src.t:
+            T["dc_edges"] = torch.zeros((B, MP), dtype=torch.int32, device=self.device)
+        if "dc_rows" in src.t and self._dc_rows:
+            T["dc_rows"] = torch.zeros((B, self.N, 32), dtype=torch.int32, device=self.device)
+        self._sync_desc()
+        self.desc.dfa_bytes = src.desc.dfa_bytes
 
     def load_state_dict(self, sd):
         for k, v in sd.items():

@@ -8,28 +8,13 @@
 // (instead of an indirection in every kernel) keeps the hot step kernels and their tiled / bulk-staged layouts unchanged;
 // the copy costs the instance's bytes once per episode.  Banks are regenerated in the background by the host side
 // (graphenvs_b200/pool.py) on another stream; a bank being regenerated is simply absent from `order`.
-#include "ge_common.cuh"
+#include "ge_static.cuh"
 
 using namespace ge;
 
-extern "C" int ge_set_error(int code, const char *fmt, ...);
-
 namespace {
 
-constexpr int POOL_MAX_BANKS = 8, POOL_MAX_ARRAYS = 24;
-
-struct PoolArr {
-    const char *src[POOL_MAX_BANKS];
-    char *dst;
-    uint32_t bytes;   // per env
-    uint32_t tiled;   // adjacency tiles of 32 envs (ge_common.cuh:adj_tiled): element = NW words, N rows at a pitch of 32 elements
-};
-struct PoolTab {
-    int n, n_banks;
-    PoolArr a[POOL_MAX_ARRAYS];
-};
-
-__global__ void __launch_bounds__(256) pool_refill_kernel(ge_batch d, PoolTab tab, const int32_t *__restrict__ order, int n_active,
+__global__ void __launch_bounds__(256) pool_refill_kernel(ge_batch d, StaticTab tab, const int32_t *__restrict__ order, int n_active,
                                                         uint32_t *__restrict__ episode, uint8_t *__restrict__ select) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int b = blockIdx.x * 8 + warp;
@@ -41,30 +26,7 @@ __global__ void __launch_bounds__(256) pool_refill_kernel(ge_batch d, PoolTab ta
     const int k = order[ep % (uint32_t)n_active];
     __syncwarp();
     if (lane == 0) episode[b] = ep + 1u;
-    for (int i = 0; i < tab.n; ++i) {
-        const PoolArr &A = tab.a[i];
-        if (A.tiled) {
-            const size_t el = (size_t)d.NW * 4, tile = (size_t)d.N * 32 * el;
-            const char *s = A.src[k] + (size_t)(b >> 5) * tile + (size_t)(b & 31) * el;
-            char *t = A.dst + (size_t)(b >> 5) * tile + (size_t)(b & 31) * el;
-            for (int r = lane; r < d.N; r += 32) {
-                if (d.NW == 1) *reinterpret_cast<uint32_t *>(t + (size_t)r * 32 * el) = *reinterpret_cast<const uint32_t *>(s + (size_t)r * 32 * el);
-                else *reinterpret_cast<uint2 *>(t + (size_t)r * 32 * el) = *reinterpret_cast<const uint2 *>(s + (size_t)r * 32 * el);
-            }
-            continue;
-        }
-        const char *s = A.src[k] + (size_t)b * A.bytes;
-        char *t = A.dst + (size_t)b * A.bytes;
-        if ((A.bytes & 15u) == 0) {
-            const uint4 *s4 = reinterpret_cast<const uint4 *>(s);
-            uint4 *t4 = reinterpret_cast<uint4 *>(t);
-            for (uint32_t j = lane; j < (A.bytes >> 4); j += 32) t4[j] = s4[j];
-        } else {
-            const uint32_t *s1 = reinterpret_cast<const uint32_t *>(s);
-            uint32_t *t1 = reinterpret_cast<uint32_t *>(t);
-            for (uint32_t j = lane; j < (A.bytes >> 2); j += 32) t1[j] = s1[j];
-        }
-    }
+    copy_static_env(d, tab, k, (size_t)b, (size_t)b, lane);
 }
 
 }  // namespace
@@ -75,40 +37,14 @@ extern "C" int ge_pool_refill(const ge_batch *live, const ge_batch *banks, int n
                               uint32_t *episode, uint8_t *select, void *stream) {
     GE_NVTX("ge_pool_refill");
     if (!live || !banks || !order || !episode || !select) return ge_set_error(GE_ERR_ARG, "ge_pool_refill: null argument");
-    if (n_banks < 1 || n_banks > POOL_MAX_BANKS || n_active < 1 || n_active > n_banks) return ge_set_error(GE_ERR_ARG, "ge_pool_refill: 1 <= n_active <= n_banks <= %d", POOL_MAX_BANKS);
-    PoolTab tab;
-    tab.n = 0;
-    tab.n_banks = n_banks;
+    if (n_banks < 1 || n_banks > STATIC_MAX_SRC || n_active < 1 || n_active > n_banks) return ge_set_error(GE_ERR_ARG, "ge_pool_refill: 1 <= n_active <= n_banks <= %d", STATIC_MAX_SRC);
     for (int k = 0; k < n_banks; ++k)
         if (banks[k].kind != live->kind || banks[k].N != live->N || banks[k].M != live->M || banks[k].B < live->B ||
             ((banks[k].flags ^ live->flags) & GE_FLAG_FORCE_WARP))
             return ge_set_error(GE_ERR_ARG, "ge_pool_refill: bank %d is not shaped like the live batch", k);
     const ge_batch &d = *live;
-    auto add = [&](const void *dst, size_t offset_in_struct, size_t bytes, bool tiled) -> int {
-        if (!dst || bytes == 0) return GE_OK;                         // the live batch does not carry this array
-        if (tab.n == POOL_MAX_ARRAYS) return ge_set_error(GE_ERR_ARG, "ge_pool_refill: array table full");
-        PoolArr &A = tab.a[tab.n];
-        for (int k = 0; k < n_banks; ++k) {
-            const void *src = *reinterpret_cast<void *const *>(reinterpret_cast<const char *>(&banks[k]) + offset_in_struct);
-            if (!src) return ge_set_error(GE_ERR_ARG, "ge_pool_refill: bank %d lacks an array the live batch has (struct offset %zu)", k, offset_in_struct);
-            A.src[k] = reinterpret_cast<const char *>(src);
-        }
-        A.dst = reinterpret_cast<char *>(const_cast<void *>(dst));
-        A.bytes = (uint32_t)bytes;
-        A.tiled = tiled ? 1u : 0u;
-        ++tab.n;
-        return GE_OK;
-    };
-    int rc = GE_OK;
-#define POOL_ADD(field, bytes) if (rc == GE_OK) rc = add(d.field, offsetof(ge_batch, field), (size_t)(bytes), false)
-    POOL_ADD(row_ptr, d.RP * 4); POOL_ADD(col, d.MP * 4); POOL_ADD(w32, d.MP * 4); POOL_ADD(w64, d.MP * 8);
-    if (rc == GE_OK) rc = add(d.adj_bits, offsetof(ge_batch, adj_bits), adj_tiled(d) ? 4 : (size_t)d.ADJS * 4, adj_tiled(d));
-    POOL_ADD(rev, d.MP * 4); POOL_ADD(esrc, d.MP * 4); POOL_ADD(wsort, d.MP * 8); POOL_ADD(wcode, d.MP); POOL_ADD(dc_edges, d.MP * 4); POOL_ADD(dc_rows, (size_t)d.N * 128); POOL_ADD(wmin, 8);
-    POOL_ADD(wmat, (size_t)d.N * d.N * 8); POOL_ADD(src, 4); POOL_ADD(dest, 4); POOL_ADD(target_bits, d.NW * 4);
-    POOL_ADD(node_cost, d.N * 4); POOL_ADD(node_xy, d.N * 8); POOL_ADD(max_dist32, 4); POOL_ADD(targets, d.n_targets * 4);
-    POOL_ADD(in_range, (size_t)d.n_targets * d.NW * 4); POOL_ADD(in_range_t, (size_t)d.N * 16); POOL_ADD(heuristic, 8); POOL_ADD(heuristic_alt, 8);
-    POOL_ADD(features, d.N * 20); POOL_ADD(mask0_bits, d.AW * 4);
-#undef POOL_ADD
+    StaticTab tab;
+    int rc = static_table(d, banks, n_banks, tab, "ge_pool_refill");
     if (rc) return rc;
     pool_refill_kernel<<<(d.B + 7) / 8, 256, 0, (cudaStream_t)stream>>>(d, tab, order, n_active, episode, select);
     cudaError_t e = cudaGetLastError();

@@ -12,7 +12,7 @@ import ctypes as C
 import torch
 
 from . import _native
-from .batch import BatchedGraphEnv, _ptr
+from .batch import _ptr
 
 
 class InstancePool:
@@ -20,15 +20,10 @@ class InstancePool:
         assert not (env.desc.flags & 1), "the live batch must run with auto_reset=False: the pool performs the resets"
         assert 2 <= banks <= 8
         self.env, self.G, self.seed = env, int(banks), int(seed)
-        P = dict(env.params)
-        n_nodes, n_edges = P.pop("n_nodes"), P.pop("n_edges")
-        P.pop("structural_features", None)          # ShortestPath's ignored ctor kwarg (shortest_path.py:23) vs the engine's own flag
         self.banks = []
         for k in range(self.G):
-            b = BatchedGraphEnv(env.env_id, env.B, n_nodes, n_edges, device=env.device, byte_mask=False, auto_reset="mask0_bits" in env.t,
-                                structural_features=env.structural_features, env_id0=env.desc.env_id0,
-                                force_warp=bool(env.desc.flags & 8), dc_rows="dc_rows" in env.t,
-                                dc_transposed="in_range_t" in env.t, **P)
+            # banks keep their float64 weights: a generate() without them synchronises, and banks regenerate in the background
+            b = env.like(env.B, byte_mask=False, keep_w64=True, dc_rows="dc_rows" in env.t)
             b.generate(seed=self._next_seed(), check=False)
             if "mask0_bits" in b.t:
                 b.reset()                       # fills mask0_bits (the first mask depends only on the instance)

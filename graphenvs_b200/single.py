@@ -9,13 +9,14 @@ reset(seed) reseeds the process-global `random` / `numpy.random` exactly like th
 (shortest_path.py:49-52) and regenerates the same instance (instances.py); state, masks,
 transitions, structural features and the tie-independent heuristics are computed on the GPU.
 """
+import copy
 import random
 import warnings
 
 import numpy as np
 import torch
 
-from .batch import BatchedGraphEnv
+from .batch import STATE_ALL, BatchedGraphEnv
 from .instances import generate_instance
 from .utils import graph_from_obs
 
@@ -54,6 +55,7 @@ _EVERY_STEP_HEURISTIC = ("LongestPath-v0", "DensestSubgraph-v0", "MulticastRouti
 class GraphEnv(_Base):
     def __init__(self, env_id, n_nodes, n_edges=-1, device=None, **kwargs):
         self.env_id = env_id
+        self._ctor = (n_nodes, n_edges, device, dict(kwargs))
         self.core = BatchedGraphEnv(env_id, 1, n_nodes, n_edges, device=device, structural_features=True, **kwargs)
         c, P = self.core, self.core.params
         self.params = P
@@ -73,6 +75,24 @@ class GraphEnv(_Base):
         self._warned = False
         self.instance = None
         self._track = None
+
+    def __deepcopy__(self, memo):
+        """Branch this env: a new env with its own engine batch holding the same instance (ge_gather_instances) and the same
+        state, env clock and statistics (ge_state_save / ge_state_load), plus deep copies of the host-side attributes.  The
+        copy and the original then evolve independently."""
+        new = type(self).__new__(type(self))
+        memo[id(self)] = new
+        for k, v in self.__dict__.items():
+            if k != "core":
+                setattr(new, k, copy.deepcopy(v, memo))
+        n_nodes, n_edges, device, kwargs = self._ctor
+        new.core = BatchedGraphEnv(self.env_id, 1, n_nodes, n_edges, device=device, structural_features=True, **kwargs)
+        if self.core.env_steps is not None:
+            new.core.enable_env_clock()
+        if self.core._loaded:
+            new.core.gather_instances(self.core)
+            new.core.load_states(self.core.save_states(), what=STATE_ALL)
+        return new
 
     # ------------------------------------------------------------------ helpers
     def _obs(self):

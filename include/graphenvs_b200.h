@@ -33,6 +33,8 @@
  *   ge_step_sampled   the same loop body fused: action draw + Env.step() in one launch
  *   ge_sample_logits  the policy side of a training loop: a masked categorical over policy logits (Gumbel-max / greedy),
  *   ge_masked_log_prob (+ _backward)  its differentiable log-prob and entropy for the update (ge_policy.cu)
+ *   ge_state_save / ge_state_load / ge_gather_instances  branching an env, i.e. copy.deepcopy(env) of a gym env: per-env state
+ *                     records and instance replication for search decoders (multi-start, beam search, lookahead; ge_state.cu)
  */
 #ifndef GRAPHENVS_B200_H
 #define GRAPHENVS_B200_H
@@ -75,7 +77,8 @@ typedef enum {
                                    resident -- and prefetch STATIC instance data (adjacency tiles, automaton tables) -- while the previous
                                    launch of the stream is still running; it waits for that launch (griddepcontrol.wait) before it touches
                                    any env state.  The caller promises that the preceding work in the stream does not write this batch's
-                                   static arrays (i.e. it is another step, not ge_generate / ge_build_adjacency / ge_pool_refill). */
+                                   static arrays (i.e. it is another step or a state save / load, not ge_generate / ge_build_adjacency /
+                                   ge_pool_refill / ge_gather_instances). */
 
 /* per-env status written by ge_step into flags[b].status */
 #define GE_STEP_OK 0
@@ -348,6 +351,46 @@ int ge_masked_log_prob(const void *logits, int dtype, int rows, int A, const uin
 int ge_masked_log_prob_backward(const void *logits, int dtype, int rows, int A, const uint32_t *mask_bits, const int32_t *actions,
                                 const float *lse, const float *entropy, const float *grad_log_prob, const float *grad_entropy,
                                 void *grad_logits, void *stream);
+
+/* ---- Branching: per-env state records and instance replication (csrc/ge_state.cu) ----
+ *
+ * A RECORD is one env's state: opaque, ge_state_record_bytes(batch) bytes long (a multiple of 16).  What counts as state:
+ *   GE_STATE_DYNAMIC  every non-NULL array among head, node_bits, node_bits2, edge_bits, dist32, bestkey, cost, counters, done,
+ *                     mask_bits, mask_cnt (what ge_step reads and writes besides its outputs);
+ *   GE_STATE_CLOCK    env_steps;
+ *   GE_STATE_STATS    the env's acc column (4 doubles at stride acc_stride) and traj.
+ * The step outputs, obs_x and mask_bytes are not state.  Sections come in the order of these lists; those of at most 64 bytes per
+ * env first, each at its element's natural alignment, then (from a 16-byte boundary) the larger ones, each at a 16-byte offset; an
+ * absent array has no section, and the record is rounded up to 16 bytes.
+ * A record can be loaded only into a batch with the same kind, N, M, parenting, n_dests, n_choices and n_targets and the same set of
+ * non-NULL state arrays, and it only makes sense in an env that holds the same instance it was saved from: the library checks
+ * neither (the Python layer checks the first).  Record buffers are 16-byte aligned device memory; offsets are size_t (a buffer may
+ * pass 2^31 bytes).  Save and load never read or write a static array, so a GE_FLAG_PDL step may follow either.  No call here
+ * synchronises or allocates: they can be captured in a CUDA graph.  Arguments are checked before any CUDA call. */
+#define GE_STATE_DYNAMIC 1u   /* required: what ge_step reads and writes besides its outputs */
+#define GE_STATE_CLOCK 2u     /* env_steps */
+#define GE_STATE_STATS 4u     /* the env's acc column (4 doubles at stride acc_stride) and traj */
+#define GE_STATE_ALL 7u
+/* Bytes of one record of this batch (> 0), or a negative ge_status. */
+int ge_state_record_bytes(const ge_batch *batch);
+/* Record i <- env env_index[i] for i in [0, count) (env i when env_index is NULL); count <= B.  Every section is written; an env
+ * index outside [0, B) leaves record i untouched.  records: device [count, ge_state_record_bytes]. */
+int ge_state_save(const ge_batch *batch, const int32_t *env_index, int count, void *records, void *stream);
+/* For each b in [0, B): env b <- record record_index[b] (record b when record_index is NULL, which requires n_records >= B).  An
+ * index < 0 or >= n_records leaves env b untouched, byte for byte.  Only the sections named in `what` are written, and `what` must
+ * include GE_STATE_DYNAMIC.  A loaded env's mask_bytes is rebuilt when ge_mask_bytes_current(batch), and its mask_mirror written
+ * when set and ge_mask_mirror_supported(batch) (the mirror is the second destination of every packed-mask write).  records must
+ * not overlap the batch's arrays: an in-place fork is a save to a separate buffer followed by a load. */
+int ge_state_load(const ge_batch *batch, const void *records, int n_records, const int32_t *record_index, unsigned what,
+                  void *stream);
+/* For each b in [0, dst->B): dst env b <- the static arrays of src env src_index[b] (src env b when src_index is NULL, which requires
+ * src->B >= dst->B); an index < 0 or >= src->B leaves env b untouched.  The arrays copied are those ge_pool_refill copies, every
+ * one dst carries.  dst and src may differ in B and either may be a ge_batch_slice.  GE_ERR_ARG when kind, N, M, parenting,
+ * n_dests, n_choices, n_targets, max_distance or GE_FLAG_FORCE_WARP differ, when dst carries an array src lacks, when dfa_bytes
+ * differ (the shared `dfa` itself is the caller's to copy) or when static ranges of dst and src overlap (no in-place gather).
+ * Writes no state: follow it with ge_reset(select) or ge_state_load.  It writes static arrays, so the step after it must not be
+ * launched with GE_FLAG_PDL. */
+int ge_gather_instances(const ge_batch *dst, const ge_batch *src, const int32_t *src_index, void *stream);
 
 #ifdef __cplusplus
 }
