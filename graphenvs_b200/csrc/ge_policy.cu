@@ -237,6 +237,133 @@ __global__ void __launch_bounds__(POL_WPB * 32) policy_logprob_bwd_kernel(const 
     }
 }
 
+// ---- beam search (ge_beam_expand): one CTA per group of W beams, one warp per beam (BEAM_WARPS warps take turns past 8) ----
+constexpr int BEAM_MAXW = 32;
+constexpr int BEAM_WARPS = 8;
+
+// THE candidate order of ge_beam_expand: score descending, then parent slot ascending, then action ascending.  Stage 1 ranks one
+// beam's candidates with it (equal parents), stage 2 merges the beams' lists with it; it is a total order, so every reduction
+// below gives the same winner whatever order it visits the candidates in.
+__device__ __forceinline__ bool beam_before(float s1, int p1, int a1, float s2, int p2, int a2) {
+    return s1 > s2 || (s1 == s2 && (p1 < p2 || (p1 == p2 && a1 < a2)));
+}
+
+// The best candidate of one live beam that comes after (ps, pa) in the order (the best overall when `first`), over its valid
+// actions: score fl32(base + fl32(l_a - lse)).  Walks the row as masked_row does (zero words skipped warp-uniformly, only
+// logits of set bits read); after the first walk the mask and the valid logits are L1-resident.  Warp-uniform result;
+// ba = INT_MAX when no candidate is left.
+template <int DT>
+__device__ __forceinline__ void beam_next(const void *row, const uint32_t *__restrict__ mrow, int A, int AW, float base, float lse,
+                                          bool first, float ps, int pa, int lane, float &bs, int &ba) {
+    float s_best = -INFINITY;
+    int a_best = INT_MAX;
+    for (int w0 = 0; w0 < AW; w0 += 32) {
+        const int wl = w0 + lane;
+        const uint32_t mw = wl < AW ? (__ldg(mrow + wl) & tail_mask(A, wl)) : 0u;
+        unsigned nz = __ballot_sync(GE_FULL, mw != 0u);
+        while (nz) {
+            float v[POL_U];
+            int idx[POL_U];
+            bool has[POL_U];
+#pragma unroll
+            for (int k = 0; k < POL_U; ++k) {
+                const int src = nz ? __ffs((int)nz) - 1 : 0;
+                const bool any = nz != 0u;
+                nz &= nz - 1u;
+                const uint32_t word = __shfl_sync(GE_FULL, mw, src);
+                idx[k] = ((w0 + src) << 5) + lane;
+                has[k] = any && ((word >> lane) & 1u);
+                v[k] = has[k] ? load_logit<DT>(row, (size_t)idx[k]) : 0.f;
+            }
+#pragma unroll
+            for (int k = 0; k < POL_U; ++k) {
+                if (!has[k]) continue;
+                const float s = __fadd_rn(base, __fsub_rn(v[k], lse));
+                if ((first || beam_before(ps, 0, pa, s, 0, idx[k])) && beam_before(s, 0, idx[k], s_best, 0, a_best)) { s_best = s; a_best = idx[k]; }
+            }
+        }
+    }
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+        const float s = __shfl_xor_sync(GE_FULL, s_best, o);
+        const int a = __shfl_xor_sync(GE_FULL, a_best, o);
+        if (beam_before(s, 0, a, s_best, 0, a_best)) { s_best = s; a_best = a; }
+    }
+    bs = s_best; ba = a_best;
+}
+
+template <int DT>
+__global__ void __launch_bounds__(BEAM_WARPS * 32) beam_expand_kernel(ge_batch d, int W, const void *__restrict__ logits,
+                                                                       const float *__restrict__ score, float *__restrict__ score_out,
+                                                                       int32_t *__restrict__ parent, int32_t *__restrict__ action,
+                                                                       int32_t *__restrict__ load_index) {
+    __shared__ float l_s[BEAM_MAXW][BEAM_MAXW];   // per beam: its best min(W, candidates) candidates, in the order
+    __shared__ int l_a[BEAM_MAXW][BEAM_MAXW];
+    __shared__ int l_n[BEAM_MAXW];
+    pdl_launch_dependents();   // as the sampler: nothing is touched before pdl_wait()
+    pdl_wait();
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    const int g0 = blockIdx.x * W;   // env index of the group's slot 0
+    const size_t esz = DT == GE_LOGITS_BF16 ? 2 : 4;
+    // Stage 1: every beam's own sorted candidate list
+    for (int p = warp; p < W; p += nwarps) {
+        const int b = g0 + p;
+        const float base = score[b];
+        int n = 0;
+        if (base == -INFINITY) {
+            n = 0;                                             // dead
+        } else if (d.done[b]) {
+            if (lane == 0) { l_s[p][0] = base; l_a[p][0] = -1; }   // stay
+            n = 1;
+        } else {
+            const void *row = reinterpret_cast<const char *>(logits) + (size_t)b * d.A * esz;
+            const uint32_t *mrow = d.mask_bits + (size_t)b * d.AW;
+            const RowStats r = masked_row<DT, MODE_STATS>(row, mrow, d.A, d.AW, 0, lane);
+            if (r.se > 0.f) {
+                const float lse = row_lse(r);
+                float ps = 0.f;
+                int pa = 0;
+                for (; n < W; ++n) {
+                    beam_next<DT>(row, mrow, d.A, d.AW, base, lse, n == 0, ps, pa, lane, ps, pa);
+                    if (pa == INT_MAX) break;
+                    if (lane == 0) { l_s[p][n] = ps; l_a[p][n] = pa; }
+                }
+            }
+        }
+        if (lane == 0) l_n[p] = n;
+    }
+    __syncthreads();
+    if (warp != 0) return;
+    // Stage 2: lane p holds the head of list p; W rounds of a warp arg-max in the order produce the W winners
+    int head = 0;
+    const int len = lane < W ? l_n[lane] : 0;
+    float my_s = -INFINITY;
+    int my_p = -1, my_a = -1;
+    for (int j = 0; j < W; ++j) {
+        float s = -INFINITY;
+        int p = INT_MAX, a = INT_MAX;                          // no candidate: after every real one
+        if (head < len) { s = l_s[lane][head]; p = lane; a = l_a[lane][head]; }
+#pragma unroll
+        for (int o = 16; o; o >>= 1) {
+            const float s2 = __shfl_xor_sync(GE_FULL, s, o);
+            const int p2 = __shfl_xor_sync(GE_FULL, p, o);
+            const int a2 = __shfl_xor_sync(GE_FULL, a, o);
+            if (beam_before(s2, p2, a2, s, p, a)) { s = s2; p = p2; a = a2; }
+        }
+        if (p == INT_MAX) break;                               // the group has fewer than W candidates: the rest stay empty
+        if (lane == p) ++head;
+        if (lane == j) { my_s = s; my_p = p; my_a = a; }
+    }
+    if (lane < W) {
+        const int b = g0 + lane;
+        const int par = my_p < 0 ? -1 : g0 + my_p;
+        score_out[b] = my_s;
+        parent[b] = par;
+        action[b] = my_a;
+        load_index[b] = par == b ? -1 : par;
+    }
+}
+
 int launched(const char *what) {
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? GE_OK : ge_set_error(GE_ERR_CUDA, "%s launch: %s", what, cudaGetErrorString(e));
@@ -300,6 +427,35 @@ int ge_masked_log_prob_backward(const void *logits, int dtype, int B, int A, con
     else
         policy_logprob_bwd_kernel<GE_LOGITS_F32><<<grid, POL_WPB * 32, 0, st>>>(logits, B, A, mask_bits, actions, lse, entropy, grad_log_prob, grad_entropy, grad_logits);
     return launched("policy_logprob_bwd_kernel");
+}
+
+int ge_beam_expand(const ge_batch *d, int W, const void *logits, int dtype, const float *score, float *score_out, int32_t *parent,
+                   int32_t *action, int32_t *load_index, void *stream) {
+    GE_NVTX("ge_beam_expand");
+    if (!d) return ge_set_error(GE_ERR_ARG, "ge_beam_expand: null batch");
+    if (dtype != GE_LOGITS_F32 && dtype != GE_LOGITS_BF16) return ge_set_error(GE_ERR_ARG, "ge_beam_expand: unknown logits dtype %d", dtype);
+    if (W < 1 || W > BEAM_MAXW) return ge_set_error(GE_ERR_ARG, "ge_beam_expand: width W = %d not in [1, %d]", W, BEAM_MAXW);
+    if (d->B <= 0 || d->A <= 0 || d->AW != (d->A + 31) / 32) return ge_set_error(GE_ERR_ARG, "ge_beam_expand: bad shape B=%d A=%d AW=%d (call ge_fill_layout)", d->B, d->A, d->AW);
+    if (d->B % W) return ge_set_error(GE_ERR_ARG, "ge_beam_expand: B = %d is not a multiple of W = %d", d->B, W);
+    if (!logits || !score || !score_out || !parent || !action || !load_index)
+        return ge_set_error(GE_ERR_ARG, "ge_beam_expand: null logits / score / score_out / parent / action / load_index");
+    if (!d->mask_bits || !d->done) return ge_set_error(GE_ERR_ARG, "ge_beam_expand: null mask_bits / done in the batch");
+    {   // no two of score, score_out, parent, action, load_index (B 4-byte elements each) may overlap
+        const uintptr_t p[5] = {(uintptr_t)score, (uintptr_t)score_out, (uintptr_t)parent, (uintptr_t)action, (uintptr_t)load_index};
+        const uintptr_t n = (uintptr_t)d->B * 4u;
+        for (int i = 0; i < 5; ++i)
+            for (int j = i + 1; j < 5; ++j)
+                if (p[i] < p[j] + n && p[j] < p[i] + n)
+                    return ge_set_error(GE_ERR_ARG, "ge_beam_expand: score, score_out, parent, action and load_index must not overlap");
+    }
+    const int warps = W < BEAM_WARPS ? W : BEAM_WARPS;
+    const dim3 grid((unsigned)(d->B / W)), block(warps * 32);
+    cudaStream_t st = (cudaStream_t)stream;
+    const cudaError_t e = dtype == GE_LOGITS_BF16
+        ? ge_launch_step(beam_expand_kernel<GE_LOGITS_BF16>, grid, block, 0, st, *d, W, logits, score, score_out, parent, action, load_index)
+        : ge_launch_step(beam_expand_kernel<GE_LOGITS_F32>, grid, block, 0, st, *d, W, logits, score, score_out, parent, action, load_index);
+    if (e != cudaSuccess) { (void)cudaGetLastError(); return ge_set_error(GE_ERR_CUDA, "beam_expand_kernel launch: %s", cudaGetErrorString(e)); }
+    return GE_OK;
 }
 
 }  // extern "C"

@@ -33,6 +33,7 @@
  *   ge_step_sampled   the same loop body fused: action draw + Env.step() in one launch
  *   ge_sample_logits  the policy side of a training loop: a masked categorical over policy logits (Gumbel-max / greedy),
  *   ge_masked_log_prob (+ _backward)  its differentiable log-prob and entropy for the update (ge_policy.cu)
+ *   ge_beam_expand    one beam-search step: every beam's valid continuations scored and the W best per instance kept (ge_policy.cu)
  *   ge_state_save / ge_state_load / ge_gather_instances  branching an env, i.e. copy.deepcopy(env) of a gym env: per-env state
  *                     records and instance replication for search decoders (multi-start, beam search, lookahead; ge_state.cu)
  */
@@ -351,6 +352,28 @@ int ge_masked_log_prob(const void *logits, int dtype, int rows, int A, const uin
 int ge_masked_log_prob_backward(const void *logits, int dtype, int rows, int A, const uint32_t *mask_bits, const int32_t *actions,
                                 const float *lse, const float *entropy, const float *grad_log_prob, const float *grad_entropy,
                                 void *grad_logits, void *stream);
+/* One beam-search step over a batch of B = G * W envs: group g is envs [g*W, g*W + W), 1 <= W <= 32 (W beams of one instance).
+ * Reads batch->mask_bits, batch->done, logits [B, A] (layout and dtype of ge_sample_logits) and score [B], the running beam
+ * scores (float32 sums of log-probs).  Beam b of group g contributes:
+ *   - nothing when score[b] == -inf (a DEAD beam);
+ *   - when done[b]: one STAY candidate (b, action -1) of score score[b];
+ *   - otherwise one candidate (b, a) per valid action a, of score fl32(score[b] + fl32(l_a - lse_b)), lse_b the masked log-sum-exp
+ *     of ge_masked_log_prob (so the log-prob term equals ge_masked_log_prob's bit for bit); a live beam with an empty mask none.
+ * Within each group, output slot j (env g*W + j) gets the j-th best candidate of the group in the total order: score descending,
+ * then parent slot ascending, then action ascending -- a stable sort of all the group's candidates, exact:
+ *   parent[j]     env index (in [0, B) of this descriptor) of the candidate's beam, -1 when the group has fewer than W candidates;
+ *   action[j]     the candidate's action, -1 for a stay or an empty slot;
+ *   score_out[j]  its score, -inf for an empty slot (which is then dead in the next step);
+ *   load_index[j] parent[j], except -1 where parent[j] == g*W + j or the slot is empty: the record_index of ge_state_load after
+ *                 ge_state_save of every env, so a slot that continues its own beam is not copied.
+ * A decode step is then: save every env, load with load_index, ge_step with action (a stay slot's -1 meets a done env and gets
+ * GE_STEP_AFTER_DONE with state and acc unchanged; an empty slot's gets GE_STEP_INVALID).  Deterministic (no atomics); logits of
+ * invalid actions are never read and rows are addressed with size_t.  Launched like ge_sample_logits: under GE_FLAG_PDL it may
+ * start under the previous step's tail and touches nothing before that step completes.  No synchronisation or allocation: it can
+ * be captured in a CUDA graph.  GE_ERR_ARG, before any CUDA call, for an unknown dtype, W outside [1, 32], B % W != 0, a NULL
+ * pointer (batch->mask_bits and batch->done included), or overlapping score / score_out / parent / action / load_index. */
+int ge_beam_expand(const ge_batch *batch, int W, const void *logits, int dtype, const float *score, float *score_out,
+                   int32_t *parent, int32_t *action, int32_t *load_index, void *stream);
 
 /* ---- Branching: per-env state records and instance replication (csrc/ge_state.cu) ----
  *
