@@ -40,11 +40,7 @@ def build(force=False, verbose=False):
     bdir = os.path.join(_PKG, "_build")
     os.makedirs(bdir, exist_ok=True)
     flags = [f for f in NVCC_FLAGS if f != "-shared"]
-    extra = os.environ.get("GE_NVCC_DEFS", "").split()      # e.g. GE_NVCC_DEFS="-DGE_INCR_MINB=6" for tuning experiments
-    if os.environ.get("GE_KNOBS"):                          # diagnostic build for profiles/knobs.py
-        extra.append("-DGE_KNOBS")
-    if verbose:
-        extra.append("-Xptxas=-v")
+    extra = ["-Xptxas=-v"] if verbose else []
     tag = os.path.join(bdir, "flags.txt")
     flag_sig = " ".join(flags + extra)
     same_flags = os.path.exists(tag) and open(tag).read() == flag_sig
@@ -84,9 +80,9 @@ class GeBatch(C.Structure):
         ("max_distance", C.c_double),
         ("row_ptr", _P), ("col", _P), ("w32", _P), ("w64", _P), ("adj_bits", _P), ("rev", _P), ("esrc", _P), ("wsort", _P), ("wcode", _P), ("dfa", _P), ("dc_edges", _P), ("wmin", _P), ("wmat", _P),
         ("src", _P), ("dest", _P), ("target_bits", _P), ("node_cost", _P), ("node_xy", _P),
-        ("max_dist32", _P), ("targets", _P), ("in_range", _P), ("in_range_t", _P), ("heuristic", _P), ("heuristic_alt", _P), ("features", _P),
+        ("max_dist32", _P), ("targets", _P), ("in_range", _P), ("heuristic", _P), ("heuristic_alt", _P), ("features", _P),
         ("head", _P), ("node_bits", _P), ("node_bits2", _P), ("edge_bits", _P), ("dist32", _P), ("bestkey", _P),
-        ("cost", _P), ("counters", _P), ("done", _P), ("mask_bits", _P), ("mask_cnt", _P), ("mask_bytes", _P), ("mask_mirror", _P), ("mask0_bits", _P), ("acc", _P), ("traj", _P), ("env_steps", _P), ("obs_x", _P), ("dc_rows", _P), ("progress", _P),
+        ("cost", _P), ("counters", _P), ("done", _P), ("mask_bits", _P), ("mask_cnt", _P), ("mask_bytes", _P), ("mask0_bits", _P), ("acc", _P), ("traj", _P), ("env_steps", _P), ("obs_x", _P), ("dc_rows", _P), ("progress", _P),
     ]
 
 
@@ -97,7 +93,7 @@ class StepOut(C.Structure):
 EXPORTS = ["ge_abi_version", "ge_last_error", "ge_fill_layout", "ge_step_smem_bytes", "ge_build_adjacency",
            "ge_prepare", "ge_features", "ge_generate", "ge_generate_fallbacks", "ge_pool_refill", "ge_reset", "ge_step", "ge_step_sampled", "ge_sample_actions", "ge_obs_len",
            "ge_obs_flat", "ge_obs_graph", "ge_obs_nodes", "ge_step_kernel_name", "ge_batch_slice", "ge_step_host", "ge_step_host_pipelined", "ge_step_host_compact", "ge_progress_supported",
-           "ge_step_host_release", "ge_mask_mirror_supported", "ge_mask_bytes_current", "ge_mask_bytes", "ge_stats",
+           "ge_step_host_release", "ge_mask_bytes_current", "ge_mask_bytes", "ge_stats",
            "ge_sample_logits", "ge_masked_log_prob", "ge_masked_log_prob_backward", "ge_beam_expand",
            "ge_state_record_bytes", "ge_state_save", "ge_state_load", "ge_gather_instances"]
 
@@ -139,15 +135,14 @@ def lib():
     L.ge_obs_flat.argtypes = [BP, C.c_int, C.c_int, _P, _P]
     L.ge_obs_graph.argtypes = [BP, C.c_int, C.c_int, _P, _P, _P, _P]
     L.ge_step_host.argtypes = [BP, _P, _P, C.POINTER(StepOut), _P, _P, _P, _P, _P, _P]
-    L.ge_step_host_pipelined.argtypes = [BP, _P, _P, C.POINTER(StepOut), _P, _P, _P, _P, C.c_int, _P]
-    L.ge_step_host_compact.argtypes = [BP, _P, _P, C.POINTER(StepOut), _P, _P, _P, _P, C.c_int, _P]
+    L.ge_step_host_pipelined.argtypes = [BP, _P, C.POINTER(StepOut), _P, _P, _P, _P, C.c_int, _P]
+    L.ge_step_host_compact.argtypes = [BP, _P, C.POINTER(StepOut), _P, _P, _P, _P, C.c_int, _P]
     L.ge_step_host_release.argtypes = [BP]
     L.ge_obs_nodes.argtypes = [BP, C.c_int, C.c_int, _P, _P]
     L.ge_step_kernel_name.argtypes = [BP, C.c_int]
     L.ge_step_kernel_name.restype = C.c_char_p
     L.ge_batch_slice.argtypes = [BP, C.c_int, C.c_int, BP]
     L.ge_stats.argtypes = [BP, _P, _P]
-    L.ge_mask_mirror_supported.argtypes = [BP]
     L.ge_mask_bytes_current.argtypes = [BP]
     L.ge_mask_bytes.argtypes = [BP, C.c_int, C.c_int, _P]
     L.ge_sample_logits.argtypes = [BP, _P, C.c_int, C.c_int, C.c_uint64, C.c_uint32, _P, _P, _P, _P]
@@ -158,7 +153,7 @@ def lib():
     L.ge_state_save.argtypes = [BP, _P, C.c_int, _P, _P]
     L.ge_state_load.argtypes = [BP, _P, C.c_int, _P, C.c_uint, _P]
     L.ge_gather_instances.argtypes = [BP, BP, _P, _P]
-    if L.ge_abi_version() != 3:
+    if L.ge_abi_version() != 4:
         raise NativeError("ABI version mismatch")
     _lib = L
     return L

@@ -7,7 +7,6 @@ All state tensors are torch tensors on the device and are exposed as zero-copy v
 """
 import ctypes as C
 import math
-import os
 
 import numpy as np
 import torch
@@ -40,7 +39,7 @@ class EnvStates:
 
 class BatchedGraphEnv:
     def __init__(self, env_id, num_envs, n_nodes, n_edges=-1, *, device=None, byte_mask=True, auto_reset=False,
-                 structural_features=False, env_id0=0, keep_w64=True, force_warp=False, dc_transposed=False, dc_rows=True, **kwargs):
+                 structural_features=False, env_id0=0, keep_w64=True, force_warp=False, **kwargs):
         self.lib = _native.lib()  # raises when the CUDA library is absent -- no fallback
         if not torch.cuda.is_available():
             raise _native.NativeError("graphenvs_b200 needs a CUDA device (sm_100a); there is no CPU path")
@@ -53,7 +52,6 @@ class BatchedGraphEnv:
         self.M = 2 * self.E
         self.is_eval_env = bool(P.get("is_eval_env", False))
         self.structural_features = bool(structural_features)
-        self._dc_rows = bool(dc_rows) and os.environ.get("GE_DC_ROWS", "1") != "0"   # (GE_DC_ROWS=0: A/B runs)  DistributionCenter: fixed-stride copy of the weight-sorted rows (64 KB per env at N=500)
         d = _native.GeBatch()
         d.kind, d.B, d.N, d.M = self.spec.kind, self.B, self.N, self.M
         d.parenting = int(P.get("parenting", -1))
@@ -120,10 +118,6 @@ class BatchedGraphEnv:
         if env_id == "DistributionCenter-v0":
             T["targets"] = z((B, max(d.n_targets, 1)), torch.int32)
             T["in_range"] = z((B, max(d.n_targets, 1), d.NW), torch.int32)
-            if (dc_transposed or os.environ.get("GE_DC_TRANSPOSED") == "1") and 0 < d.n_targets <= 128 and N <= 1024 and not force_warp and int(P.get("parenting", 2)) == 2:
-                # transposed table (per node the targets that have it in range): an alternative mask build measured
-                # equal in time with 16 % more HBM traffic at config 5, hence off by default (DESIGN.md 6b)
-                T["in_range_t"] = z((B, N, 4), torch.int32)
         T["heuristic"] = z((B,), torch.float64)
         self.heuristic_device_name = None
         if self.is_eval_env:
@@ -163,7 +157,7 @@ class BatchedGraphEnv:
 
     def like(self, num_envs, **overrides):
         """A new batch of `num_envs` envs, nothing loaded yet, with this batch's env id, parameters and engine options (device,
-        byte_mask, auto_reset, structural_features, env_id0, keep_w64, force_warp, dc_rows, dc_transposed); `overrides` replace
+        byte_mask, auto_reset, structural_features, env_id0, keep_w64, force_warp); `overrides` replace
         any of them.  Fill it with gather_instances(), e.g. the wide batch of a multi-start decoder."""
         P = {k: v for k, v in self.params.items() if k in dict(self.spec.defaults)}   # ctor kwargs only, not derived values
         P.pop("structural_features", None)          # ShortestPath's ignored ctor kwarg (shortest_path.py:23) vs the engine's own flag
@@ -171,7 +165,7 @@ class BatchedGraphEnv:
         d = self.desc
         opts = dict(device=self.device, byte_mask="mask_bytes" in self.t, auto_reset=bool(d.flags & 1),
                     structural_features=self.structural_features, env_id0=d.env_id0, keep_w64="w64" in self.t,
-                    force_warp=bool(d.flags & 8), dc_rows=self._dc_rows, dc_transposed="in_range_t" in self.t)
+                    force_warp=bool(d.flags & 8))
         opts.update(P)
         opts.update(overrides)
         return BatchedGraphEnv(self.env_id, num_envs, n_nodes, n_edges, **opts)
@@ -179,7 +173,7 @@ class BatchedGraphEnv:
     # ------------------------------------------------------------------ plumbing
     def _sync_desc(self):
         for name in ("row_ptr", "col", "w32", "w64", "adj_bits", "rev", "esrc", "bestkey", "wsort", "wcode", "dfa", "dc_edges", "dc_rows", "wmin", "wmat", "src", "dest", "target_bits", "node_cost", "node_xy",
-                     "max_dist32", "targets", "in_range", "in_range_t", "heuristic", "heuristic_alt", "features", "head", "node_bits", "node_bits2",
+                     "max_dist32", "targets", "in_range", "heuristic", "heuristic_alt", "features", "head", "node_bits", "node_bits2",
                      "edge_bits", "dist32", "cost", "counters", "done", "mask_bits", "mask_cnt", "mask_bytes", "mask0_bits", "acc", "traj"):
             t = self.t.get(name)
             setattr(self.desc, name, t.data_ptr() if t is not None else None)
@@ -370,8 +364,7 @@ class BatchedGraphEnv:
         T["dfa"] = torch.from_numpy(np.concatenate([np.array([S, W], dtype=np.uint8), tab.ravel(), expand, cmax])).to(self.device)
         if self.N <= 1024 and self.N < 65536:
             T["dc_edges"] = torch.zeros((B, d.MP), dtype=torch.int32, device=self.device)   # weight-sorted rows for csrc/ge_dc.cu
-            if self._dc_rows:                                                                # the same rows at a fixed 128-byte stride
-                T["dc_rows"] = torch.zeros((B, self.N, 32), dtype=torch.int32, device=self.device)
+            T["dc_rows"] = torch.zeros((B, self.N, 32), dtype=torch.int32, device=self.device)  # their first 32 entries at a fixed 128-byte stride (64 KB per env at N=500)
         self._sync_desc()
         self.desc.dfa_bytes = int(T["dfa"].numel())
         return True
@@ -514,22 +507,6 @@ class BatchedGraphEnv:
         return (blk, blk[:4 * B].view(torch.float32), blk[4 * Bp:4 * Bp + 4 * B].view(B, 4),
                 blk[8 * Bp:8 * Bp + 8 * B].view(torch.float64), blk[16 * Bp:].view(torch.int32).view(B, AW))
 
-    def enable_zero_copy(self, h_mask_bits):
-        """Mirror every packed-mask write into `h_mask_bits` (pinned host memory, e.g. from host_io()).  Returns
-        False for the incremental-mask kinds, whose mask then comes back with one copy in step_host_direct()."""
-        ok = bool(self.lib.ge_mask_mirror_supported(C.byref(self.desc)))
-        if ok:
-            self._mirror_keep = h_mask_bits
-            self.desc.mask_mirror = h_mask_bits.data_ptr()
-            h_mask_bits.copy_(self.t["mask_bits"])
-        return ok
-
-    def step_host_direct(self, h_actions, h_reward, h_flags, h_cost, h_mask_bits=None):
-        """Zero-copy end-to-end step: the kernel reads the pinned actions and writes reward / flags /
-        solution_cost (/ packed mask) straight into pinned host memory; one launch + one sync."""
-        _native.check(self.lib.ge_step_host(C.byref(self.desc), _ptr(h_actions), None, C.byref(self._out), _ptr(h_reward),
-                                            _ptr(h_flags), _ptr(h_cost), None, _ptr(h_mask_bits), self._stream()))
-
     def host_io_compact(self):
         """Pinned host buffers of the COMPACT result format (ge_step_host_compact): reward f32[B], flags8 u8[B], solution_cost f32[B],
         mask_bits i32[B, AW].  unpack_flags8() decodes the flag byte."""
@@ -563,7 +540,7 @@ class BatchedGraphEnv:
         if compact:   # flags as one byte per env, solution_cost as float32 (host_io_compact() buffers)
             assert pipelined and st.cuda_stream != 0 and h_mask is None and h_flags.dtype == torch.uint8 and h_cost.dtype == torch.float32
         if pipelined and st.cuda_stream != 0 and h_mask is None:
-            args = (C.byref(self.desc), _ptr(h_actions), _ptr(self.actions_dev), C.byref(self._out), _ptr(h_reward), _ptr(h_flags),
+            args = (C.byref(self.desc), _ptr(h_actions), C.byref(self._out), _ptr(h_reward), _ptr(h_flags),
                     _ptr(h_cost), _ptr(h_mask_bits), int(chunks), C.c_void_p(st.cuda_stream))
             fn = self.lib.ge_step_host_compact if compact else self.lib.ge_step_host_pipelined
         else:
@@ -762,7 +739,6 @@ class BatchedGraphEnv:
         T["wcode"] = torch.zeros((B, MP), dtype=torch.uint8, device=self.device)
         if "dc_edges" in src.t:
             T["dc_edges"] = torch.zeros((B, MP), dtype=torch.int32, device=self.device)
-        if "dc_rows" in src.t and self._dc_rows:
             T["dc_rows"] = torch.zeros((B, self.N, 32), dtype=torch.int32, device=self.device)
         self._sync_desc()
         self.desc.dfa_bytes = src.desc.dfa_bytes

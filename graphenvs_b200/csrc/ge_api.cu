@@ -2,7 +2,6 @@
 // See include/graphenvs_b200.h for the ABI and the reference interfaces each call replaces.
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 
@@ -548,7 +547,6 @@ bool ge_dc_eligible(const ge_batch *d);
 int ge_dc_step(const ge_batch *d, int32_t *actions, const ge_step_out *out, bool sampled, uint64_t seed, uint32_t t, cudaStream_t st);
 int ge_dc_reset(const ge_batch *d, const uint8_t *select, cudaStream_t st);
 int ge_dc_build_edges(const ge_batch *d, cudaStream_t st);
-int ge_dc_build_transposed(const ge_batch *d, cudaStream_t st);
 // PerishableProductDelivery (ge_ppd.cu)
 int ge_ppd_step(const ge_batch *d, int32_t *actions, const ge_step_out *out, bool sampled, uint64_t seed, uint32_t t, cudaStream_t st);
 int ge_ppd_reset(const ge_batch *d, const uint8_t *select, cudaStream_t st);
@@ -688,7 +686,6 @@ int ge_prepare(const ge_batch *d, int what, const double *u01, void *stream) {
         if ((rc = set_smem(prep_inrange_kernel, smem))) return rc;
         prep_inrange_kernel<<<(unsigned)((jobs + GE_WPB - 1) / GE_WPB), GE_WPB * 32, smem, st>>>(*d, wpw);
         GE_CUDA_OK(cudaGetLastError());
-        if ((rc = ge_dc_build_transposed(d, st))) return rc;
     }
     return GE_OK;
 }
@@ -728,7 +725,7 @@ static int step_impl(const ge_batch *d, int32_t *actions, const ge_step_out *out
     // (TSP / DensestSubgraph ran best at 8 / 6 blocks per SM, but they now live in the group family for N <= 1024;
     //  what is left here -- DistributionCenter, Multicast p=1, N > 1024 -- is shared-memory limited at 4.)
     // DistributionCenter on the distance automaton needs half the scratch: 6 blocks per SM fit.
-    const bool six = d->kind == GE_DISTRIBUTION_CENTER && d->wcode && d->dfa && !getenv("GE_DC_MINB4");
+    const bool six = d->kind == GE_DISTRIBUTION_CENTER && d->wcode && d->dfa;
     auto kernel = sampled ? (six ? step_kernel<true, 6> : step_kernel<true, 4>) : (six ? step_kernel<false, 6> : step_kernel<false, 4>);
     if ((rc = set_smem(kernel, smem))) return rc;
     {
@@ -804,8 +801,6 @@ int ge_obs_nodes(const ge_batch *d, int env_lo, int count, float *x, void *strea
     GE_CUDA_OK(cudaGetLastError());
     return GE_OK;
 }
-
-int ge_mask_mirror_supported(const ge_batch *d) { return d && !ge_incr_eligible(d); }   // (a sampler / obs call never mirrors)
 
 int ge_progress_supported(const ge_batch *d) {
     if (!d || d->kind == GE_PERISHABLE_DELIVERY) return 0;
@@ -898,16 +893,10 @@ HostStepGraph g_hsg[HSG_SLOTS];
 bool g_streamed_off = false;                             // set when a streamed write-back ever timed out: sliced path from then on
 int g_hsg_next = 0;
 std::mutex g_hsg_mu;
-cudaStream_t g_side[2];                                  // copy-in lane, write-back lane (the kernels stay on the caller's stream)
-cudaEvent_t g_fork, g_in[HSG_MAX_CHUNKS], g_stepped[HSG_MAX_CHUNKS], g_join;
+cudaStream_t g_side;                                     // write-back lane (the kernels stay on the caller's stream)
+cudaEvent_t g_fork, g_stepped[HSG_MAX_CHUNKS], g_join;
 bool g_side_ready = false;
 
-cudaGraphExec_t hsg_find(const ge_batch *d, const void *const *key, cudaStream_t st, int chunks) {
-    for (HostStepGraph &g : g_hsg)
-        if (g.valid && g.st == st && g.chunks == chunks && memcmp(&g.d, d, sizeof(ge_batch)) == 0 && memcmp(g.p, key, sizeof(g.p)) == 0)
-            return g.exec;
-    return nullptr;
-}
 void hsg_drop(HostStepGraph &g) {
     if (!g.valid) return;
     cudaGraphExecDestroy(g.exec);
@@ -1058,16 +1047,6 @@ __global__ void __launch_bounds__(256) writeback_stream_kernel(uint32_t *progres
 }
 }  // namespace
 
-// GE_PIPE_ZC (default on): the step kernels of ge_step_host_pipelined read the actions straight from the caller's pinned
-// host buffer (coalesced PCIe reads) and the copy-in lane disappears -- measured 59.2 -> 53.0 us per 65,536-env step at two
-// slices (profiles/r02_e2e_breakdown.jsonl); GE_PIPE_ZC=0 restores the H2D copies.  GE_HOST_SPIN=1: ge_step_host also polls
-// for completion instead of a blocking synchronize (no measurable difference on the test boxes).
-static bool env_flag(const char *name, int *cache, bool dflt = false) {
-    if (*cache < 0) { const char *e = getenv(name); *cache = e ? (e[0] != '0' ? 1 : 0) : (dflt ? 1 : 0); }
-    return *cache == 1;
-}
-static int g_pipe_zc = -1, g_host_spin = -1;
-
 int ge_batch_slice(const ge_batch *d, int lo, int count, ge_batch *o) {
     if (!d || !o) return fail(GE_ERR_ARG, "null batch");
     if (lo < 0 || count <= 0 || lo + count > d->B || (lo & 31)) return fail(GE_ERR_ARG, "bad slice [%d, %d) of %d envs (lo must be a multiple of 32)", lo, lo + count, d->B);
@@ -1080,9 +1059,9 @@ int ge_batch_slice(const ge_batch *d, int lo, int count, ge_batch *o) {
     if (d->adj_bits) o->adj_bits = d->adj_bits + (adj_tiled(*d) ? (b >> 5) * (size_t)d->N * 32 * d->NW : b * (size_t)d->ADJS);
     ADV(rev, d->MP); ADV(esrc, d->MP); ADV(wsort, d->MP); ADV(wcode, d->MP); ADV(dc_edges, d->MP); ADV(wmin, 1); ADV(wmat, (size_t)d->N * d->N);
     ADV(src, 1); ADV(dest, 1); ADV(target_bits, d->NW); ADV(node_cost, d->N); ADV(node_xy, 2 * d->N); ADV(max_dist32, 1);
-    ADV(targets, d->n_targets); ADV(in_range, (size_t)d->n_targets * d->NW); ADV(in_range_t, 4 * (size_t)d->N); ADV(heuristic, 1); ADV(heuristic_alt, 1); ADV(features, 5 * d->N);
+    ADV(targets, d->n_targets); ADV(in_range, (size_t)d->n_targets * d->NW); ADV(heuristic, 1); ADV(heuristic_alt, 1); ADV(features, 5 * d->N);
     ADV(head, 1); ADV(node_bits, d->NW); ADV(node_bits2, d->NW); ADV(edge_bits, d->MW); ADV(dist32, d->N); ADV(bestkey, d->N);
-    ADV(cost, 1); ADV(counters, 4); ADV(done, 1); ADV(mask_bits, d->AW); ADV(mask_cnt, 8); ADV(mask_bytes, d->AP); ADV(mask_mirror, d->AW);
+    ADV(cost, 1); ADV(counters, 4); ADV(done, 1); ADV(mask_bits, d->AW); ADV(mask_cnt, 8); ADV(mask_bytes, d->AP);
     ADV(mask0_bits, d->AW); ADV(acc, 1); ADV(traj, 1); ADV(env_steps, 1);
     ADV(dc_rows, (size_t)d->N * 32);
     ADV(obs_x, ge_obs_len(d) - (size_t)(is_edge_kind(d->kind) ? 4 : 3) * d->M);   // N * F floats per env
@@ -1103,36 +1082,19 @@ int ge_step_host(const ge_batch *d, const int32_t *h_actions, int32_t *d_actions
     GE_NVTX("ge_step_host");
     cudaStream_t st = (cudaStream_t)stream;
     if (!d) return fail(GE_ERR_ARG, "null batch");
-    const size_t B = (size_t)d->B;
-    if (!d_actions) {  // zero-copy: the kernel reads/writes the pinned host buffers itself
-        if (!h_actions || !h_reward || !h_flags || !h_solution_cost) return fail(GE_ERR_ARG, "zero-copy step needs all host buffers");
-        ge_step_out direct = {h_reward, h_flags, h_solution_cost};
-        int rc0 = ge_step(d, h_actions, &direct, stream);
-        if (rc0) return rc0;
-        if (h_mask_bits && !(d->mask_mirror == h_mask_bits && ge_mask_mirror_supported(d)))
-            GE_CUDA_OK(cudaMemcpyAsync(h_mask_bits, d->mask_bits, sizeof(uint32_t) * B * d->AW, cudaMemcpyDeviceToHost, st));
-        if (h_mask) {
-            if (!d->mask_bytes) return fail(GE_ERR_ARG, "byte mask not enabled");
-            if (!ge_mask_bytes_current(d) && (rc0 = ge_mask_bytes(d, 0, d->B, stream))) return rc0;
-            GE_CUDA_OK(cudaMemcpyAsync(h_mask, d->mask_bytes, B * d->AP, cudaMemcpyDeviceToHost, st));
-        }
-        GE_CUDA_OK(cudaStreamSynchronize(st));
-        return GE_OK;
-    }
-    if (!out) return fail(GE_ERR_ARG, "null step buffers");
+    if (!d_actions || !out) return fail(GE_ERR_ARG, "null step buffers");
     const void *key[10] = {h_actions, d_actions, out->reward, out->flags, out->solution_cost, h_reward, h_flags, h_solution_cost, h_mask,
                            h_mask_bits};
-    const bool capturable = st != nullptr && st != cudaStreamLegacy && st != cudaStreamPerThread && !getenv("GE_NO_HOST_GRAPH");
+    const bool capturable = st != nullptr && st != cudaStreamLegacy && st != cudaStreamPerThread;
     if (capturable) {
-        cudaGraphExec_t exec;
+        cudaGraphExec_t exec = nullptr;
         {
             std::lock_guard<std::mutex> lock(g_hsg_mu);
-            exec = hsg_find(d, key, st, 0);
+            if (HostStepGraph *g = hsg_entry(d, key, st, 0)) exec = g->exec;
         }
         if (exec) {
             GE_CUDA_OK(cudaGraphLaunch(exec, st));
-            if (env_flag("GE_HOST_SPIN", &g_host_spin)) GE_CUDA_OK(spin_until_done(st));
-            else GE_CUDA_OK(cudaStreamSynchronize(st));
+            GE_CUDA_OK(cudaStreamSynchronize(st));
             return GE_OK;
         }
         // first call for this (descriptor, buffers, stream): run once directly (also sets kernel attributes), then capture
@@ -1162,21 +1124,18 @@ int ge_step_host(const ge_batch *d, const int32_t *h_actions, int32_t *d_actions
     return GE_OK;
 }
 
-// The three stages of one slice of the pipelined step (enqueue only).
-static int pipelined_copy_in(const ge_batch *d, int lo, int n, const int32_t *h_actions, int32_t *d_actions, cudaStream_t s) {
-    GE_CUDA_OK(cudaMemcpyAsync(d_actions + lo, h_actions + lo, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, s));
-    return GE_OK;
-}
-static int g_pipe_pdl = -1;
-static int pipelined_step(const ge_batch *d, int lo, int n, const int32_t *d_actions, const ge_step_out *out, cudaStream_t s) {
+// The two stages of one slice of the pipelined step (enqueue only).  The step kernels read the actions straight from the
+// caller's pinned host buffer (coalesced PCIe reads): measured 59.2 -> 53.0 us per 65,536-env step at two slices against
+// H2D copies on a lane of their own (profiles/r02_e2e_breakdown.jsonl).
+static int pipelined_step(const ge_batch *d, int lo, int n, const int32_t *h_actions, const ge_step_out *out, cudaStream_t s) {
     ge_batch sl;
     int rc = ge_batch_slice(d, lo, n, &sl);
     if (rc) return rc;
     // slices after the first follow another slice's step kernel on this stream (different envs): programmatic dependent launch
-    // lets them become resident under its tail (GE_PIPE_PDL=0 switches it off)
-    if (lo > 0 && env_flag("GE_PIPE_PDL", &g_pipe_pdl, true)) sl.flags |= GE_FLAG_PDL;
+    // lets them become resident under its tail
+    if (lo > 0) sl.flags |= GE_FLAG_PDL;
     ge_step_out so = {out->reward + lo, out->flags + lo, out->solution_cost + lo};
-    return ge_step(&sl, d_actions + lo, &so, (void *)s);
+    return ge_step(&sl, h_actions + lo, &so, (void *)s);
 }
 static int pipelined_write_back(const ge_batch *d, int lo, int n, const ge_step_out *out, float *h_reward, void *h_flags,
                                 void *h_solution_cost, uint32_t *h_mask_bits, bool compact, cudaStream_t s) {
@@ -1200,38 +1159,34 @@ static int pipelined_write_back(const ge_batch *d, int lo, int n, const ge_step_
     return GE_OK;
 }
 
-static int step_host_pipelined_impl(const ge_batch *d, const int32_t *h_actions, int32_t *d_actions, const ge_step_out *out, float *h_reward,
+static int step_host_pipelined_impl(const ge_batch *d, const int32_t *h_actions, const ge_step_out *out, float *h_reward,
                                     void *h_flags, void *h_solution_cost, uint32_t *h_mask_bits, int chunks, bool compact, void *stream);
 
-int ge_step_host_pipelined(const ge_batch *d, const int32_t *h_actions, int32_t *d_actions, const ge_step_out *out, float *h_reward,
+int ge_step_host_pipelined(const ge_batch *d, const int32_t *h_actions, const ge_step_out *out, float *h_reward,
                            ge_step_flags *h_flags, double *h_solution_cost, uint32_t *h_mask_bits, int chunks, void *stream) {
     GE_NVTX("ge_step_host_pipelined");
-    return step_host_pipelined_impl(d, h_actions, d_actions, out, h_reward, h_flags, h_solution_cost, h_mask_bits, chunks, false, stream);
+    return step_host_pipelined_impl(d, h_actions, out, h_reward, h_flags, h_solution_cost, h_mask_bits, chunks, false, stream);
 }
 
-int ge_step_host_compact(const ge_batch *d, const int32_t *h_actions, int32_t *d_actions, const ge_step_out *out, float *h_reward,
+int ge_step_host_compact(const ge_batch *d, const int32_t *h_actions, const ge_step_out *out, float *h_reward,
                          uint8_t *h_flags8, float *h_solution_cost32, uint32_t *h_mask_bits, int chunks, void *stream) {
     GE_NVTX("ge_step_host_compact");
-    return step_host_pipelined_impl(d, h_actions, d_actions, out, h_reward, h_flags8, h_solution_cost32, h_mask_bits, chunks, true, stream);
+    return step_host_pipelined_impl(d, h_actions, out, h_reward, h_flags8, h_solution_cost32, h_mask_bits, chunks, true, stream);
 }
 
 static int ensure_side_streams() {   // (g_hsg_mu held)
     if (g_side_ready) return GE_OK;
-    for (int i = 0; i < 2; ++i) GE_CUDA_OK(cudaStreamCreateWithFlags(&g_side[i], cudaStreamNonBlocking));
-    for (int i = 0; i < HSG_MAX_CHUNKS; ++i) {
-        GE_CUDA_OK(cudaEventCreateWithFlags(&g_in[i], cudaEventDisableTiming));
-        GE_CUDA_OK(cudaEventCreateWithFlags(&g_stepped[i], cudaEventDisableTiming));
-    }
+    GE_CUDA_OK(cudaStreamCreateWithFlags(&g_side, cudaStreamNonBlocking));
+    for (int i = 0; i < HSG_MAX_CHUNKS; ++i) GE_CUDA_OK(cudaEventCreateWithFlags(&g_stepped[i], cudaEventDisableTiming));
     GE_CUDA_OK(cudaEventCreateWithFlags(&g_fork, cudaEventDisableTiming));
     GE_CUDA_OK(cudaEventCreateWithFlags(&g_join, cudaEventDisableTiming));
     g_side_ready = true;
     return GE_OK;
 }
 
-// chunks = 0: one full-batch step kernel that signals ge_batch.progress + the concurrent writer.  Zero-copy action reads.
-static int step_host_streamed(const ge_batch *d, const int32_t *h_actions, int32_t *d_actions, const ge_step_out *out, float *h_reward,
+// chunks = 0: one full-batch step kernel that signals ge_batch.progress + the concurrent writer.
+static int step_host_streamed(const ge_batch *d, const void *const *key, const int32_t *h_actions, const ge_step_out *out, float *h_reward,
                               void *h_flags, void *h_solution_cost, uint32_t *h_mask_bits, bool compact, cudaStream_t st) {
-    const void *key[10] = {h_actions, d_actions, out->reward, out->flags, out->solution_cost, h_reward, h_flags, h_solution_cost, nullptr, h_mask_bits};
     const int code = 0x200 | (compact ? 0x100 : 0);
     const int n_chunks = (d->B + (1 << GE_PROGRESS_SHIFT) - 1) >> GE_PROGRESS_SHIFT;
     cudaGraphExec_t exec = nullptr;
@@ -1272,7 +1227,7 @@ static int step_host_streamed(const ge_batch *d, const int32_t *h_actions, int32
     cudaGraph_t graph = nullptr;
     bool inserted = false;
     if (cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
-        cudaStream_t s_out = g_side[1];
+        cudaStream_t s_out = g_side;
         bool ok = cudaEventRecord(g_fork, st) == cudaSuccess && cudaStreamWaitEvent(s_out, g_fork, 0) == cudaSuccess;
         int nb = n_chunks < 32 ? n_chunks : 32;
         writeback_stream_kernel<<<nb, 256, 0, s_out>>>(progress, n_chunks, d->B, out->reward, out->flags, out->solution_cost, d->mask_bits, h_reward,
@@ -1295,63 +1250,53 @@ static int step_host_streamed(const ge_batch *d, const int32_t *h_actions, int32
     return GE_OK;
 }
 
-static int step_host_pipelined_impl(const ge_batch *d, const int32_t *h_actions, int32_t *d_actions, const ge_step_out *out, float *h_reward,
+static int step_host_pipelined_impl(const ge_batch *d, const int32_t *h_actions, const ge_step_out *out, float *h_reward,
                                     void *h_flags, void *h_solution_cost, uint32_t *h_mask_bits, int chunks, bool compact, void *stream) {
     cudaStream_t st = (cudaStream_t)stream;
     int rc = check_batch(d);
     if (rc) return rc;
-    if (!h_actions || !d_actions || !out || !h_reward || !h_flags) return fail(GE_ERR_ARG, "null step buffers");
+    if (!h_actions || !out || !h_reward || !h_flags) return fail(GE_ERR_ARG, "null step buffers");
     if (st == nullptr || st == cudaStreamLegacy || st == cudaStreamPerThread) return fail(GE_ERR_ARG, "ge_step_host_pipelined needs a created (capturable) stream");
+    const void *key[10] = {h_actions, out->reward, out->flags, out->solution_cost, h_reward, h_flags, h_solution_cost, h_mask_bits};
     if (chunks <= 0) {   // streamed write-back: ONE step kernel + a concurrent writer fed by ge_batch.progress (see writeback_stream_kernel)
-        static int off = -1;
-        if (off < 0) off = getenv("GE_NO_STREAMED") ? 1 : 0;
-        if (!off && !g_streamed_off && ge_progress_supported(d) && env_flag("GE_PIPE_ZC", &g_pipe_zc, true))
-            return step_host_streamed(d, h_actions, d_actions, out, h_reward, h_flags, h_solution_cost, h_mask_bits, compact, st);
+        if (!g_streamed_off && ge_progress_supported(d))
+            return step_host_streamed(d, key, h_actions, out, h_reward, h_flags, h_solution_cost, h_mask_bits, compact, st);
         chunks = 2;      // kernel family without progress counters: two slices
     }
     if (chunks > HSG_MAX_CHUNKS) chunks = HSG_MAX_CHUNKS;
     int per = ((d->B + chunks - 1) / chunks + 127) & ~127;    // slice starts are multiples of 128 envs (tiles, vector alignment)
     chunks = (d->B + per - 1) / per;
-    const void *key[10] = {h_actions, d_actions, out->reward, out->flags, out->solution_cost, h_reward, h_flags, h_solution_cost, nullptr, h_mask_bits};
-    cudaGraphExec_t exec;
+    cudaGraphExec_t exec = nullptr;
     {
         std::lock_guard<std::mutex> lock(g_hsg_mu);
-        exec = hsg_find(d, key, st, chunks | (compact ? 0x100 : 0));
+        if (HostStepGraph *g = hsg_entry(d, key, st, chunks | (compact ? 0x100 : 0))) exec = g->exec;
     }
     if (!exec) {
         // first call: one direct pass on the caller's stream (sets kernel attributes, does THIS step), then capture the
-        // three-lane sequence for the following calls
-        const bool zc = env_flag("GE_PIPE_ZC", &g_pipe_zc, true);
+        // two-lane sequence for the following calls
         // (Step kernels storing reward / flags / solution_cost / packed mask straight into the pinned host arrays -- no write-back
         //  kernels -- measured 99-111 us per 65,536-env step against 55-59 us: 4-8 byte stores per lane reach PCIe as 32-byte
         //  sectors, the write-back kernel's 16 bytes per lane as full lines.  profiles/r02_e2e_direct_writes.jsonl)
-        const int32_t *acts = zc ? h_actions : d_actions;
         for (int i = 0; i < chunks; ++i) {
             const int lo = i * per, n = (lo + per <= d->B) ? per : d->B - lo;
-            if (!zc && (rc = pipelined_copy_in(d, lo, n, h_actions, d_actions, st))) return rc;
-            if ((rc = pipelined_step(d, lo, n, acts, out, st))) return rc;
+            if ((rc = pipelined_step(d, lo, n, h_actions, out, st))) return rc;
             if ((rc = pipelined_write_back(d, lo, n, out, h_reward, h_flags, h_solution_cost, h_mask_bits, compact, st))) return rc;
         }
         GE_CUDA_OK(cudaStreamSynchronize(st));
         std::lock_guard<std::mutex> lock(g_hsg_mu);
         if ((rc = ensure_side_streams())) return rc;
-        // Three lanes: copy-in chain (g_side[0]) -> step-kernel chain (caller's stream) -> write-back chain (g_side[1]).
+        // Two lanes: step-kernel chain (caller's stream) -> write-back chain (g_side).
         // The kernels of the slices run ONE AFTER THE OTHER: launched side by side they would share the GPU, finish
         // together, and every write-back would start as late as after a single big kernel (measured: no gain).  Chained,
         // slice i's results cross PCIe while slice i+1 steps.
         cudaGraph_t graph = nullptr;
         if (cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
             int rc2 = GE_OK;
-            cudaStream_t s_in = g_side[0], s_out = g_side[1];
-            bool ok = cudaEventRecord(g_fork, st) == cudaSuccess && (zc || cudaStreamWaitEvent(s_in, g_fork, 0) == cudaSuccess) &&
-                      cudaStreamWaitEvent(s_out, g_fork, 0) == cudaSuccess;
+            cudaStream_t s_out = g_side;
+            bool ok = cudaEventRecord(g_fork, st) == cudaSuccess && cudaStreamWaitEvent(s_out, g_fork, 0) == cudaSuccess;
             for (int i = 0; ok && i < chunks && rc2 == GE_OK; ++i) {
                 const int lo = i * per, n = (lo + per <= d->B) ? per : d->B - lo;
-                if (!zc) {
-                    rc2 = pipelined_copy_in(d, lo, n, h_actions, d_actions, s_in);
-                    ok = ok && cudaEventRecord(g_in[i], s_in) == cudaSuccess && cudaStreamWaitEvent(st, g_in[i], 0) == cudaSuccess;
-                }
-                if (rc2 == GE_OK) rc2 = pipelined_step(d, lo, n, acts, out, st);
+                rc2 = pipelined_step(d, lo, n, h_actions, out, st);
                 ok = ok && cudaEventRecord(g_stepped[i], st) == cudaSuccess && cudaStreamWaitEvent(s_out, g_stepped[i], 0) == cudaSuccess;
                 if (rc2 == GE_OK) rc2 = pipelined_write_back(d, lo, n, out, h_reward, h_flags, h_solution_cost, h_mask_bits, compact, s_out);
             }

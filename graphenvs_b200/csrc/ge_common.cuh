@@ -28,15 +28,9 @@ struct GeNvtxRange {
 #define GE_FULL 0xffffffffu
 #define GE_WPB 8  // warps (= environments) per thread block
 
-// Step-kernel launch.  With GE_FLAG_PDL in the descriptor (or GE_PDL=1 in the environment, for A/B runs) the launch carries the
-// programmatic-stream-serialization attribute: the kernel may become resident while the previous launch of the stream is
-// still running; its pdl_wait() (below) is then what orders it behind that launch (include/graphenvs_b200.h: GE_FLAG_PDL).
-#include <cstdlib>
-inline bool ge_pdl_env() {
-    static int on = -1;
-    if (on < 0) { const char *e = getenv("GE_PDL"); on = (e && e[0] == '1') ? 1 : 0; }
-    return on == 1;
-}
+// Step-kernel launch.  With GE_FLAG_PDL in the descriptor the launch carries the programmatic-stream-serialization
+// attribute: the kernel may become resident while the previous launch of the stream is still running; its pdl_wait()
+// (below) is then what orders it behind that launch (include/graphenvs_b200.h: GE_FLAG_PDL).
 template <class... KArgs, class... Args>
 inline cudaError_t ge_launch_step(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, const ge_batch &d, Args... args) {
     cudaLaunchConfig_t cfg = {};
@@ -45,7 +39,7 @@ inline cudaError_t ge_launch_step(void (*kernel)(KArgs...), dim3 grid, dim3 bloc
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
-    cfg.numAttrs = ((d.flags & GE_FLAG_PDL) || ge_pdl_env()) ? 1 : 0;
+    cfg.numAttrs = (d.flags & GE_FLAG_PDL) ? 1 : 0;
     return cudaLaunchKernelEx(&cfg, kernel, d, args...);   // a failure is also left for cudaGetLastError() (the callers' *_launched() checks)
 }
 
@@ -288,7 +282,6 @@ __device__ inline int emit_mask(const ge_batch &d, int b, int lane, uint32_t *ms
         msk[w] = m;
         cnt += __popc(m);
         d.mask_bits[(size_t)b * d.AW + w] = m;
-        if (d.mask_mirror) d.mask_mirror[(size_t)b * d.AW + w] = m;
     }
     cnt = __reduce_add_sync(GE_FULL, cnt);
     if (d.mask_bytes) {

@@ -11,14 +11,12 @@
 //   * the cutoff search (find_nodes_in_range = nx single_source_dijkstra_path_length(cutoff), label-correcting on the
 //     exact automaton, see ge_common.cuh:sssp_cutoff_dfa) walks the frontier LIST with a group of 8 lanes per row, four
 //     rows per trip, over WEIGHT-SORTED rows of which only the prefix that can stay within the cutoff is visited: no
-//     scan, no owner search; the next rows' bounds are loaded one trip ahead; the automaton's tables sit in shared
+//     scan, no owner search; the next rows' first pass is loaded one trip ahead; the automaton's tables sit in shared
 //     memory (one copy per block);
 //   * distances are automaton state ids in a per-warp shared array (native 32-bit atomicMin);
 //   * the mask is the OR of the in-range rows of the still uncovered targets, rows fetched 32/L at a time by groups
 //     of L >= NW lanes, four passes in flight.
 // Bit-identical to the general family (tests run both and the oracle).
-#include <cstdlib>
-
 #include "ge_common.cuh"
 
 using namespace ge;
@@ -49,78 +47,21 @@ __device__ __forceinline__ DcScr dc_carve(uint32_t *base, const ge_batch &d) {
     return s;
 }
 
-// find_nodes_in_range(a): leaves the reached set in s.reach (shared, NW words).
+// find_nodes_in_range(a): returns the reached set in registers, lane w = word w.
 //
-// The rows are read from ge_batch.dc_edges: every row sorted by WEIGHT (code ascending), entry = col | code << 16.  A node
-// at automaton state du can only relax edges whose weight keeps the sum within the cutoff, and those form a PREFIX of its
-// weight-sorted row (cmax[du] = the largest such code; fl(dist + w) is monotone in w): with cutoff 1.0 and weights
-// 0.3..0.9 a node at distance 0.6 uses 2/7 of its edges.  Skipping the rest is exact -- they would have been looked up as
-// "beyond the cutoff" and dropped.  Eight lanes per row, four rows per trip; a row continues with another pass of eight
-// while its last lane was still inside the prefix.  (The first version walked whole rows, 16 lanes per row: 430 edge
-// visits per step where ~175 can matter; profiles/r02_dc_step_kernel_v1.md.)
-__device__ __forceinline__ void dc_cutoff_search(const ge_batch &d, const int32_t *__restrict__ rp, const uint32_t *__restrict__ edges,
-                                                 const uint8_t *tab, const uint8_t *expand, const uint8_t *cmax, int W,
-                                                 DcScr &s, int lane, int source) {
-    const int N = d.N, NW = d.NW;
-    {   // q[v] = 255
-        uint4 *q4 = reinterpret_cast<uint4 *>(s.q);
-        const uint4 f = make_uint4(255u, 255u, 255u, 255u);
-        for (int i = lane; i < (N + 3) >> 2; i += 32) q4[i] = f;      // the slice is padded to whole quads
-        if (lane < NW) { s.reach[lane] = 0; s.queued[lane] = 0; }
-    }
-    __syncwarp();
-    if (lane == 0) { s.q[source] = 0u; s.reach[source >> 5] = 1u << (source & 31); s.cur[0] = (uint16_t)source; *s.cnt = 0; }
-    __syncwarp();
-    int ncur = expand[0] ? 1 : 0;
-    const int grp = lane >> 3, gl = lane & 7;
-    uint16_t *cur = s.cur, *nxt = s.nxt;
-    while (ncur > 0) {
-        int lo = 0, hi = 0, du = 0;                                     // bounds of the first four rows
-        if (grp < ncur) { const int u = cur[grp]; lo = rp[u]; hi = rp[u + 1]; du = (int)s.q[u]; }
-        for (int i0 = 0; i0 < ncur; i0 += 4) {
-            int lo_n = 0, hi_n = 0, du_n = 0;                          // next four rows, loaded while these are relaxed
-            if (i0 + 4 + grp < ncur) { const int u = cur[i0 + 4 + grp]; lo_n = rp[u]; hi_n = rp[u + 1]; du_n = (int)s.q[u]; }
-            const uint8_t *trow = tab + du * W;
-            const uint32_t cm = hi > lo ? (uint32_t)cmax[du] : 0u;      // 255 = nothing within the cutoff (never queued, but harmless)
-            for (int e = lo + gl;; e += 8) {
-                uint32_t pk = 0xffffffffu;
-                if (e < hi) pk = edges[e];
-                const uint32_t code = pk >> 16;
-                const bool act = e < hi && cm != 255u && code <= cm;
-                if (act) {
-                    const int v = (int)(pk & 0xffffu);
-                    const uint32_t nid = trow[code];                    // state of fl(dist + w); inside the prefix => never 255
-                    if (nid < s.q[v]) {
-                        const uint32_t old = atomicMin(&s.q[v], nid);
-                        if (nid < old) {
-                            const uint32_t bit = 1u << (v & 31);
-                            if (old == 255u) atomicOr(&s.reach[v >> 5], bit);
-                            if (expand[nid] && !(atomicOr(&s.queued[v >> 5], bit) & bit)) {
-                                nxt[atomicAdd(s.cnt, 1)] = (uint16_t)v;
-                                asm volatile("prefetch.global.L2 [%0];" ::"l"(rp + v));   // next round's row bounds
-                            }
-                        }
-                    }
-                }
-                if (!__any_sync(GE_FULL, act && gl == 7)) break;        // no row filled its whole pass: every prefix is exhausted
-            }
-            lo = lo_n; hi = hi_n; du = du_n;
-        }
-        __syncwarp();
-        ncur = *s.cnt;
-        __syncwarp();
-        if (lane == 0) *s.cnt = 0;
-        if (lane < NW) s.queued[lane] = 0;
-        uint16_t *tmp = cur; cur = nxt; nxt = tmp;
-        __syncwarp();
-    }
-}
-
-// The same search over ge_batch.dc_rows: the first DC_ROW entries of every weight-sorted row at a fixed stride (128 bytes,
-// 0xffffffff-padded, code 0xffff is beyond every prefix).  No row_ptr lookup -- the row address follows from the node id, one
-// dependent memory round less per level -- sector-aligned rows, and the row's first sector is prefetched into L2 when
-// its node is queued.  The first pass of the NEXT four rows is loaded while the current four are relaxed.  A prefix longer
-// than DC_ROW entries (a node of degree > 32 whose whole row is within the cutoff) continues in the CSR copy (rp / edges).
+// A node at automaton state du can only relax edges whose weight keeps the sum within the cutoff, and those form a PREFIX
+// of its WEIGHT-sorted row (code ascending; cmax[du] = the largest such code; fl(dist + w) is monotone in w): with cutoff
+// 1.0 and weights 0.3..0.9 a node at distance 0.6 uses 2/7 of its edges.  Skipping the rest is exact -- they would have
+// been looked up as "beyond the cutoff" and dropped.  Eight lanes per row, four rows per trip; a row continues with
+// another pass of eight while its last lane was still inside the prefix.  (The first version walked whole rows, 16 lanes
+// per row: 430 edge visits per step where ~175 can matter; profiles/r02_dc_step_kernel_v1.md.)
+//
+// The rows are read from ge_batch.dc_rows: the first DC_ROW entries of every weight-sorted row (entry = col | code << 16)
+// at a fixed stride (128 bytes, 0xffffffff-padded, code 0xffff is beyond every prefix).  No row_ptr lookup -- the row
+// address follows from the node id, one dependent memory round less per level -- sector-aligned rows, and the row's first
+// sector is prefetched into L2 when its node is queued.  The first pass of the NEXT four rows is loaded while the current
+// four are relaxed.  A prefix longer than DC_ROW entries (a node of degree > 32 whose whole row is within the cutoff)
+// continues in ge_batch.dc_edges, where the same rows sit at their CSR offsets (rp).
 #define DC_ROW 32
 __device__ __forceinline__ uint32_t dc_cutoff_search_rows(const ge_batch &d, const int32_t *__restrict__ rp, const uint32_t *__restrict__ edges,
                                                       const uint32_t *__restrict__ rows, const uint8_t *tab, const uint8_t *expand,
@@ -245,46 +186,9 @@ __device__ __forceinline__ uint32_t dc_union_in_range(const ge_batch &d, int b, 
     return (lane < NW) ? acc : 0u;
 }
 
-// The same union from the TRANSPOSED table (ge_batch.in_range_t: per node v a 128-bit set of the targets that have v in
-// range): mask[v] = (tin[v] & uncovered targets) != 0.  One coalesced 16-byte load per node, no compaction of the target
-// list, no dependent row loads: 16 independent loads per lane at N=500 instead of ~50 rows of 64 bytes fetched through a
-// list (the OR of rows was 16.5 % of the instructions and 15 % of the stall samples of the step,
-// profiles/r02_dc_step_kernel_v2.md).  More bytes (8 KB instead of ~3 KB per step), fewer instructions and no chain.
-__device__ __forceinline__ uint32_t dc_union_transposed(const ge_batch &d, int b, int lane, uint32_t covw) {
-    const int N = d.N, NW = d.NW, NT = d.n_targets;
-    const int32_t *tg = d.targets + (size_t)b * NT;
-    uint32_t U[4] = {0u, 0u, 0u, 0u};                                 // uncovered targets, bit t = target t (warp-uniform)
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        const int t = 32 * k + lane;
-        int node = 0;
-        if (t < NT) node = tg[t];
-        const uint32_t cw = __shfl_sync(GE_FULL, covw, (node >> 5) & 31);
-        U[k] = __ballot_sync(GE_FULL, t < NT && !((cw >> (node & 31)) & 1u));
-    }
-    const uint4 *tin = reinterpret_cast<const uint4 *>(d.in_range_t) + (size_t)b * N;
-    uint32_t mine = 0;
-    for (int j0 = 0; j0 < NW; j0 += 4) {
-        uint4 x[4];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int v = ((j0 + k) << 5) + lane;
-            x[k] = (j0 + k < NW && v < N) ? __ldg(tin + v) : make_uint4(0u, 0u, 0u, 0u);
-        }
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const uint32_t hit = (x[k].x & U[0]) | (x[k].y & U[1]) | (x[k].z & U[2]) | (x[k].w & U[3]);
-            const uint32_t wd = __ballot_sync(GE_FULL, hit != 0u);
-            if (lane == j0 + k) mine = wd;
-        }
-    }
-    return mine;
-}
-
 __device__ __forceinline__ void dc_store_mask(const ge_batch &d, int b, int lane, uint32_t m) {
     if (lane >= d.AW) return;
     d.mask_bits[(size_t)b * d.AW + lane] = m;
-    if (d.mask_mirror) d.mask_mirror[(size_t)b * d.AW + lane] = m;
     if (d.mask_bytes) {  // the lane's 32 mask entries = two 128-bit stores
         uint4 *mb = reinterpret_cast<uint4 *>(d.mask_bytes + (size_t)b * d.AP);
 #pragma unroll
@@ -301,7 +205,7 @@ __device__ __forceinline__ void dc_store_mask(const ge_batch &d, int b, int lane
 // mask right after reset(): nothing taken, nothing covered
 __device__ __forceinline__ uint32_t dc_reset_mask(const ge_batch &d, int b, int lane, uint32_t tail, uint16_t *live) {
     if (d.parenting != 2) return tail;
-    return ((d.in_range_t && d.n_targets <= 128) ? dc_union_transposed(d, b, lane, 0u) : dc_union_in_range(d, b, lane, 0u, live)) & tail;
+    return dc_union_in_range(d, b, lane, 0u, live) & tail;
 }
 
 template <bool SAMPLED>
@@ -372,17 +276,15 @@ __global__ void __launch_bounds__(GE_WPB * 32, 6) dc_step_kernel(ge_batch d, int
         cost = (double)__fadd_rn((float)cost, w);
         float rew = -w;
         if (lane == (a >> 5)) takenw |= 1u << (a & 31);
-        uint32_t reachw;                                                          // find_nodes_in_range (:25-26,155)
-        if (d.dc_rows) reachw = dc_cutoff_search_rows(d, d.row_ptr + (size_t)b * d.RP, d.dc_edges + (size_t)b * d.MP, d.dc_rows + (size_t)b * N * DC_ROW, tab, expand, cmax, W, s, lane, a);
-        else { dc_cutoff_search(d, d.row_ptr + (size_t)b * d.RP, d.dc_edges + (size_t)b * d.MP, tab, expand, cmax, W, s, lane, a); reachw = WL ? s.reach[lane] : 0u; }
+        const uint32_t reachw =                                                   // find_nodes_in_range (:25-26,155)
+            dc_cutoff_search_rows(d, d.row_ptr + (size_t)b * d.RP, d.dc_edges + (size_t)b * d.MP, d.dc_rows + (size_t)b * N * DC_ROW, tab, expand, cmax, W, s, lane, a);
         const int gained = __reduce_add_sync(GE_FULL, __popc(reachw & ~covw & tgtw));
         covw |= reachw;
         rew += (float)gained;
         reward = (double)rew;
         __syncwarp();
         if (d.parenting == 2)
-            maskw = ((d.in_range_t && d.n_targets <= 128) ? dc_union_transposed(d, b, lane, covw)
-                                                           : dc_union_in_range(d, b, lane, covw, s.cur /* free again */)) & ~takenw & tail;
+            maskw = dc_union_in_range(d, b, lane, covw, s.cur /* free again */) & ~takenw & tail;
         else maskw = ~takenw & tail;
         if (!__any_sync(GE_FULL, (tgtw & ~covw) != 0u)) { done = 1; solved = 1; sol = cost; }
     }
@@ -473,36 +375,7 @@ __global__ void __launch_bounds__(256) dc_edges_kernel(ge_batch d) {
     }
 }
 
-// in_range_t[v] bit t = in_range[t] bit v (128 targets per node).  One warp per env.
-__global__ void __launch_bounds__(256) dc_transpose_kernel(ge_batch d) {
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int b = blockIdx.x * 8 + warp;
-    if (b >= d.B) return;
-    const int N = d.N, NW = d.NW, NT = d.n_targets;
-    uint32_t *tin = d.in_range_t + (size_t)b * N * 4;
-    for (int i = lane; i < 4 * N; i += 32) tin[i] = 0;
-    __syncwarp();
-    __threadfence_block();
-    const uint32_t *ir = d.in_range + (size_t)b * NT * NW;
-    for (int t = 0; t < NT; ++t)
-        for (int w = lane; w < NW; w += 32) {
-            uint32_t bits = ir[(size_t)t * NW + w];
-            while (bits) {
-                const int v = (w << 5) + __ffs(bits) - 1;
-                bits &= bits - 1;
-                if (v < N) atomicOr(&tin[4 * v + (t >> 5)], 1u << (t & 31));
-            }
-        }
-}
-
 }  // namespace
-
-int ge_dc_build_transposed(const ge_batch *d, cudaStream_t st) {
-    if (!d->in_range_t || !d->in_range || d->n_targets > 128) return GE_OK;
-    dc_transpose_kernel<<<(d->B + 7) / 8, 256, 0, st>>>(*d);
-    cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? GE_OK : ge_set_error(GE_ERR_CUDA, "dc_transpose_kernel launch: %s", cudaGetErrorString(e));
-}
 
 int ge_dc_build_edges(const ge_batch *d, cudaStream_t st) {
     if (!d->dc_edges || !d->wcode) return GE_OK;
@@ -514,10 +387,8 @@ int ge_dc_build_edges(const ge_batch *d, cudaStream_t st) {
 
 // ------------------------------------------------------------------ host launchers (called from ge_api.cu)
 bool ge_dc_eligible(const ge_batch *d) {
-    static int off = -1;                                   // GE_NO_DC=1: A/B runs against the general warp-per-env kernel
-    if (off < 0) off = getenv("GE_NO_DC") ? 1 : 0;
-    if (off || (d->flags & GE_FLAG_FORCE_WARP)) return false;
-    if (d->kind != GE_DISTRIBUTION_CENTER || d->N > 1024 || !d->wcode || !d->dfa || !d->dc_edges) return false;
+    if (d->flags & GE_FLAG_FORCE_WARP) return false;
+    if (d->kind != GE_DISTRIBUTION_CENTER || d->N > 1024 || !d->wcode || !d->dfa || !d->dc_edges || !d->dc_rows) return false;
     if (d->parenting == 2 && (!d->in_range || !d->targets || d->n_targets > 1024 || d->n_targets > d->N)) return false;
     return d->node_bits2 != nullptr && d->target_bits != nullptr;
 }

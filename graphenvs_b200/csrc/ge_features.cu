@@ -23,8 +23,6 @@
 // 190 us/env at TSP N=200 dense, 73 us/env at N=500) is kept as features_warp_kernel for N > 1024.
 // Sums are reassociated relative to networkx (sigma sums are integers < 2^53 => exact; delta and
 // pagerank differ by fp64 rounding, ~1e-16 relative; the tests compare at 1e-5 in float32).
-#include <cstdlib>
-
 #include "ge_common.cuh"
 
 using namespace ge;
@@ -579,7 +577,7 @@ extern "C" int ge_features(const ge_batch *d, void *stream) {
     const size_t budget = 227 * 1024;
     const int avg = N > 0 ? d->M / N : 1;
     // sparse graphs: 16-bit CSR copy in shared memory for the predecessor / successor gathers
-    bool csrp = avg <= 32 && d->M < 65536 && !getenv("GE_FEAT_NO_CSR");
+    bool csrp = avg <= 32 && d->M < 65536;
     size_t csr_bytes = csrp ? (((size_t)2 * (N + 1) + (size_t)2 * d->M + 15) & ~(size_t)15) : 0;
     if (csrp && mat_bytes + csr_bytes + 4 * (size_t)wb + 128 > budget) { csrp = false; csr_bytes = 0; }
     int W = (N + 7) / 8;                         // sources per warp >= 8 where there are that many

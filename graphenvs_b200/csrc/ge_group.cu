@@ -9,8 +9,6 @@
 // is one instruction per word, cross-word facts (popcounts, the rank of the chosen node in its adjacency
 // row) are group reductions, and a warp advances 32/G envs.  Same rules as ge_envs.cuh / ge_lane.cu
 // (same reference line map); tests run every eligible case through both families.
-#include <cstdlib>
-
 #include "ge_common.cuh"
 
 using namespace ge;
@@ -140,7 +138,6 @@ template <int G>
 __device__ __forceinline__ void store_mask_word(const ge_batch &d, int b, int lane, uint32_t m) {
     if (lane >= d.AW) return;
     d.mask_bits[(size_t)b * d.AW + lane] = m;
-    if (d.mask_mirror) d.mask_mirror[(size_t)b * d.AW + lane] = m;
     if (d.mask_bytes) {  // the lane's 32 mask entries = two 128-bit stores
         uint4 *mb = reinterpret_cast<uint4 *>(d.mask_bytes + (size_t)b * d.AP);
 #pragma unroll
@@ -366,13 +363,7 @@ bool ge_group_eligible(const ge_batch *d) {
     return d->kind == GE_DENSEST_SUBGRAPH || d->wsort != nullptr;
 }
 
-static int group_lanes(const ge_batch *d) {
-    static int forced = -1;
-    if (forced < 0) { const char *e = getenv("GE_GROUP_G"); forced = e ? atoi(e) : 0; }
-    int G = d->NW <= 8 ? 8 : d->NW <= 16 ? 16 : 32;
-    if ((forced == 8 || forced == 16 || forced == 32) && forced >= G) G = forced;
-    return G;
-}
+static int group_lanes(const ge_batch *d) { return d->NW <= 8 ? 8 : d->NW <= 16 ? 16 : 32; }
 
 static int group_launched(const char *what) {
     cudaError_t e = cudaGetLastError();

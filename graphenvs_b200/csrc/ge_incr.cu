@@ -18,8 +18,6 @@
 // on the row-set expansion (profiles/r01_step_kernel_cfg5_multicast_warp_v1.md).
 //
 // One warp per env (a CSR row is 10-20 edges: one warp iteration); MaxIndependentSet one lane per env.
-#include <cstdlib>
-
 #include "ge_common.cuh"
 
 using namespace ge;
@@ -29,11 +27,9 @@ extern "C" int ge_set_error(int code, const char *fmt, ...);
 namespace {
 
 constexpr u64 KEY_NONE = ~0ull;
-#ifndef GE_INCR_MINB
 #define GE_INCR_MINB 8  // resident blocks per SM the tree step kernel is compiled for: 32 registers => 64 warps/SM.
                         // The kernel is a chain of ~5 dependent memory rounds per env, i.e. latency-bound: measured
                         // 0.70 / 0.84 / 0.96 G env-steps/s at cfg3 for 4 / 6 / 8 blocks per SM.
-#endif
 
 // The incremental kernels keep only the PACKED mask current.  Writing the byte view as well meant one scattered 1-byte
 // store per changed edge, each a 32-byte sector read-modify-write in HBM: 2.3 KB of the 4.7 KB a Multicast step moved
@@ -419,10 +415,7 @@ int ge_incr_step(const ge_batch *d, int32_t *actions, const ge_step_out *out, bo
         return launched("incr_mis_step_kernel");
     }
     // lanes per env: wide enough to hold the node bitsets in registers (NW <= G) and a typical row in one pass
-    static int forced = -1;
-    if (forced < 0) { const char *e = getenv("GE_INCR_G"); forced = e ? atoi(e) : 0; }
-    int G = forced ? forced : (d->NW <= 8 ? 8 : d->NW <= 16 ? 16 : 32);
-    if (G != 8 && G != 16) G = 32;
+    const int G = d->NW <= 8 ? 8 : d->NW <= 16 ? 16 : 32;
     const int per_block = GE_WPB * 32 / G;
     const int blocks = (d->B + per_block - 1) / per_block;
     auto kernel = G == 8 ? (sampled ? incr_tree_step_kernel<true, 8> : incr_tree_step_kernel<false, 8>)

@@ -12,15 +12,20 @@
 //
 // Semantics are those of ge_envs.cuh (same reference line map); tests run every N <= 64 case
 // through both paths (GE_FLAG_FORCE_WARP).
-#include <cstdlib>
-
 #include "ge_common.cuh"
 
 using namespace ge;
 
 extern "C" int ge_set_error(int code, const char *fmt, ...);
 
-#define GE_LANE_T 128  // max threads (= envs) per block; the launch picks blockDim.x (multiple of 32)
+// Envs (= threads) per block: one tile.  Small blocks spread the arrival times of the staged copies, so the searches of
+// early blocks overlap the transfers of late ones (single-wave launches otherwise alternate between an
+// all-memory and an all-compute phase): 9.96 vs 10.17 us per cfg2 step under the streaming protocol; no
+// difference when a step runs alone.
+constexpr int LANE_T = 32;
+// __launch_bounds__ of the lane kernels.  It sets their register budget: with a bound of 32 the compiler gives the
+// step kernels 63 instead of 56 registers, a build nobody has measured.
+constexpr int LANE_BOUND = 128;
 
 namespace {
 
@@ -127,9 +132,6 @@ __device__ __forceinline__ u64 lane_mask(const ge_batch &d, const Rows<STAGED> &
         if (d.parenting < 2) return m;
         if ((s.vis >> dest) & 1ull) return m;                                  // dest not in alt_G (:135-136)
         u64 allowed = ~s.vis & full;
-#ifdef GE_KNOBS
-        if (d.flags & 0x100u) return m;
-#endif
         if (m) m &= reach_within(R, 1ull << dest, allowed, m);               // has_path(k, dest) for the candidates k (:137-140)
         if (d.parenting == 3 && __popcll(allowed) <= N / 3) m |= allowed;     // :141-143
         return m; }
@@ -198,13 +200,6 @@ __device__ __forceinline__ void lane_store_state(const ge_batch &d, int b, const
     // mask: packed words + bytes (AP <= 64: up to four 128-bit stores)
     if (d.AW == 1) d.mask_bits[b] = (uint32_t)mask;
     else reinterpret_cast<uint2 *>(d.mask_bits)[b] = make_uint2((uint32_t)mask, (uint32_t)(mask >> 32));
-    if (d.mask_mirror) {
-        if (d.AW == 1) d.mask_mirror[b] = (uint32_t)mask;
-        else reinterpret_cast<uint2 *>(d.mask_mirror)[b] = make_uint2((uint32_t)mask, (uint32_t)(mask >> 32));
-    }
-#ifdef GE_KNOBS
-    if (d.flags & 0x400u) return;
-#endif
     if (d.mask_bytes) {
         uint4 *mb = reinterpret_cast<uint4 *>(d.mask_bytes + (size_t)b * d.AP);
         for (int c = 0; c < (d.AP >> 4); ++c) {
@@ -239,9 +234,6 @@ __device__ __forceinline__ Rows<STAGED> stage_rows(const ge_batch &d, int b0, ui
     if (!STAGED) return R;
     if (threadIdx.x == 0) mbar_init(bar, 1);
     __syncthreads();
-#ifdef GE_KNOBS
-    if (d.flags & 0x200u) { if (threadIdx.x == 0) mbar_expect_tx(bar, 0); R.sp = smem_u32(smem + (size_t)(threadIdx.x >> 5) * tile_words + (size_t)(threadIdx.x & 31) * d.NW); return R; }
-#endif
     if (threadIdx.x == 0) {
         const int ntiles = (min((int)blockDim.x, d.B - b0) + 31) >> 5;     // adj_bits holds whole tiles (B rounded up to 32 envs)
         const uint32_t bytes = (uint32_t)(ntiles * tile_words * 4);        // a multiple of 128
@@ -263,7 +255,7 @@ __device__ __forceinline__ int lane_sample(u64 m, uint64_t seed, uint32_t env, u
 }
 
 template <bool STAGED, bool SAMPLED>
-__global__ void __launch_bounds__(GE_LANE_T) lane_step_kernel(ge_batch d, int32_t *__restrict__ actions, ge_step_out out,
+__global__ void __launch_bounds__(LANE_BOUND) lane_step_kernel(ge_batch d, int32_t *__restrict__ actions, ge_step_out out,
                                                             uint64_t seed, uint32_t t) {
     extern __shared__ __align__(128) uint32_t smem[];
     __shared__ __align__(8) uint64_t bar;
@@ -285,10 +277,6 @@ __global__ void __launch_bounds__(GE_LANE_T) lane_step_kernel(ge_batch d, int32_
     float w_node = 0.f;
     bool was_done = false;
     uint32_t nsteps = 0;
-#ifdef GE_KNOBS
-    if (d.flags & 0x1000u) { if (STAGED) mbar_wait(&bar, 0); if (live && R.row(0) == 0x1234567ull) out.reward[b] = 1.f; return; }
-    if (d.flags & 0x2000u) { return; }   // empty kernel (launch floor)
-#endif
     if (live) {
         if (!SAMPLED) a = actions[b];
         if (d.env_steps) nsteps = d.env_steps[b];
@@ -310,9 +298,6 @@ __global__ void __launch_bounds__(GE_LANE_T) lane_step_kernel(ge_batch d, int32_
         if (d.traj) cs = d.traj[b];
         // the one dependent load of the step, issued before waiting for the staged rows
         const bool needs_w = kind == GE_SHORTEST_PATH || kind == GE_LONGEST_PATH || kind == GE_TSP;
-#ifdef GE_KNOBS
-        if (!(d.flags & 0x800u))
-#endif
         if (needs_w && a >= 0 && a < N) w_edge = lane_edge_weight(d, b, s.head, a);
         if (kind == GE_MAX_INDEPENDENT_SET && a >= 0 && a < N) w_node = d.node_cost[(size_t)b * N + a];
     }
@@ -428,7 +413,7 @@ __global__ void __launch_bounds__(GE_LANE_T) lane_step_kernel(ge_batch d, int32_
 }
 
 template <bool STAGED>
-__global__ void __launch_bounds__(GE_LANE_T) lane_reset_kernel(ge_batch d, const uint8_t *__restrict__ select) {
+__global__ void __launch_bounds__(LANE_BOUND) lane_reset_kernel(ge_batch d, const uint8_t *__restrict__ select) {
     extern __shared__ __align__(128) uint32_t smem[];
     __shared__ __align__(8) uint64_t bar;
     const int b0 = blockIdx.x * blockDim.x, b = b0 + threadIdx.x;
@@ -469,46 +454,31 @@ bool ge_lane_eligible(const ge_batch *d) {
            (d->adj_bits != nullptr || d->kind == GE_MAX_INDEPENDENT_SET);
 }
 
-// Envs per block.  Blocks smaller than the maximum spread the arrival times of the staged copies, so
-// the searches of early blocks overlap the transfers of late ones (single-wave launches otherwise
-// alternate between an all-memory and an all-compute phase).  GE_LANE_T=<32|64|128> overrides.
-static int lane_threads(const ge_batch *d) {
-    static int forced = -1;
-    if (forced < 0) {
-        const char *e = getenv("GE_LANE_T");
-        forced = e ? atoi(e) : 0;
-        if (forced != 32 && forced != 64 && forced != 128) forced = 0;
-    }
-    if (forced) return forced;
-    return 32;   // one tile per block: 9.96 vs 10.17 us per cfg2 step under the streaming protocol; no difference when a step runs alone
-}
-static size_t lane_smem(const ge_batch *d, int T) { return lane_stages(*d) ? (size_t)T * d->N * d->NW * 4 : 0; }
+static size_t lane_smem(const ge_batch *d) { return lane_stages(*d) ? (size_t)LANE_T * d->N * d->NW * 4 : 0; }
 
 int ge_grant_smem(const void *kernel, size_t smem);  // ge_api.cu
 template <class K>
 static int lane_prepare(K kernel, size_t smem) { return ge_grant_smem((const void *)kernel, smem); }
 
 int ge_lane_step(const ge_batch *d, int32_t *actions, const ge_step_out *out, bool sampled, uint64_t seed, uint32_t t, cudaStream_t st) {
-    const int T = lane_threads(d);
-    size_t smem = lane_smem(d, T);
+    const size_t smem = lane_smem(d);
     const bool needs_w = d->kind == GE_SHORTEST_PATH || d->kind == GE_LONGEST_PATH || d->kind == GE_TSP;
     if (needs_w && !d->wmat) return ge_set_error(GE_ERR_ARG, "kind %d with N <= 64 needs wmat (ge_build_adjacency fills it)", d->kind);
     auto kernel = lane_stages(*d) ? (sampled ? lane_step_kernel<true, true> : lane_step_kernel<true, false>)
                                   : (sampled ? lane_step_kernel<false, true> : lane_step_kernel<false, false>);
     int rc = lane_prepare(kernel, smem);
     if (rc) return rc;
-    cudaError_t e = ge_launch_step(kernel, dim3((d->B + T - 1) / T), dim3(T), smem, st, *d, actions, *out, seed, t);
+    cudaError_t e = ge_launch_step(kernel, dim3((d->B + LANE_T - 1) / LANE_T), dim3(LANE_T), smem, st, *d, actions, *out, seed, t);
     if (e != cudaSuccess) (void)cudaGetLastError();
     return e == cudaSuccess ? GE_OK : ge_set_error(GE_ERR_CUDA, "lane_step_kernel launch: %s", cudaGetErrorString(e));
 }
 
 int ge_lane_reset(const ge_batch *d, const uint8_t *select, cudaStream_t st) {
-    const int T = lane_threads(d);
-    size_t smem = lane_smem(d, T);
+    const size_t smem = lane_smem(d);
     auto kernel = lane_stages(*d) ? lane_reset_kernel<true> : lane_reset_kernel<false>;
     int rc = lane_prepare(kernel, smem);
     if (rc) return rc;
-    kernel<<<(d->B + T - 1) / T, T, smem, st>>>(*d, select);
+    kernel<<<(d->B + LANE_T - 1) / LANE_T, LANE_T, smem, st>>>(*d, select);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? GE_OK : ge_set_error(GE_ERR_CUDA, "lane_reset_kernel launch: %s", cudaGetErrorString(e));
 }

@@ -26,7 +26,6 @@ __device__ __forceinline__ void ppd_store_mask(const ge_batch &d, int b, int lan
         uint32_t m = adj[(size_t)head * d.NW + w] & tail_mask(d.N, w);        //  when a product waits there: "pick up")
         if (waiting && w == (head >> 5)) m |= 1u << (head & 31);
         mb[w] = m;
-        if (d.mask_mirror) d.mask_mirror[(size_t)b * d.AW + w] = m;
     }
     if (d.mask_bytes) {
         __syncwarp();
@@ -244,7 +243,6 @@ __global__ void __launch_bounds__(128) ppd_lane_step_kernel(ge_batch d, int32_t 
         if (waiting) m |= 1ull << head;
         if (NW == 1) d.mask_bits[b] = (uint32_t)m;
         else { d.mask_bits[2 * (size_t)b] = (uint32_t)m; d.mask_bits[2 * (size_t)b + 1] = (uint32_t)(m >> 32); }
-        if (d.mask_mirror) { for (int w = 0; w < NW; ++w) d.mask_mirror[(size_t)b * NW + w] = (uint32_t)(m >> (32 * w)); }
         if (d.mask_bytes) {
             uint4 *mb = reinterpret_cast<uint4 *>(d.mask_bytes + (size_t)b * d.AP);
             for (int k = 0; k < (d.AP >> 4); ++k) {

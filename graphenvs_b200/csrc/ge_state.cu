@@ -10,7 +10,7 @@
 //     access, not a warp per env;
 //   - every body section (Multicast edge_bits / dist32 / bestkey / mask_bits: hundreds of bytes per env) is copied by one
 //     warp per env with the widest vector both sides allow.
-// The packed mask's byte view and host mirror are rebuilt from the loaded mask in the same launch.  Nothing here touches a
+// The packed mask's byte view is rebuilt from the loaded mask in the same launch.  Nothing here touches a
 // static array, so a load may precede a GE_FLAG_PDL step.
 #include "ge_static.cuh"
 
@@ -160,9 +160,9 @@ __global__ void __launch_bounds__(THREADS) state_save_kernel(ge_batch d, Layout 
 }
 
 // Env b <- record record_index[b] (b, when record_index is NULL); an index outside [0, n_records) leaves env b untouched.
-// Only the sections in `what` are written.  mask_bytes / mirror: rebuild the byte view / write the host mirror.
+// Only the sections in `what` are written.  mask_bytes: rebuild the byte view.
 __global__ void __launch_bounds__(THREADS) state_load_kernel(ge_batch d, Layout L, int te_max, const char *__restrict__ rec, int n_records,
-                                                             const int32_t *__restrict__ record_index, unsigned what, int mask_bytes, int mirror) {
+                                                             const int32_t *__restrict__ record_index, unsigned what, int mask_bytes) {
     extern __shared__ uint4 sh4[];
     const char *sh = reinterpret_cast<const char *>(sh4);
     __shared__ int rsel[TILE];
@@ -199,28 +199,20 @@ __global__ void __launch_bounds__(THREADS) state_load_kernel(ge_batch d, Layout 
             warp_copy(S.soa + (size_t)(b0 + e) * bytes, r + S.off, bytes, S.vec, lane);
         }
     }
-    if (!(mask_bytes | mirror) || L.mask < 0) return;
-    // the derived views of the loaded packed mask, read from the header tile or the record itself
+    if (!mask_bytes || L.mask < 0) return;
+    // the byte view of the loaded packed mask, read from the header tile or the record itself
     const Sec &Mk = L.s[L.mask];
     auto word = [&](int e, int w) -> uint32_t {
         const char *base = L.mask < L.n_head ? sh + (size_t)e * L.head : rec + (size_t)rsel[e] * L.bytes;
         return reinterpret_cast<const uint32_t *>(base + Mk.off)[w];
     };
-    if (mask_bytes) {
-        const int per = d.AP >> 4;   // 16 mask entries per 128-bit store (ge_api.cu:mask_bytes_kernel)
-        for (uint32_t k = tid; k < (uint32_t)te * per; k += THREADS) {
-            const int e = (int)(k / per), c = (int)(k % per);
-            if (rsel[e] < 0) continue;
-            const uint32_t bits = c < 2 * d.AW ? (word(e, c >> 1) >> ((c & 1) * 16)) & 0xffffu : 0u;
-            reinterpret_cast<uint4 *>(d.mask_bytes + (size_t)(b0 + e) * d.AP)[c] =
-                make_uint4(expand4(bits), expand4(bits >> 4), expand4(bits >> 8), expand4(bits >> 12));
-        }
-    }
-    if (mirror) {
-        for (uint32_t k = tid; k < (uint32_t)te * d.AW; k += THREADS) {
-            const int e = (int)(k / d.AW), w = (int)(k % d.AW);
-            if (rsel[e] >= 0) d.mask_mirror[(size_t)(b0 + e) * d.AW + w] = word(e, w);
-        }
+    const int per = d.AP >> 4;   // 16 mask entries per 128-bit store (ge_api.cu:mask_bytes_kernel)
+    for (uint32_t k = tid; k < (uint32_t)te * per; k += THREADS) {
+        const int e = (int)(k / per), c = (int)(k % per);
+        if (rsel[e] < 0) continue;
+        const uint32_t bits = c < 2 * d.AW ? (word(e, c >> 1) >> ((c & 1) * 16)) & 0xffffu : 0u;
+        reinterpret_cast<uint4 *>(d.mask_bytes + (size_t)(b0 + e) * d.AP)[c] =
+            make_uint4(expand4(bits), expand4(bits >> 4), expand4(bits >> 8), expand4(bits >> 12));
     }
 }
 
@@ -290,9 +282,8 @@ extern "C" int ge_state_load(const ge_batch *batch, const void *records, int n_r
     build_layout(*batch, L);
     const int te = tile_for(L);
     const int mb = ge_mask_bytes_current(batch) ? 1 : 0;
-    const int mirror = (batch->mask_mirror && ge_mask_mirror_supported(batch)) ? 1 : 0;
     state_load_kernel<<<(batch->B + te - 1) / te, THREADS, (size_t)te * L.head, (cudaStream_t)stream>>>(
-        *batch, L, te, reinterpret_cast<const char *>(records), n_records, record_index, what, mb, mirror);
+        *batch, L, te, reinterpret_cast<const char *>(records), n_records, record_index, what, mb);
     return launched("state_load_kernel");
 }
 

@@ -50,7 +50,7 @@ inline int static_table(const ge_batch &d, const ge_batch *srcs, int n_src, Stat
     STATIC_ADD(rev, d.MP * 4); STATIC_ADD(esrc, d.MP * 4); STATIC_ADD(wsort, d.MP * 8); STATIC_ADD(wcode, d.MP); STATIC_ADD(dc_edges, d.MP * 4); STATIC_ADD(dc_rows, (size_t)d.N * 128); STATIC_ADD(wmin, 8);
     STATIC_ADD(wmat, (size_t)d.N * d.N * 8); STATIC_ADD(src, 4); STATIC_ADD(dest, 4); STATIC_ADD(target_bits, d.NW * 4);
     STATIC_ADD(node_cost, d.N * 4); STATIC_ADD(node_xy, d.N * 8); STATIC_ADD(max_dist32, 4); STATIC_ADD(targets, d.n_targets * 4);
-    STATIC_ADD(in_range, (size_t)d.n_targets * d.NW * 4); STATIC_ADD(in_range_t, (size_t)d.N * 16); STATIC_ADD(heuristic, 8); STATIC_ADD(heuristic_alt, 8);
+    STATIC_ADD(in_range, (size_t)d.n_targets * d.NW * 4); STATIC_ADD(heuristic, 8); STATIC_ADD(heuristic_alt, 8);
     STATIC_ADD(features, d.N * 20); STATIC_ADD(mask0_bits, d.AW * 4);
 #undef STATIC_ADD
     return rc;

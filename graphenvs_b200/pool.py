@@ -23,7 +23,7 @@ class InstancePool:
         self.banks = []
         for k in range(self.G):
             # banks keep their float64 weights: a generate() without them synchronises, and banks regenerate in the background
-            b = env.like(env.B, byte_mask=False, keep_w64=True, dc_rows="dc_rows" in env.t)
+            b = env.like(env.B, byte_mask=False, keep_w64=True)
             b.generate(seed=self._next_seed(), check=False)
             if "mask0_bits" in b.t:
                 b.reset()                       # fills mask0_bits (the first mask depends only on the instance)

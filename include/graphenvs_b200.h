@@ -46,7 +46,7 @@
 extern "C" {
 #endif
 
-#define GE_ABI_VERSION 3
+#define GE_ABI_VERSION 4
 
 typedef enum {
     GE_SHORTEST_PATH = 0,      /* ShortestPath-v0        shortest_path.py        node actions */
@@ -148,8 +148,6 @@ typedef struct ge_batch {
     float *max_dist32;            /* [B]      Multicast MAX_DISTANCE column value */
     int32_t *targets;             /* [B, n_targets] DistributionCenter target node ids */
     uint32_t *in_range;           /* [B, n_targets, NW] nodes within max_distance of each target */
-    uint32_t *in_range_t;         /* [B, N, 4] the same table transposed: per node a 128-bit set of the targets that have it in
-                                              range (n_targets <= 128; derived by ge_prepare bit 2 when non-NULL), or NULL */
     double *heuristic;            /* [B]      info['heuristic_solution'] */
     double *heuristic_alt;        /* [B]      info['heuristic_device']: labelled alternative where the reference's value is defined by
                                               networkx iteration order (Steiner shortest-path heuristic, TSP nearest neighbour, greedy
@@ -175,9 +173,6 @@ typedef struct ge_batch {
                                               rewrite the whole mask; the INCREMENTAL-mask kernels (SteinerTree, Multicast p >= 2,
                                               MaxIndependentSet N > 64: ge_mask_bytes_current() == 0) update only the packed mask and
                                               the byte view is produced on demand by ge_mask_bytes */
-    uint32_t *mask_mirror;        /* [B, AW]  optional second destination of every packed-mask write, e.g. PINNED HOST memory
-                                              (zero-copy results, see ge_step_host); honoured by the kernels that rewrite
-                                              the whole mask, not by the incremental ones (ge_mask_mirror_supported) */
     uint32_t *mask0_bits;         /* [B, AW]  mask right after reset(), written by ge_reset, or NULL.  It depends only on the
                                               instance, so auto-reset inside ge_step copies it instead of recomputing it */
     double *acc;                  /* [4, acc_stride] per-env statistics: episodes, solved, sum reward, sum final cost */
@@ -189,11 +184,12 @@ typedef struct ge_batch {
     float *obs_x;                 /* [B, N, F] optional DEVICE buffer, or NULL: ge_step_host_pipelined rewrites the node columns of the
                                               observation (ge_obs_nodes; utils.py:14-23 `x`) of every slice on its write-back lane, while
                                               the next slice steps -- the dynamic part of the observation for a device-resident consumer */
-    uint32_t *dc_rows;            /* [B, N, 32] DistributionCenter with an automaton, optional (derived by ge_prepare bit 4 next to dc_edges):
-                                              the first 32 entries of every weight-sorted row at a FIXED stride of 128 bytes, padded with
-                                              0xffffffff.  The cutoff search then needs no row_ptr lookup (one dependent memory round
-                                              less per search level), reads sector-aligned rows, and prefetches a row when its node is
-                                              queued; a prefix longer than 32 entries continues in dc_edges */
+    uint32_t *dc_rows;            /* [B, N, 32] DistributionCenter with an automaton (derived by ge_prepare bit 4 next to dc_edges; the
+                                              dedicated kernel needs both, without them the batch steps in the general family): the first
+                                              32 entries of every weight-sorted row at a FIXED stride of 128 bytes, padded with 0xffffffff.
+                                              The cutoff search then needs no row_ptr lookup (one dependent memory round less per search
+                                              level), reads sector-aligned rows, and prefetches a row when its node is queued; a prefix
+                                              longer than 32 entries continues in dc_edges */
     uint32_t *progress;           /* [ceil(B / 1024)] optional DEVICE counters, or NULL: a step kernel that supports it (ge_progress_supported)
                                               adds the number of envs it has finished -- every store of those envs made visible first -- to
                                               progress[env >> 10].  ge_step_host_pipelined with chunks = 0 uses it to stream results to the host
@@ -264,34 +260,29 @@ int ge_obs_nodes(const ge_batch *batch, int env_lo, int count, float *x, void *s
 /* Name of the CUDA kernel ge_step / ge_step_sampled dispatches this descriptor to (reports, profiles). */
 const char *ge_step_kernel_name(const ge_batch *batch, int sampled);
 
-/* End-to-end entry with HOST buffers: copies actions H2D, steps, copies reward / flags /
- * solution_cost (and the byte mask [B, AP] when h_mask != NULL, the packed mask [B, AW] when
- * h_mask_bits != NULL) D2H, and synchronises the stream.  If reward | flags | solution_cost |
- * mask_bits are laid out back to back in that order on the device AND on the host (B even), the
- * results come back in one copy.
- * d_actions / out are device staging buffers owned by the caller. */
-/* ZERO-COPY mode (d_actions == NULL): h_actions / h_reward / h_flags / h_solution_cost must be pinned host
- * memory (device-accessible under UVA); the step kernel reads the actions from it and writes its results
- * to it directly over PCIe -- no copy calls, one launch, one stream sync.  The packed mask arrives the same
- * way when batch->mask_mirror == h_mask_bits and ge_mask_mirror_supported(batch), otherwise by one copy. */
-int ge_mask_mirror_supported(const ge_batch *batch);
 /* 1 when every ge_step / ge_reset leaves mask_bytes equal to the packed mask; 0 when the byte view must be refreshed with
  * ge_mask_bytes before it is read (incremental-mask kernels: a scattered byte store per changed edge was 2.3 KB of HBM
  * traffic per Multicast step against 1.8 KB of useful bytes). */
 int ge_mask_bytes_current(const ge_batch *batch);
 /* Expands the packed mask of envs [env_lo, env_lo + count) into mask_bytes (one coalesced pass). */
 int ge_mask_bytes(const ge_batch *batch, int env_lo, int count, void *stream);
+/* End-to-end entry with HOST buffers: copies actions H2D, steps, copies reward / flags /
+ * solution_cost (and the byte mask [B, AP] when h_mask != NULL, the packed mask [B, AW] when
+ * h_mask_bits != NULL) D2H, and synchronises the stream.  If reward | flags | solution_cost |
+ * mask_bits are laid out back to back in that order on the device AND on the host (B even), the
+ * results come back in one copy.
+ * d_actions / out are device staging buffers owned by the caller (GE_ERR_ARG when NULL). */
 int ge_step_host(const ge_batch *batch, const int32_t *h_actions, int32_t *d_actions, const ge_step_out *out,
                  float *h_reward, ge_step_flags *h_flags, double *h_solution_cost, uint8_t *h_mask,
                  uint32_t *h_mask_bits, void *stream);
 
 /* PIPELINED end-to-end step with pinned (device-mapped) HOST buffers.  The batch is cut into `chunks` slices; each slice
- * runs copy-in -> step kernel -> write-back on its own branch of ONE CUDA graph, so slice i's results cross PCIe while
- * slice i+1 is stepping and slice i+2's actions arrive.  Results are written back by a small copy kernel straight into
- * the caller's four host arrays (coalesced 128-byte PCIe writes; no staging layout imposed on the host side), and the step
- * kernels read the actions straight from h_actions (zero-copy; GE_PIPE_ZC=0 copies them to d_actions first).  Blocks
- * until the results are visible to the host (spin on stream completion).  h_solution_cost / h_mask_bits may be NULL. */
-int ge_step_host_pipelined(const ge_batch *batch, const int32_t *h_actions, int32_t *d_actions, const ge_step_out *out,
+ * runs step kernel -> write-back on its own branch of ONE CUDA graph, so slice i's results cross PCIe while slice i+1 is
+ * stepping.  The step kernels read the actions straight from h_actions (zero-copy), and results are written back by a small
+ * copy kernel straight into the caller's four host arrays (coalesced 128-byte PCIe writes; no staging layout imposed on the
+ * host side).  Blocks until the results are visible to the host (spin on stream completion).  h_solution_cost / h_mask_bits
+ * may be NULL. */
+int ge_step_host_pipelined(const ge_batch *batch, const int32_t *h_actions, const ge_step_out *out,
                            float *h_reward, ge_step_flags *h_flags, double *h_solution_cost, uint32_t *h_mask_bits,
                            int chunks, void *stream);
 /* ge_step_host_pipelined with COMPACT host results: 9 instead of 16 bytes per env next to the packed mask (PCIe write time is what a
@@ -302,7 +293,7 @@ int ge_step_host_pipelined(const ge_batch *batch, const int32_t *h_actions, int3
 #define GE_FLAGS8_SOLVED(f) ((int)(((f) >> 1) & 3) - 1)
 #define GE_FLAGS8_STATUS(f) (((f) >> 3) & 3)
 #define GE_FLAGS8_HAS_MASK(f) (((f) >> 5) & 1)
-int ge_step_host_compact(const ge_batch *batch, const int32_t *h_actions, int32_t *d_actions, const ge_step_out *out,
+int ge_step_host_compact(const ge_batch *batch, const int32_t *h_actions, const ge_step_out *out,
                          float *h_reward, uint8_t *h_flags8, float *h_solution_cost32, uint32_t *h_mask_bits, int chunks, void *stream);
 /* 1 when the step kernel this batch dispatches to signals ge_batch.progress (the lane-per-env families, DistributionCenter). */
 int ge_progress_supported(const ge_batch *batch);
@@ -401,9 +392,8 @@ int ge_state_record_bytes(const ge_batch *batch);
 int ge_state_save(const ge_batch *batch, const int32_t *env_index, int count, void *records, void *stream);
 /* For each b in [0, B): env b <- record record_index[b] (record b when record_index is NULL, which requires n_records >= B).  An
  * index < 0 or >= n_records leaves env b untouched, byte for byte.  Only the sections named in `what` are written, and `what` must
- * include GE_STATE_DYNAMIC.  A loaded env's mask_bytes is rebuilt when ge_mask_bytes_current(batch), and its mask_mirror written
- * when set and ge_mask_mirror_supported(batch) (the mirror is the second destination of every packed-mask write).  records must
- * not overlap the batch's arrays: an in-place fork is a save to a separate buffer followed by a load. */
+ * include GE_STATE_DYNAMIC.  A loaded env's mask_bytes is rebuilt when ge_mask_bytes_current(batch).  records must not overlap
+ * the batch's arrays: an in-place fork is a save to a separate buffer followed by a load. */
 int ge_state_load(const ge_batch *batch, const void *records, int n_records, const int32_t *record_index, unsigned what,
                   void *stream);
 /* For each b in [0, dst->B): dst env b <- the static arrays of src env src_index[b] (src env b when src_index is NULL, which requires

@@ -31,7 +31,7 @@ DEFAULT = "cfg2_longest_path,cfg3_mst,cfg5_multicast,cfg5_distcenter"
 STATE = ("head", "node_bits", "node_bits2", "edge_bits", "dist32", "bestkey", "cost", "counters", "done", "mask_bits", "mask_cnt",
          "acc", "traj")
 STATIC = ("row_ptr", "col", "w32", "w64", "adj_bits", "rev", "esrc", "wsort", "wcode", "dc_edges", "dc_rows", "wmin", "wmat",
-          "src", "dest", "target_bits", "node_cost", "node_xy", "max_dist32", "targets", "in_range", "in_range_t", "heuristic",
+          "src", "dest", "target_bits", "node_cost", "node_xy", "max_dist32", "targets", "in_range", "heuristic",
           "heuristic_alt", "features", "mask0_bits")
 
 

@@ -4,7 +4,7 @@ independent resident batches whose per-step traffic adds up to more than L2, so 
 step of a batch is C sub-batch launches on C free-running streams (graphenvs_b200.batch.SliceStreams).
 
   python profiles/stream_sweep.py --workload cfg2_longest_path --chunks 1,2,4,8 [--replicas R] [--steps K]
-Prints one JSON line per (C) setting.  GE_PDL=1 in the environment adds programmatic dependent launch.
+Prints one JSON line per (C) setting.  --pdl launches every step with programmatic dependent launch (enable_pdl()).
 """
 import argparse
 import json
@@ -29,6 +29,7 @@ def main():
     ap.add_argument("--replicas", type=int, default=0)
     ap.add_argument("--steps", type=int, default=2000)
     ap.add_argument("--envs", type=int, default=0)
+    ap.add_argument("--pdl", action="store_true", help="step launches may start under the previous launch's tail (GE_FLAG_PDL)")
     args = ap.parse_args()
     wl = args.workload
     env_id, N, E, kw, B, _, desc = bench.WORKLOADS[wl]
@@ -46,6 +47,9 @@ def main():
         e.enable_env_clock()
         envs.append(e)
     torch.cuda.synchronize()
+    if args.pdl:
+        for e in envs:
+            e.enable_pdl()
     mem = sum(e.memory_bytes() for e in envs)
     lib_bytes = bench.layout_bytes_per_step(envs[0])
     for e in envs:
@@ -82,8 +86,8 @@ def main():
         b.record()
         torch.cuda.synchronize()
         ms = a.elapsed_time(b) / (reps * G)
-        print(json.dumps({"workload": wl, "envs": B, "replicas": R, "rotation_bytes": per_launch * R, "chunks": C, "pdl": os.environ.get("GE_PDL"),
-                          "lane_t": os.environ.get("GE_LANE_T"), "steps": reps * G, "us_per_step": 1e3 * ms, "env_steps_per_s": B / (ms * 1e-3),
+        print(json.dumps({"workload": wl, "envs": B, "replicas": R, "rotation_bytes": per_launch * R, "chunks": C, "pdl": args.pdl,
+                          "steps": reps * G, "us_per_step": 1e3 * ms, "env_steps_per_s": B / (ms * 1e-3),
                           "frac_hbm": lib_bytes * B / (ms * 1e-3) / 1e9 / 6545.3, "mem_gb": mem / 1e9,
                           "kernel": envs[0].step_kernel_name(sampled=True)}), flush=True)
         del graph

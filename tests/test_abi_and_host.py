@@ -23,7 +23,7 @@ def _declared_symbols():
     return sorted(set(re.findall(r"\b(ge_[a-z0-9_]+)\s*\(", src)))
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_the_declared_symbols_and_abi_version():
     path = _native.build()
     lib = C.CDLL(path)
     syms = _declared_symbols()
@@ -32,7 +32,7 @@ def test_library_exports_every_declared_symbol():
         assert hasattr(lib, s), "missing export %s" % s
     assert sorted(_native.EXPORTS) == syms
     lib.ge_abi_version.restype = C.c_int
-    assert lib.ge_abi_version() == 3
+    assert lib.ge_abi_version() == 4
 
 
 def test_ctypes_struct_matches_c_layout():

@@ -38,7 +38,7 @@ IDS = ["%s-N%d%s%s" % (c[0][:-3], c[1], "".join("-%s%s" % (k[0], v) for k, v in 
 STATE = ("head", "node_bits", "node_bits2", "edge_bits", "dist32", "bestkey", "cost", "counters", "done", "mask_bits", "mask_cnt",
          "acc", "traj")
 STATIC = ("row_ptr", "col", "w32", "w64", "adj_bits", "rev", "esrc", "wsort", "wcode", "dfa", "dc_edges", "dc_rows", "wmin", "wmat",
-          "src", "dest", "target_bits", "node_cost", "node_xy", "max_dist32", "targets", "in_range", "in_range_t", "heuristic",
+          "src", "dest", "target_bits", "node_cost", "node_xy", "max_dist32", "targets", "in_range", "heuristic",
           "heuristic_alt", "features", "mask0_bits")
 M64 = (1 << 64) - 1
 

@@ -174,38 +174,6 @@ def test_fused_sampled_step_equals_sample_then_step(cfg):
     assert torch.equal(a.env_steps, b.env_steps) and int(a.env_steps.min()) == T
 
 
-@pytest.mark.parametrize("cfg", [("LongestPath-v0", 50, 200, {"parenting": 2}), ("TSP-v0", 70, 300, {"parenting": 2}),
-                                 ("SteinerTree-v0", 60, 150, {"n_dests": 5}), ("DistributionCenter-v0", 90, 300, {"parenting": 2})],
-                         ids=lambda c: c[0][:-3])
-def test_zero_copy_host_step_equals_copy_path(cfg):
-    """ge_step_host in zero-copy mode (kernel reads/writes pinned host memory) == the memcpy mode == device step."""
-    env_id, N, E, kw = cfg
-    B, T = 200, 25
-    res = []
-    for mode in ("copies", "zero-copy"):
-        e = BatchedGraphEnv(env_id, B, N, E, auto_reset=True, **kw)
-        e.generate(seed=33)
-        e.reset()
-        blk, h_rew, h_flg, h_cost, h_bits = e.host_io()
-        h_act = torch.zeros(B, dtype=torch.int32).pin_memory()
-        if mode == "zero-copy":
-            e.enable_zero_copy(h_bits)
-        log = []
-        for t in range(T):
-            acts = e.sample_actions(9, t).cpu()
-            h_act.copy_(acts)
-            if mode == "zero-copy":
-                e.step_host_direct(h_act, h_rew, h_flg, h_cost, h_bits)
-            else:
-                e.step_host(h_act, h_rew, h_flg, h_cost, None, h_bits)
-            assert torch.equal(h_bits, e.t["mask_bits"].cpu()), "host mask must equal the device mask after the call"
-            log.append((h_rew.clone(), h_flg.clone(), h_cost.clone(), h_bits.clone()))
-        res.append(log)
-    for (r0, f0, c0, m0), (r1, f1, c1, m1) in zip(*res):
-        assert torch.equal(r0, r1) and torch.equal(f0, f1) and torch.equal(m0, m1)
-        assert torch.equal(torch.nan_to_num(c0, nan=-7.0), torch.nan_to_num(c1, nan=-7.0))
-
-
 def test_host_stepper_graph_replay_matches_direct_calls():
     """ge_step_host on a side stream is captured once and replayed as a CUDA graph: identical results to the
     uncaptured path (default stream) step after step."""
@@ -347,42 +315,28 @@ def test_obs_nodes_is_the_x_tensor_of_obs_graph():
 
 
 @pytest.mark.parametrize("shape", [(120, 500), (80, 1500), (500, 4000)], ids=["sparse", "degree>32", "cfg5"])
-def test_distribution_center_fixed_stride_rows_equal_csr_rows(shape):
-    """ge_batch.dc_rows (weight-sorted rows at a fixed 128-byte stride, no row_ptr lookups) is a layout choice: same
-    trajectories, masks and covered sets as the search over the CSR copy (dc_edges)."""
+def test_distribution_center_fixed_stride_rows_equal_general_family(shape):
+    """The dedicated DistributionCenter kernel, whose cutoff search reads ge_batch.dc_rows (weight-sorted rows at a fixed
+    128-byte stride, prefixes longer than 32 entries continued in dc_edges), gives the same trajectories, masks and covered
+    sets as the general warp-per-env family (GE_FLAG_FORCE_WARP), whose search walks the CSR rows."""
     N, E = shape
     B, T = 256, 40
     envs = []
-    for rows in (False, True):
-        e = BatchedGraphEnv("DistributionCenter-v0", B, N, E, parenting=2, target_count=min(100, N // 4), max_distance=1, auto_reset=True, dc_rows=rows)
+    for force_warp in (False, True):
+        e = BatchedGraphEnv("DistributionCenter-v0", B, N, E, parenting=2, target_count=min(100, N // 4), max_distance=1, auto_reset=True,
+                            force_warp=force_warp)
         e.generate(seed=21)
         e.reset()
-        assert ("dc_rows" in e.t) == rows and e.step_kernel_name() .startswith("dc_step_kernel")
+        assert e.step_kernel_name().startswith("step_kernel<" if force_warp else "dc_step_kernel")
         for t in range(T):
             e.step_sampled(4, t)
         torch.cuda.synchronize()
         envs.append(e)
     a, b = envs
+    assert "dc_rows" in a.t
+    assert torch.equal(a.t["row_ptr"], b.t["row_ptr"]) and torch.equal(a.t["col"], b.t["col"]), "both batches must hold the same graphs"
     if N == 80:
         deg = (a.t["row_ptr"][:, 1:N + 1] - a.t["row_ptr"][:, :N]).max().item()
         assert deg > 32, "this shape is meant to overflow the 32-entry rows"
     for k in ("traj", "mask_bits", "node_bits", "node_bits2", "cost", "acc", "done"):
         assert torch.equal(a.t[k], b.t[k]), k
-
-
-def test_distribution_center_transposed_mask_equals_row_union():
-    """The optional transposed in-range table (per node a 128-bit target set, csrc/ge_dc.cu:dc_union_transposed) builds
-    the same masks and trajectories as the OR of the uncovered targets' rows."""
-    B, T = 400, 40
-    envs = []
-    for tr in (False, True):
-        e = BatchedGraphEnv("DistributionCenter-v0", B, 120, 500, parenting=2, auto_reset=True, dc_transposed=tr)
-        e.generate(seed=12)
-        e.reset()
-        assert ("in_range_t" in e.t) == tr
-        for t in range(T):
-            e.step_sampled(6, t)
-        torch.cuda.synchronize()
-        envs.append(e)
-    for name in ("traj", "acc", "mask_bits", "node_bits", "node_bits2", "cost"):
-        assert torch.equal(envs[0].t[name], envs[1].t[name]), name
