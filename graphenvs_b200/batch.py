@@ -591,7 +591,8 @@ class BatchedGraphEnv:
 
     @property
     def mask(self):
-        """bool[B, A] view of the current valid-action masks (None when byte_mask=False).  For the incremental-mask kinds
+        """bool[B, A] view of the current valid-action masks (None when byte_mask=False).  For the lane-per-env kinds
+        (N <= 64: ShortestPath, LongestPath, TSP, MaxIndependentSet, DensestSubgraph) and the incremental-mask kinds
         (SteinerTree, Multicast parenting >= 2, MaxIndependentSet N > 64) the step kernels keep only the packed mask
         current and this property expands it into the byte view first (ge_mask_bytes, one coalesced pass)."""
         mb = self.t.get("mask_bytes")

@@ -807,7 +807,8 @@ int ge_progress_supported(const ge_batch *d) {
     return ge_lane_eligible(d) || ge_dc_eligible(d);
 }
 
-int ge_mask_bytes_current(const ge_batch *d) { return d && d->mask_bytes && !ge_incr_eligible(d); }
+// The incremental-mask and lane-per-env families keep only the packed mask current.
+int ge_mask_bytes_current(const ge_batch *d) { return d && d->mask_bytes && !ge_incr_eligible(d) && !ge_lane_eligible(d); }
 
 int ge_mask_bytes(const ge_batch *d, int env_lo, int count, void *stream) {
     GE_NVTX("ge_mask_bytes");

@@ -197,16 +197,11 @@ __device__ __forceinline__ void lane_store_state(const ge_batch &d, int b, const
     d.head[b] = s.head;
     d.cost[b] = s.cost;
     if (counters) *reinterpret_cast<int4 *>(d.counters + (size_t)b * 4) = make_int4(s.k, s.ecnt, 0, 0);
-    // mask: packed words + bytes (AP <= 64: up to four 128-bit stores)
+    // mask: the packed words only.  The byte view (mask_bytes) is expanded on demand by ge_mask_bytes
+    // (ge_mask_bytes_current() == 0 for this family): keeping it current costs AP bytes per env and ~16 % of the
+    // step's warp instructions, for a view the samplers and the packed host results do not read.
     if (d.AW == 1) d.mask_bits[b] = (uint32_t)mask;
     else reinterpret_cast<uint2 *>(d.mask_bits)[b] = make_uint2((uint32_t)mask, (uint32_t)(mask >> 32));
-    if (d.mask_bytes) {
-        uint4 *mb = reinterpret_cast<uint4 *>(d.mask_bytes + (size_t)b * d.AP);
-        for (int c = 0; c < (d.AP >> 4); ++c) {
-            uint32_t bits = (uint32_t)(mask >> (16 * c)) & 0xffffu;
-            mb[c] = make_uint4(expand4(bits), expand4(bits >> 4), expand4(bits >> 8), expand4(bits >> 12));
-        }
-    }
 }
 
 // adj[u, v] of the reference's dense float64 matrix (shortest_path.py:82); 0 when there is no edge.
@@ -392,9 +387,23 @@ __global__ void __launch_bounds__(LANE_BOUND) lane_step_kernel(ge_batch d, int32
         if (d.env_steps) d.env_steps[b] = nsteps + 1u;
         d.acc[2 * (size_t)d.acc_stride + b] = acc_r + reward;
         if (done) {
-            d.acc[b] += 1.0;
-            if (solved == 1) d.acc[(size_t)d.acc_stride + b] += 1.0;
-            if (sol == sol) d.acc[3 * (size_t)d.acc_stride + b] += sol;
+            if (STAGED) {
+                d.acc[b] += 1.0;
+                if (solved == 1) d.acc[(size_t)d.acc_stride + b] += 1.0;
+                if (sol == sol) d.acc[3 * (size_t)d.acc_stride + b] += sol;
+            } else {
+                // The unstaged kernels load the three rows before storing any: one memory round trip at the end of the warp
+                // instead of three dependent ones (each `+=` waits for the previous store, which may alias).  cfg1: 9.55 ->
+                // 10.8 G env-steps/s.  The staged kernels keep the `+=`: with the rows loaded together (or at the top of
+                // the kernel) their cfg2 streaming step measured slower (DESIGN §6b).
+                const size_t st = (size_t)d.acc_stride;
+                const double episodes = d.acc[b];
+                const double n_solved = solved == 1 ? d.acc[st + b] : 0.0;
+                const double cost_sum = sol == sol ? d.acc[3 * st + b] : 0.0;
+                d.acc[b] = episodes + 1.0;
+                if (solved == 1) d.acc[st + b] = n_solved + 1.0;
+                if (sol == sol) d.acc[3 * st + b] = cost_sum + sol;
+            }
         }
     }
     if (done && (d.flags & GE_FLAG_AUTO_RESET)) {                               // tail of reset()

@@ -169,10 +169,12 @@ typedef struct ge_batch {
     uint32_t *mask_bits;          /* [B, AW]  current valid-action mask, packed */
     uint32_t *mask_cnt;           /* [B, 8]   incremental-mask kernels with large masks: popcounts of the 16 chunks of ceil(AW/16) words
                                               of the packed mask, 16 bits each (state, maintained with the mask), or NULL */
-    uint8_t *mask_bytes;          /* [B, AP]  same mask as bytes (torch.bool view) or NULL.  Kept current by the kernels that
-                                              rewrite the whole mask; the INCREMENTAL-mask kernels (SteinerTree, Multicast p >= 2,
-                                              MaxIndependentSet N > 64: ge_mask_bytes_current() == 0) update only the packed mask and
-                                              the byte view is produced on demand by ge_mask_bytes */
+    uint8_t *mask_bytes;          /* [B, AP]  same mask as bytes (torch.bool view) or NULL.  Kept current by the group,
+                                              DistributionCenter, PerishableProductDelivery and general kernels; the LANE-PER-ENV
+                                              kernels (N <= 64: ShortestPath, LongestPath, TSP, MaxIndependentSet, DensestSubgraph) and
+                                              the INCREMENTAL-mask kernels (SteinerTree, Multicast p >= 2, MaxIndependentSet N > 64)
+                                              update only the packed mask (ge_mask_bytes_current() == 0) and the byte view is produced
+                                              on demand by ge_mask_bytes */
     uint32_t *mask0_bits;         /* [B, AW]  mask right after reset(), written by ge_reset, or NULL.  It depends only on the
                                               instance, so auto-reset inside ge_step copies it instead of recomputing it */
     double *acc;                  /* [4, acc_stride] per-env statistics: episodes, solved, sum reward, sum final cost */
@@ -261,8 +263,9 @@ int ge_obs_nodes(const ge_batch *batch, int env_lo, int count, float *x, void *s
 const char *ge_step_kernel_name(const ge_batch *batch, int sampled);
 
 /* 1 when every ge_step / ge_reset leaves mask_bytes equal to the packed mask; 0 when the byte view must be refreshed with
- * ge_mask_bytes before it is read (incremental-mask kernels: a scattered byte store per changed edge was 2.3 KB of HBM
- * traffic per Multicast step against 1.8 KB of useful bytes). */
+ * ge_mask_bytes before it is read: the incremental-mask kernels (a scattered byte store per changed edge was 2.3 KB of HBM
+ * traffic per Multicast step against 1.8 KB of useful bytes) and the lane-per-env kernels (AP bytes per env and about 16 %
+ * of the step's instructions for a view that the samplers and the packed host results do not read). */
 int ge_mask_bytes_current(const ge_batch *batch);
 /* Expands the packed mask of envs [env_lo, env_lo + count) into mask_bytes (one coalesced pass). */
 int ge_mask_bytes(const ge_batch *batch, int env_lo, int count, void *stream);
