@@ -7,6 +7,7 @@ Public surface:
                                      save_states / load_states / gather_instances / like: branching for search decoders)
   masked_log_prob(logits, mask_bits, actions)   differentiable masked log-prob + entropy for the update (policy.py)
   BeamSearch(venv, width)            beam search / multi-start decoding of a policy on the device (beam.py)
+  StochasticBeamSearch(venv, width, seed)   width distinct sequences per instance sampled without replacement (beam.py)
   utils.vectorize_graph / devectorize_graph / get_env_info   (graph_envs/utils.py layout contract)
 """
 from .spec import ENV_SPECS, get_env_info, get_num_features  # noqa: F401
@@ -25,9 +26,9 @@ def __getattr__(attr):  # lazy: keeps `import graphenvs_b200` cheap and torch-fr
     if attr == "masked_log_prob":
         from .policy import masked_log_prob
         return masked_log_prob
-    if attr == "BeamSearch":
-        from .beam import BeamSearch
-        return BeamSearch
+    if attr in ("BeamSearch", "StochasticBeamSearch"):
+        from . import beam
+        return getattr(beam, attr)
     if attr in ("Instance", "generate_instance"):
         from . import instances
         return getattr(instances, attr)

@@ -94,7 +94,7 @@ EXPORTS = ["ge_abi_version", "ge_last_error", "ge_fill_layout", "ge_step_smem_by
            "ge_prepare", "ge_features", "ge_generate", "ge_generate_fallbacks", "ge_pool_refill", "ge_reset", "ge_step", "ge_step_sampled", "ge_sample_actions", "ge_obs_len",
            "ge_obs_flat", "ge_obs_graph", "ge_obs_nodes", "ge_step_kernel_name", "ge_batch_slice", "ge_step_host", "ge_step_host_pipelined", "ge_step_host_compact", "ge_progress_supported",
            "ge_step_host_release", "ge_mask_bytes_current", "ge_mask_bytes", "ge_stats",
-           "ge_sample_logits", "ge_masked_log_prob", "ge_masked_log_prob_backward", "ge_beam_expand",
+           "ge_sample_logits", "ge_masked_log_prob", "ge_masked_log_prob_backward", "ge_beam_expand", "ge_beam_expand_sampled",
            "ge_state_record_bytes", "ge_state_save", "ge_state_load", "ge_gather_instances"]
 
 LOGITS_F32, LOGITS_BF16 = 0, 1   # GE_LOGITS_*
@@ -149,6 +149,7 @@ def lib():
     L.ge_masked_log_prob.argtypes = [_P, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P]
     L.ge_masked_log_prob_backward.argtypes = [_P, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P]
     L.ge_beam_expand.argtypes = [BP, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P, _P]
+    L.ge_beam_expand_sampled.argtypes = [BP, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]
     L.ge_state_record_bytes.argtypes = [BP]
     L.ge_state_save.argtypes = [BP, _P, C.c_int, _P, _P]
     L.ge_state_load.argtypes = [BP, _P, C.c_int, _P, C.c_uint, _P]

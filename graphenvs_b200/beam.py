@@ -11,10 +11,17 @@ candidate with its score and is stepped with -1 (GE_STEP_AFTER_DONE: state and s
 column -- zeroed at the start and forked with its beam -- is that branch's own return, final cost and solved flag.  The
 initial scores [0, -inf, ..., -inf] make the first expansion pick W distinct first actions: multi-start decoding is the
 same loop.
+
+    sbs = StochasticBeamSearch(venv, width=16, seed=0)   # 16 distinct sequences per instance, sampled without replacement
+    res = sbs.run(policy)                                # as above, plus res.kappa and res.beams.log_prob / key / weight
+
+StochasticBeamSearch is the same loop with ge_beam_expand_sampled: candidates ranked by Gumbel-perturbed log-probs conditioned
+on their parent's (Kool, van Hoof, Welling 2019), with noise keyed by (seed, global instance id, action prefix).
 """
 import ctypes as C
 from types import SimpleNamespace
 
+import numpy as np
 import torch
 
 from . import _native
@@ -178,3 +185,130 @@ class BeamSearch:
                 break
             self.advance(policy(self.wide))
         return self.result()
+
+
+# ---------------------------------------------------------------------- stochastic beam search
+_M64 = (1 << 64) - 1
+ROOT_T = 0x52DCE729          # the counter of the root node keys (include/graphenvs_b200.h, ge_beam_expand_sampled)
+
+
+def _mix32(seed, env, t):
+    """csrc/ge_common.cuh:mix32 in numpy uint64 arithmetic (wrapping); seed / env broadcast."""
+    with np.errstate(over="ignore"):
+        seed, env, t = np.asarray(seed, dtype=np.uint64), np.asarray(env, dtype=np.uint64), np.uint64(t)
+        z = seed + np.uint64(0x9E3779B97F4A7C15) * (env * np.uint64(0x100000001) + ((t << np.uint64(32)) | np.uint64(0x5bd1e995)))
+        z = (z ^ (z >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
+        z = (z ^ (z >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
+        z = z ^ (z >> np.uint64(31))
+        return z >> np.uint64(32)
+
+
+def root_key(seed, instance):
+    """Node key of the root of global instance id(s) `instance` (numpy uint64):
+    (uint64) mix32(seed, i, 0x52DCE729) << 32 | mix32(seed ^ 0xD1B54A32D192ED03, i, 0x52DCE729)."""
+    i = np.asarray(instance, dtype=np.uint64)
+    return (_mix32(np.uint64(seed), i, ROOT_T) << np.uint64(32)) | _mix32(np.uint64(seed ^ 0xD1B54A32D192ED03), i, ROOT_T)
+
+
+def root_gumbel(node_key):
+    """The Gumbel(0) key of a root: the noise of ge_sample_logits' formula at action 0xFFFFFFFF of the root's node key, in
+    float64 (the caller rounds it to float32)."""
+    h = _mix32(np.asarray(node_key, dtype=np.uint64), 0xFFFFFFFF, 0x85EBCA6B)
+    u = ((h >> np.uint64(8)).astype(np.float64) + 0.5) / 2.0 ** 24
+    return -np.log(-np.log(u))
+
+
+class StochasticBeamSearch(BeamSearch):
+    """Stochastic beam search (Kool, van Hoof, Welling 2019): per instance of `venv`, `width` distinct sequences drawn without
+    replacement from the policy's sequence distribution, with ge_beam_expand_sampled as the expand step.
+
+    It is BeamSearch's loop (wide batch, forks, steps, history, backtracking) with three ping-pong arrays per slot instead of
+    the score: the log-prob phi (kept in `score`, so an empty slot is still score -inf), the perturbed log-prob `key` and the
+    tree-node key `node_key` that keys the Gumbel noise.  The noise of a node depends only on (seed, global instance id,
+    action prefix), so a wider search extends a narrower one (its first W slots are the width-W search), a rank slice of the
+    instances (venv.desc.env_id0 > 0) draws what the full batch draws for them, and width 1 is ancestral sampling."""
+
+    def __init__(self, venv, width=16, seed=0):
+        if isinstance(seed, bool) or not isinstance(seed, int):
+            raise TypeError("StochasticBeamSearch: seed must be an int, got %r" % (seed,))
+        if not 0 <= seed <= _M64:
+            raise ValueError("StochasticBeamSearch: seed must be in [0, 2^64), got %d" % seed)
+        super().__init__(venv, width)
+        self.seed = seed
+        dev = self.wide.device
+        rk = root_key(seed, int(venv.desc.env_id0) + np.arange(self.G, dtype=np.uint64))
+        self._root_key = torch.from_numpy(rk.view(np.int64).copy()).to(dev)
+        self._root_gumbel = torch.from_numpy(root_gumbel(rk).astype(np.float32)).to(dev)
+        self.key = torch.empty(self.B, dtype=torch.float32, device=dev)
+        self._key_next = torch.empty_like(self.key)
+        self.node_key = torch.empty(self.B, dtype=torch.int64, device=dev)       # uint64 bit patterns
+        self._node_key_next = torch.empty_like(self.node_key)
+        self._thresholds = torch.empty((0, self.G), dtype=torch.float32, device=dev)
+
+    def reserve(self, steps):
+        super().reserve(steps)
+        cap = self._parents.shape[0]
+        if self._thresholds.shape[0] < cap:
+            th = torch.empty((cap, self.G), dtype=torch.float32, device=self.wide.device)
+            th[:self.t].copy_(self._thresholds[:self.t])
+            self._thresholds = th
+
+    def start(self, from_current=False):
+        """BeamSearch.start, then slot 0 of group g becomes the root: logp 0, key G_root(g), node key root_key(seed,
+        venv.desc.env_id0 + g); the other slots are dead (key -inf)."""
+        super().start(from_current)
+        self.key.fill_(float("-inf"))
+        self.key.view(self.G, self.W)[:, 0] = self._root_gumbel
+        self.node_key.zero_()
+        self.node_key.view(self.G, self.W)[:, 0] = self._root_key
+
+    def expand(self, logits, parent=None, action=None):
+        """One ge_beam_expand_sampled over the wide batch's current masks: per group the W children of largest conditioned
+        key.  Replaces score (phi), key and node_key, records the group thresholds at history row t (reserve(t + 1) first) and
+        returns (parent, action, load_index) as BeamSearch.expand does."""
+        x = self._check_logits(logits)
+        dev = self.wide.device
+        if parent is None:
+            parent = torch.empty(self.B, dtype=torch.int32, device=dev)
+        if action is None:
+            action = torch.empty(self.B, dtype=torch.int32, device=dev)
+        self.reserve(self.t + 1)
+        wide = self.wide
+        _native.check(wide.lib.ge_beam_expand_sampled(
+            C.byref(wide.desc), self.W, _ptr(x), _DTYPES[x.dtype], _ptr(self.score), _ptr(self.key), _ptr(self.node_key),
+            _ptr(self._score_next), _ptr(self._key_next), _ptr(self._node_key_next), _ptr(parent), _ptr(action),
+            _ptr(self.load_index), _ptr(self._thresholds[self.t]), wide._stream()))
+        self.score, self._score_next = self._score_next, self.score
+        self.key, self._key_next = self._key_next, self.key
+        self.node_key, self._node_key_next = self._node_key_next, self.node_key
+        return parent, action, self.load_index
+
+    def result(self):
+        """BeamSearch.result() (the best finished return per group, every slot), plus:
+          beams.log_prob  float32 [G, W] phi, the sum of each sequence's masked log-probs (= beams.score)
+          beams.key       float32 [G, W] its perturbed log-prob G; slots come in descending key order, so slot 0 is an exact
+                          draw from the policy's sequence distribution
+          kappa           float32 [G] the largest group threshold over the steps: the (W+1)-th largest leaf key, -inf when
+                          the search enumerated every sequence
+          beams.weight    float64 [G, W] exp(phi) / q, q = -expm1(-exp(phi - kappa)) the inclusion probability (q = 1 when
+                          kappa = -inf); 0 for an empty slot, NaN for every slot of a group with a live unfinished beam.
+        sum_j weight[g, j] f(y_j) is an unbiased estimate of E_y[f(y)] (priority sampling)."""
+        res = super().result()
+        G, W, T = self.G, self.W, self.t
+        neg = float("-inf")
+        if T:
+            kappa = self._thresholds[:T].amax(dim=0)
+        else:
+            kappa = torch.full((G,), neg, dtype=torch.float32, device=self.wide.device)
+        phi = self.score.view(G, W).double()
+        k = kappa.double()[:, None]
+        q = torch.where(k == neg, torch.ones_like(phi), -torch.expm1(-torch.exp(phi - k)))
+        alive = phi > neg
+        weight = torch.where(alive, torch.exp(phi) / q, torch.zeros_like(phi))
+        unfinished = (alive & ~res.beams.done).any(dim=1, keepdim=True)
+        weight = torch.where(unfinished, torch.full_like(weight, float("nan")), weight)
+        res.beams.log_prob = res.beams.score
+        res.beams.key = self.key.clone().view(G, W)
+        res.beams.weight = weight
+        res.kappa = kappa
+        return res

@@ -25,7 +25,7 @@ namespace {
 constexpr int POL_WPB = 8;  // warps (= rows) per block
 constexpr int POL_U = 4;    // nonzero mask words whose logits are loaded together
 
-enum { MODE_STATS = 0, MODE_GREEDY = 1, MODE_GUMBEL = 2 };
+enum { MODE_STATS = 0, MODE_GREEDY = 1, MODE_GUMBEL = 2, MODE_NODE_GUMBEL = 3 };
 
 template <int DT>
 __device__ __forceinline__ float load_logit(const void *row, size_t i) {
@@ -45,6 +45,13 @@ __device__ __forceinline__ void store_grad(void *row, size_t i, float g) {
 __device__ __forceinline__ float gumbel(uint64_t key, int a) {
     const uint32_t h = mix32(key, (uint32_t)a, 0x85EBCA6Bu);
     const float u = __fmul_rn((float)(h >> 8) + 0.5f, 5.9604644775390625e-8f);  // ((h >> 8) + 1/2) / 2^24, exact, in (0, 1)
+    return -logf(-logf(u));
+}
+// The noise of ge_beam_expand_sampled: gumbel() with u kept below 1.  (h >> 8) + 0.5 rounds to even in float32 once h >> 8 >= 2^23,
+// so h >> 8 = 2^24 - 1 gives u = 1 and g = +inf there; here u is clamped to 1 - 2^-24, and every key is finite.
+__device__ __forceinline__ float node_gumbel(uint64_t key, int a) {
+    const uint32_t h = mix32(key, (uint32_t)a, 0x85EBCA6Bu);
+    const float u = fminf(__fmul_rn((float)(h >> 8) + 0.5f, 5.9604644775390625e-8f), 0.99999994f);
     return -logf(-logf(u));
 }
 __device__ __forceinline__ uint64_t row_key(uint64_t seed, uint32_t env, uint32_t t) {
@@ -120,7 +127,8 @@ __device__ __forceinline__ RowStats masked_row(const void *row, const uint32_t *
                 if (!has[k]) continue;
                 acc_one(r, v[k]);
                 if (MODE != MODE_STATS) {
-                    const float s = MODE == MODE_GUMBEL ? __fadd_rn(v[k], gumbel(key, idx[k])) : v[k];
+                    const float s = MODE == MODE_GUMBEL ? __fadd_rn(v[k], gumbel(key, idx[k]))
+                                  : MODE == MODE_NODE_GUMBEL ? __fadd_rn(v[k], node_gumbel(key, idx[k])) : v[k];
                     if (s > r.bs) { r.bs = s; r.bi = idx[k]; r.bl = v[k]; }   // strictly greater: a lane visits its actions in order
                 }
             }
@@ -248,12 +256,22 @@ __device__ __forceinline__ bool beam_before(float s1, int p1, int a1, float s2, 
     return s1 > s2 || (s1 == s2 && (p1 < p2 || (p1 == p2 && a1 < a2)));
 }
 
+// Per-candidate scores of the two expand kernels: what beam_next ranks by.
+struct LogProbScore {     // ge_beam_expand: the beam's score after action a, fl32(base + fl32(l_a - lse))
+    float base, lse;
+    __device__ __forceinline__ float operator()(float l, int) const { return __fadd_rn(base, __fsub_rn(l, lse)); }
+};
+struct PerturbedScore {   // ge_beam_expand_sampled: the Gumbel-max score keyed by the beam's node key, fl32(l_a + g_a)
+    uint64_t key;
+    __device__ __forceinline__ float operator()(float l, int a) const { return __fadd_rn(l, node_gumbel(key, a)); }
+};
+
 // The best candidate of one live beam that comes after (ps, pa) in the order (the best overall when `first`), over its valid
-// actions: score fl32(base + fl32(l_a - lse)).  Walks the row as masked_row does (zero words skipped warp-uniformly, only
-// logits of set bits read); after the first walk the mask and the valid logits are L1-resident.  Warp-uniform result;
-// ba = INT_MAX when no candidate is left.
-template <int DT>
-__device__ __forceinline__ void beam_next(const void *row, const uint32_t *__restrict__ mrow, int A, int AW, float base, float lse,
+// actions, ranked by score(l_a, a).  Walks the row as masked_row does (zero words skipped warp-uniformly, only logits of set
+// bits read); after the first walk the mask and the valid logits are L1-resident.  Warp-uniform result; ba = INT_MAX when no
+// candidate is left.
+template <int DT, class Score>
+__device__ __forceinline__ void beam_next(const void *row, const uint32_t *__restrict__ mrow, int A, int AW, Score score,
                                           bool first, float ps, int pa, int lane, float &bs, int &ba) {
     float s_best = -INFINITY;
     int a_best = INT_MAX;
@@ -278,7 +296,7 @@ __device__ __forceinline__ void beam_next(const void *row, const uint32_t *__res
 #pragma unroll
             for (int k = 0; k < POL_U; ++k) {
                 if (!has[k]) continue;
-                const float s = __fadd_rn(base, __fsub_rn(v[k], lse));
+                const float s = score(v[k], idx[k]);
                 if ((first || beam_before(ps, 0, pa, s, 0, idx[k])) && beam_before(s, 0, idx[k], s_best, 0, a_best)) { s_best = s; a_best = idx[k]; }
             }
         }
@@ -324,7 +342,7 @@ __global__ void __launch_bounds__(BEAM_WARPS * 32) beam_expand_kernel(ge_batch d
                 float ps = 0.f;
                 int pa = 0;
                 for (; n < W; ++n) {
-                    beam_next<DT>(row, mrow, d.A, d.AW, base, lse, n == 0, ps, pa, lane, ps, pa);
+                    beam_next<DT>(row, mrow, d.A, d.AW, LogProbScore{base, lse}, n == 0, ps, pa, lane, ps, pa);
                     if (pa == INT_MAX) break;
                     if (lane == 0) { l_s[p][n] = ps; l_a[p][n] = pa; }
                 }
@@ -358,6 +376,129 @@ __global__ void __launch_bounds__(BEAM_WARPS * 32) beam_expand_kernel(ge_batch d
         const int b = g0 + lane;
         const int par = my_p < 0 ? -1 : g0 + my_p;
         score_out[b] = my_s;
+        parent[b] = par;
+        action[b] = my_a;
+        load_index[b] = par == b ? -1 : par;
+    }
+}
+
+// ---- stochastic beam search (ge_beam_expand_sampled): beam_expand_kernel's layout, ranked by conditioned Gumbel keys ----
+// log(1 - e^x) for x <= 0, accurate on both sides of -ln 2 (log1mexp(0) = -inf).
+__device__ __forceinline__ float log1mexp(float x) {
+    return x > -0.6931472f ? logf(-expm1f(x)) : log1pf(-expf(x));
+}
+// The key of the child whose perturbed score lies x = fl32(s_a - S_b) <= 0 below the beam's best, given the beam's key T and
+// D = T - (its children's unconditioned maximum): T - softplus(v), v = (D - x) + log1mexp(x).  x = 0 gives T exactly.
+__device__ __forceinline__ float conditioned_key(float T, float D, float x) {
+    const float v = __fadd_rn(__fsub_rn(D, x), log1mexp(x));
+    return __fsub_rn(T, __fadd_rn(fmaxf(v, 0.f), log1pf(expf(-fabsf(v)))));
+}
+// The node key of the child of node h by action a (include/graphenvs_b200.h, ge_beam_expand_sampled).
+__device__ __forceinline__ uint64_t child_key(uint64_t h, int a) {
+    return ((uint64_t)mix32(h, (uint32_t)a, 0x2545F491u) << 32) | (uint64_t)mix32(h ^ 0x9E3779B97F4A7C15ull, (uint32_t)a, 0x6C8E9CF5u);
+}
+
+template <int DT>
+__global__ void __launch_bounds__(BEAM_WARPS * 32) beam_expand_sampled_kernel(ge_batch d, int W, const void *__restrict__ logits,
+                                                                               const float *__restrict__ logp, const float *__restrict__ key,
+                                                                               const uint64_t *__restrict__ node_key, float *__restrict__ logp_out,
+                                                                               float *__restrict__ key_out, uint64_t *__restrict__ node_key_out,
+                                                                               int32_t *__restrict__ parent, int32_t *__restrict__ action,
+                                                                               int32_t *__restrict__ load_index, float *__restrict__ threshold) {
+    __shared__ float l_g[BEAM_MAXW][BEAM_MAXW + 1];   // per beam: its best min(W + 1, candidates) candidates and their keys
+    __shared__ int l_a[BEAM_MAXW][BEAM_MAXW + 1];
+    __shared__ int l_n[BEAM_MAXW];
+    __shared__ float l_lse[BEAM_MAXW];
+    pdl_launch_dependents();   // as the sampler: nothing is touched before pdl_wait()
+    pdl_wait();
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+    const int g0 = blockIdx.x * W;
+    const size_t esz = DT == GE_LOGITS_BF16 ? 2 : 4;
+    // Stage 1: every beam's W + 1 best candidates in the order (s_a desc, a asc), and their conditioned keys
+    for (int p = warp; p < W; p += nwarps) {
+        const int b = g0 + p;
+        const float T = key[b];
+        int n = 0;
+        if (T == -INFINITY) {
+            n = 0;                                                 // dead
+        } else if (d.done[b]) {
+            if (lane == 0) { l_g[p][0] = T; l_a[p][0] = -1; }    // stay
+            n = 1;
+        } else {
+            const void *row = reinterpret_cast<const char *>(logits) + (size_t)b * d.A * esz;
+            const uint32_t *mrow = d.mask_bits + (size_t)b * d.AW;
+            const uint64_t nk = node_key[b];
+            const RowStats r = masked_row<DT, MODE_NODE_GUMBEL>(row, mrow, d.A, d.AW, nk, lane);   // lse and the best (S_b, a)
+            if (r.se > 0.f) {
+                const float lse = row_lse(r), S = r.bs;
+                const float D = __fsub_rn(T, __fadd_rn(logp[b], __fsub_rn(S, lse)));
+                if (lane == 0) l_lse[p] = lse;
+                float ps = S;
+                int pa = r.bi;
+                for (;;) {
+                    if (lane == 0) { l_g[p][n] = conditioned_key(T, D, __fsub_rn(ps, S)); l_a[p][n] = pa; }
+                    if (++n == W + 1) break;
+                    beam_next<DT>(row, mrow, d.A, d.AW, PerturbedScore{nk}, false, ps, pa, lane, ps, pa);
+                    if (pa == INT_MAX) break;
+                }
+            }
+        }
+        if (lane == 0) l_n[p] = n;
+    }
+    __syncthreads();
+    if (warp != 0) return;
+    // Lane p puts list p in the merge order (G desc, a asc): the keys follow s_a only up to rounding, so the list is nearly sorted
+    const int len = lane < W ? l_n[lane] : 0;
+    for (int i = 1; i < len; ++i) {
+        const float g = l_g[lane][i];
+        const int a = l_a[lane][i];
+        int k = i;
+        for (; k > 0 && beam_before(g, 0, a, l_g[lane][k - 1], 0, l_a[lane][k - 1]); --k) {
+            l_g[lane][k] = l_g[lane][k - 1];
+            l_a[lane][k] = l_a[lane][k - 1];
+        }
+        l_g[lane][k] = g;
+        l_a[lane][k] = a;
+    }
+    // Stage 2: beam_expand_kernel's warp arg-max merge in the order (G desc, parent slot asc, action asc); round W is the threshold
+    const int rounds = threshold ? W + 1 : W;
+    int head = 0;
+    float my_g = -INFINITY, thr = -INFINITY;
+    int my_p = -1, my_a = -1;
+    for (int j = 0; j < rounds; ++j) {
+        float s = -INFINITY;
+        int p = INT_MAX, a = INT_MAX;
+        if (head < len) { s = l_g[lane][head]; p = lane; a = l_a[lane][head]; }
+#pragma unroll
+        for (int o = 16; o; o >>= 1) {
+            const float s2 = __shfl_xor_sync(GE_FULL, s, o);
+            const int p2 = __shfl_xor_sync(GE_FULL, p, o);
+            const int a2 = __shfl_xor_sync(GE_FULL, a, o);
+            if (beam_before(s2, p2, a2, s, p, a)) { s = s2; p = p2; a = a2; }
+        }
+        if (p == INT_MAX) break;
+        if (j == W) { thr = s; break; }
+        if (lane == p) ++head;
+        if (lane == j) { my_g = s; my_p = p; my_a = a; }
+    }
+    if (threshold && lane == 0) threshold[blockIdx.x] = thr;
+    if (lane < W) {
+        const int b = g0 + lane;
+        const int par = my_p < 0 ? -1 : g0 + my_p;
+        float lp = -INFINITY;
+        uint64_t nk = 0;
+        if (par >= 0) {
+            lp = logp[par];
+            nk = node_key[par];
+            if (my_a >= 0) {   // a valid action of a live beam: its logit is read again, for the log-prob of ge_beam_expand
+                const void *row = reinterpret_cast<const char *>(logits) + (size_t)par * d.A * esz;
+                lp = __fadd_rn(lp, __fsub_rn(load_logit<DT>(row, (size_t)my_a), l_lse[my_p]));
+                nk = child_key(nk, my_a);
+            }
+        }
+        logp_out[b] = lp;
+        key_out[b] = my_g;
+        node_key_out[b] = nk;
         parent[b] = par;
         action[b] = my_a;
         load_index[b] = par == b ? -1 : par;
@@ -455,6 +596,42 @@ int ge_beam_expand(const ge_batch *d, int W, const void *logits, int dtype, cons
         ? ge_launch_step(beam_expand_kernel<GE_LOGITS_BF16>, grid, block, 0, st, *d, W, logits, score, score_out, parent, action, load_index)
         : ge_launch_step(beam_expand_kernel<GE_LOGITS_F32>, grid, block, 0, st, *d, W, logits, score, score_out, parent, action, load_index);
     if (e != cudaSuccess) { (void)cudaGetLastError(); return ge_set_error(GE_ERR_CUDA, "beam_expand_kernel launch: %s", cudaGetErrorString(e)); }
+    return GE_OK;
+}
+
+int ge_beam_expand_sampled(const ge_batch *d, int W, const void *logits, int dtype, const float *logp, const float *key,
+                           const uint64_t *node_key, float *logp_out, float *key_out, uint64_t *node_key_out, int32_t *parent,
+                           int32_t *action, int32_t *load_index, float *threshold, void *stream) {
+    GE_NVTX("ge_beam_expand_sampled");
+    const char *fn = "ge_beam_expand_sampled";
+    if (!d) return ge_set_error(GE_ERR_ARG, "%s: null batch", fn);
+    if (dtype != GE_LOGITS_F32 && dtype != GE_LOGITS_BF16) return ge_set_error(GE_ERR_ARG, "%s: unknown logits dtype %d", fn, dtype);
+    if (W < 1 || W > BEAM_MAXW) return ge_set_error(GE_ERR_ARG, "%s: width W = %d not in [1, %d]", fn, W, BEAM_MAXW);
+    if (d->B <= 0 || d->A <= 0 || d->AW != (d->A + 31) / 32) return ge_set_error(GE_ERR_ARG, "%s: bad shape B=%d A=%d AW=%d (call ge_fill_layout)", fn, d->B, d->A, d->AW);
+    if (d->B % W) return ge_set_error(GE_ERR_ARG, "%s: B = %d is not a multiple of W = %d", fn, d->B, W);
+    if (!logits || !logp || !key || !node_key || !logp_out || !key_out || !node_key_out || !parent || !action || !load_index)
+        return ge_set_error(GE_ERR_ARG, "%s: null logits / logp / key / node_key / logp_out / key_out / node_key_out / parent / action / load_index", fn);
+    if (!d->mask_bits || !d->done) return ge_set_error(GE_ERR_ARG, "%s: null mask_bits / done in the batch", fn);
+    {   // no two of the arrays may overlap: B elements of 4 bytes each (8 for the node keys), B / W floats of threshold
+        const uintptr_t B = (uintptr_t)d->B;
+        const uintptr_t p[10] = {(uintptr_t)logp, (uintptr_t)key, (uintptr_t)node_key, (uintptr_t)logp_out, (uintptr_t)key_out,
+                                 (uintptr_t)node_key_out, (uintptr_t)parent, (uintptr_t)action, (uintptr_t)load_index, (uintptr_t)threshold};
+        const uintptr_t n[10] = {4 * B, 4 * B, 8 * B, 4 * B, 4 * B, 8 * B, 4 * B, 4 * B, 4 * B, threshold ? 4 * (B / W) : 0};
+        for (int i = 0; i < 10; ++i)
+            for (int j = i + 1; j < 10; ++j)
+                if (n[i] && n[j] && p[i] < p[j] + n[j] && p[j] < p[i] + n[i])
+                    return ge_set_error(GE_ERR_ARG, "%s: logp, key, node_key, logp_out, key_out, node_key_out, parent, action, load_index "
+                                                    "and threshold must not overlap", fn);
+    }
+    const int warps = W < BEAM_WARPS ? W : BEAM_WARPS;
+    const dim3 grid((unsigned)(d->B / W)), block(warps * 32);
+    cudaStream_t st = (cudaStream_t)stream;
+    const cudaError_t e = dtype == GE_LOGITS_BF16
+        ? ge_launch_step(beam_expand_sampled_kernel<GE_LOGITS_BF16>, grid, block, 0, st, *d, W, logits, logp, key, node_key, logp_out,
+                         key_out, node_key_out, parent, action, load_index, threshold)
+        : ge_launch_step(beam_expand_sampled_kernel<GE_LOGITS_F32>, grid, block, 0, st, *d, W, logits, logp, key, node_key, logp_out,
+                         key_out, node_key_out, parent, action, load_index, threshold);
+    if (e != cudaSuccess) { (void)cudaGetLastError(); return ge_set_error(GE_ERR_CUDA, "beam_expand_sampled_kernel launch: %s", cudaGetErrorString(e)); }
     return GE_OK;
 }
 

@@ -34,6 +34,7 @@
  *   ge_sample_logits  the policy side of a training loop: a masked categorical over policy logits (Gumbel-max / greedy),
  *   ge_masked_log_prob (+ _backward)  its differentiable log-prob and entropy for the update (ge_policy.cu)
  *   ge_beam_expand    one beam-search step: every beam's valid continuations scored and the W best per instance kept (ge_policy.cu)
+ *   ge_beam_expand_sampled  one stochastic-beam-search step: W distinct sequences per instance sampled without replacement
  *   ge_state_save / ge_state_load / ge_gather_instances  branching an env, i.e. copy.deepcopy(env) of a gym env: per-env state
  *                     records and instance replication for search decoders (multi-start, beam search, lookahead; ge_state.cu)
  */
@@ -368,6 +369,41 @@ int ge_masked_log_prob_backward(const void *logits, int dtype, int rows, int A, 
  * pointer (batch->mask_bits and batch->done included), or overlapping score / score_out / parent / action / load_index. */
 int ge_beam_expand(const ge_batch *batch, int W, const void *logits, int dtype, const float *score, float *score_out,
                    int32_t *parent, int32_t *action, int32_t *load_index, void *stream);
+/* One step of STOCHASTIC beam search (Kool, van Hoof, Welling 2019): the W beams of a group become W sequences drawn without
+ * replacement from the policy's sequence distribution.  Groups, batch fields, logits, parent, action, load_index, the empty-slot
+ * conventions, determinism, PDL and graph capture are those of ge_beam_expand.  Per beam b the inputs are
+ *   logp[b]      phi_b, the float32 sum of its masked log-probs (ge_beam_expand's score);
+ *   key[b]       T_b, its perturbed log-prob (conditioned Gumbel value); -inf marks a DEAD beam;
+ *   node_key[b]  a 64-bit key of the beam's tree node (its action prefix).
+ * Beam b contributes nothing when dead; when done[b], one STAY candidate (b, -1) carrying logp[b], key[b] and node_key[b]; otherwise
+ * one candidate per valid action a, with lse_b the masked log-sum-exp of ge_masked_log_prob and, all in float32:
+ *   g_a  = the Gumbel noise of ge_sample_logits with the row key replaced by node_key[b]:
+ *          h = mix32(node_key[b], a, 0x85EBCA6B), u = min(fl32((h >> 8) + 0.5) / 2^24, 1 - 2^-24), g_a = -logf(-logf(u))
+ *          (the float32 sum rounds to even once h >> 8 >= 2^23, as in ge_sample_logits; the clamp keeps the one u it rounds to 1,
+ *          where ge_sample_logits' g is +inf, below 1, so every key is finite)
+ *   s_a  = l_a + g_a (ge_sample_logits' score),  S_b = max_a s_a
+ *   phi  = logp[b] + (l_a - lse_b)                                   (bit-identical to ge_beam_expand's score)
+ *   x_a  = s_a - S_b <= 0,   D_b = T_b - (logp[b] + (S_b - lse_b))
+ *   v_a  = (D_b - x_a) + log1mexp(x_a),   log1mexp(x) = log(-expm1(x)) for x > -ln 2, log1p(-exp(x)) otherwise
+ *   G_a  = T_b - (max(v_a, 0) + log1p(exp(-|v_a|)))
+ * G_a is the stable form of -log(e^-T - e^-Z + e^-(Z + x_a)), Z = logp[b] + S_b - lse_b the largest unconditioned perturbed child:
+ * the children's keys conditioned on their maximum being T_b.  log1mexp(0) = -inf, so the best child inherits G = T_b exactly.
+ * The child's node key is (uint64) mix32(h, a, 0x2545F491) << 32 | mix32(h ^ 0x9E3779B97F4A7C15, a, 0x6C8E9CF5), h = node_key[b].
+ * graphenvs_b200.StochasticBeamSearch(venv, width, seed) starts group g (global instance i = env_id0 + g) from the root node key
+ * (uint64) mix32(seed, i, 0x52DCE729) << 32 | mix32(seed ^ 0xD1B54A32D192ED03, i, 0x52DCE729) and the root key G_root = -log(-log(u)),
+ * u = ((mix32(root node key, 0xFFFFFFFF, 0x85EBCA6B) >> 8) + 0.5) / 2^24, computed in float64 on the host and rounded to float32.
+ * Selection: stage 1 keeps each beam's W + 1 best candidates in the order (s_a desc, a asc) (in exact arithmetic the order of G_a);
+ * stage 2 fills output slot j of the group with the j-th of those lists' union in the order (G desc, parent slot asc, action asc),
+ * writing parent / action / load_index as ge_beam_expand does and logp_out = phi, key_out = G, node_key_out = the child's node key
+ * (-inf, -inf and 0 for an empty slot).  threshold [B / W] (may be NULL): per group the G of the (W+1)-th candidate of that order,
+ * -inf when the group has at most W candidates.  Starting from one root per group (logp 0, key a Gumbel(0) draw, the other slots
+ * dead), the final keys are the W largest perturbed log-probs of the complete sequences, and the largest threshold over the steps
+ * is the (W+1)-th (the kappa of the inclusion probabilities q(y) = 1 - exp(-exp(phi_y - kappa))).  GE_ERR_ARG, before any CUDA
+ * call, for an unknown dtype, W outside [1, 32], B % W != 0, a NULL pointer (threshold excepted), or any two overlapping arrays
+ * among the ten (node_key and node_key_out hold 8 bytes per env, threshold 4 bytes per group). */
+int ge_beam_expand_sampled(const ge_batch *batch, int W, const void *logits, int dtype, const float *logp, const float *key,
+                           const uint64_t *node_key, float *logp_out, float *key_out, uint64_t *node_key_out, int32_t *parent,
+                           int32_t *action, int32_t *load_index, float *threshold, void *stream);
 
 /* ---- Branching: per-env state records and instance replication (csrc/ge_state.cu) ----
  *
