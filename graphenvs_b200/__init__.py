@@ -8,6 +8,7 @@ Public surface:
   masked_log_prob(logits, mask_bits, actions)   differentiable masked log-prob + entropy for the update (policy.py)
   BeamSearch(venv, width)            beam search / multi-start decoding of a policy on the device (beam.py)
   StochasticBeamSearch(venv, width, seed)   width distinct sequences per instance sampled without replacement (beam.py)
+  MCTS(venv, num_simulations, c_puct)   Monte Carlo tree search with PUCT selection on the device (mcts.py)
   utils.vectorize_graph / devectorize_graph / get_env_info   (graph_envs/utils.py layout contract)
 """
 from .spec import ENV_SPECS, get_env_info, get_num_features  # noqa: F401
@@ -29,6 +30,9 @@ def __getattr__(attr):  # lazy: keeps `import graphenvs_b200` cheap and torch-fr
     if attr in ("BeamSearch", "StochasticBeamSearch"):
         from . import beam
         return getattr(beam, attr)
+    if attr == "MCTS":
+        from .mcts import MCTS
+        return MCTS
     if attr in ("Instance", "generate_instance"):
         from . import instances
         return getattr(instances, attr)

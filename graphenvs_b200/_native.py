@@ -90,11 +90,22 @@ class StepOut(C.Structure):
     _fields_ = [("reward", _P), ("flags", _P), ("solution_cost", _P)]
 
 
+class MctsTree(C.Structure):
+    """Mirror of `struct ge_mcts_tree` (include/graphenvs_b200.h) -- keep field order in sync."""
+    _fields_ = [
+        ("G", C.c_int32), ("S", C.c_int32), ("A", C.c_int32), ("AW", C.c_int32), ("flags", C.c_uint32), ("c_puct", C.c_double),
+        ("parent", _P), ("action", _P), ("visits", _P), ("wsum", _P), ("reward", _P), ("value", _P), ("terminal", _P),
+        ("child", _P), ("prior", _P), ("mask", _P), ("qmin", _P), ("qmax", _P),
+        ("sel_node", _P), ("sel_action", _P), ("load_index", _P), ("depth", _P),
+    ]
+
+
 EXPORTS = ["ge_abi_version", "ge_last_error", "ge_fill_layout", "ge_step_smem_bytes", "ge_build_adjacency",
            "ge_prepare", "ge_features", "ge_generate", "ge_generate_fallbacks", "ge_pool_refill", "ge_reset", "ge_step", "ge_step_sampled", "ge_sample_actions", "ge_obs_len",
            "ge_obs_flat", "ge_obs_graph", "ge_obs_nodes", "ge_step_kernel_name", "ge_batch_slice", "ge_step_host", "ge_step_host_pipelined", "ge_step_host_compact", "ge_progress_supported",
            "ge_step_host_release", "ge_mask_bytes_current", "ge_mask_bytes", "ge_stats",
            "ge_sample_logits", "ge_masked_log_prob", "ge_masked_log_prob_backward", "ge_beam_expand", "ge_beam_expand_sampled",
+           "ge_mcts_select", "ge_mcts_expand",
            "ge_state_record_bytes", "ge_state_save", "ge_state_load", "ge_gather_instances"]
 
 LOGITS_F32, LOGITS_BF16 = 0, 1   # GE_LOGITS_*
@@ -150,6 +161,9 @@ def lib():
     L.ge_masked_log_prob_backward.argtypes = [_P, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P]
     L.ge_beam_expand.argtypes = [BP, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P, _P]
     L.ge_beam_expand_sampled.argtypes = [BP, C.c_int, _P, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]
+    TP = C.POINTER(MctsTree)
+    L.ge_mcts_select.argtypes = [TP, C.c_int, _P]
+    L.ge_mcts_expand.argtypes = [TP, C.c_int, BP, _P, _P, C.c_int, _P, _P]
     L.ge_state_record_bytes.argtypes = [BP]
     L.ge_state_save.argtypes = [BP, _P, C.c_int, _P, _P]
     L.ge_state_load.argtypes = [BP, _P, C.c_int, _P, C.c_uint, _P]

@@ -1,4 +1,5 @@
-// ge_policy.cu -- masked categorical over policy logits (sm_100a): ge_sample_logits, ge_masked_log_prob and its backward.
+// ge_policy.cu -- masked categorical over policy logits (sm_100a): ge_sample_logits, ge_masked_log_prob and its backward, and the
+// search kernels built on it (beam search, stochastic beam search, Monte Carlo tree search).
 //
 // One device routine, masked_row(), is the whole reduction: for one row of logits it walks the packed valid-action mask
 // and reads ONLY the logits of set bits.  Lane l of the warp owns actions 32w + l; per nonzero mask word it loads its
@@ -505,6 +506,164 @@ __global__ void __launch_bounds__(BEAM_WARPS * 32) beam_expand_sampled_kernel(ge
     }
 }
 
+// ---- Monte Carlo tree search (ge_mcts_select / ge_mcts_expand): one warp per instance; the tree arithmetic is float64 with
+// every operation explicitly rounded (include/graphenvs_b200.h), so a float64 restatement reproduces it exactly ----
+constexpr int MCTS_WPB = 8;   // warps (= instances) per block
+
+__global__ void __launch_bounds__(MCTS_WPB * 32) mcts_select_kernel(ge_mcts_tree t, int k) {
+    pdl_launch_dependents();   // as the sampler: nothing is touched before pdl_wait()
+    pdl_wait();
+    const int lane = threadIdx.x & 31;
+    const int g = blockIdx.x * MCTS_WPB + (threadIdx.x >> 5);
+    if (g >= t.G) return;
+    const int G = t.G, A = t.A, AW = t.AW;
+    const double qmin = t.qmin[g], qmax = t.qmax[g];
+    const bool norm = qmax > qmin;
+    const double qden = norm ? __dsub_rn(qmax, qmin) : 1.0;
+    int s = 0, depth = 0, load = -1, act = -1;
+    while (!t.terminal[(size_t)s * G + g]) {   // a terminal node is revisited
+        const size_t row = (size_t)s * G + g;
+        const double sq = __dsqrt_rn((double)t.visits[row]);
+        const uint32_t *mrow = t.mask + row * AW;
+        const float *prow = t.prior + row * A;
+        const int32_t *crow = t.child + row * A;
+        double best = -INFINITY;
+        int ba = INT_MAX, bc = -1;
+        // the valid actions of s, walked as masked_row walks a mask row: lane l owns action 32 w + l of every nonzero word w
+        for (int w0 = 0; w0 < AW; w0 += 32) {
+            const int wl = w0 + lane;
+            const uint32_t mw = wl < AW ? (mrow[wl] & tail_mask(A, wl)) : 0u;
+            unsigned nz = __ballot_sync(GE_FULL, mw != 0u);
+            while (nz) {
+                const int src = __ffs((int)nz) - 1;
+                nz &= nz - 1u;
+                const uint32_t word = __shfl_sync(GE_FULL, mw, src);
+                if (!((word >> lane) & 1u)) continue;
+                const int a = ((w0 + src) << 5) + lane;
+                const int c = crow[a];
+                double q = 0.0;
+                int n = 0;
+                if (c >= 0) {
+                    const size_t rc = (size_t)c * G + g;
+                    n = t.visits[rc];
+                    if (norm) {
+                        const double Q = __dadd_rn((double)t.reward[rc], __ddiv_rn(t.wsum[rc], (double)n));
+                        q = __ddiv_rn(__dsub_rn(Q, qmin), qden);
+                    }
+                }
+                const double u = __dadd_rn(q, __ddiv_rn(__dmul_rn(__dmul_rn(t.c_puct, (double)prow[a]), sq), (double)(1 + n)));
+                if (u > best) { best = u; ba = a; bc = c; }   // strictly greater: a lane visits its actions in order
+            }
+        }
+#pragma unroll
+        for (int o = 16; o; o >>= 1) {
+            const double u2 = __shfl_xor_sync(GE_FULL, best, o);
+            const int a2 = __shfl_xor_sync(GE_FULL, ba, o);
+            const int c2 = __shfl_xor_sync(GE_FULL, bc, o);
+            if (u2 > best || (u2 == best && a2 < ba)) { best = u2; ba = a2; bc = c2; }
+        }
+        if (ba == INT_MAX) break;                          // a dead end: revisit s
+        ++depth;
+        if (bc < 0) { load = (int)row; act = ba; break; }  // an unexpanded edge: expand s by ba
+        s = bc;
+    }
+    if (lane == 0) {
+        t.sel_node[g] = s;
+        t.sel_action[g] = act;
+        t.load_index[g] = load;
+        t.depth[g] = depth;
+    }
+}
+
+template <int DT>
+__global__ void __launch_bounds__(MCTS_WPB * 32) mcts_expand_kernel(ge_batch d, ge_mcts_tree t, int k, const float *__restrict__ reward,
+                                                                     const void *__restrict__ logits, const float *__restrict__ value) {
+    pdl_launch_dependents();   // as the sampler: nothing is touched before pdl_wait()
+    pdl_wait();
+    const int lane = threadIdx.x & 31;
+    const int g = blockIdx.x * MCTS_WPB + (threadIdx.x >> 5);
+    if (g >= t.G) return;
+    const int G = t.G, A = t.A, AW = t.AW;
+    const size_t rk = (size_t)k * G + g;
+    const int a = k ? t.sel_action[g] : -1;
+    const int par = k ? t.sel_node[g] : -1;
+    int leaf = par;                                        // a revisit backs up from the selected node
+    if (k == 0 || a >= 0) {                                // node k: its mask, and over its valid actions its priors and no child
+        const size_t esz = DT == GE_LOGITS_BF16 ? 2 : 4;
+        const void *row = reinterpret_cast<const char *>(logits) + (size_t)g * A * esz;
+        const uint32_t *lm = d.mask_bits + (size_t)g * d.AW;
+        const float lse = row_lse(masked_row<DT, MODE_STATS>(row, lm, A, AW, 0, lane));
+        uint32_t *nm = t.mask + rk * AW;
+        float *prow = t.prior + rk * A;
+        int32_t *crow = t.child + rk * A;
+        for (int w0 = 0; w0 < AW; w0 += 32) {
+            const int wl = w0 + lane;
+            const uint32_t mw = wl < AW ? (__ldg(lm + wl) & tail_mask(A, wl)) : 0u;
+            if (wl < AW) nm[wl] = mw;
+            unsigned nz = __ballot_sync(GE_FULL, mw != 0u);
+            while (nz) {
+                const int src = __ffs((int)nz) - 1;
+                nz &= nz - 1u;
+                const uint32_t word = __shfl_sync(GE_FULL, mw, src);
+                if ((word >> lane) & 1u) {
+                    const int i = ((w0 + src) << 5) + lane;
+                    prow[i] = expf(__fsub_rn(load_logit<DT>(row, (size_t)i), lse));
+                    crow[i] = -1;
+                }
+            }
+        }
+        if (lane == 0) {
+            const bool term = d.done[g] != 0;
+            t.parent[rk] = par;
+            t.action[rk] = a;
+            t.reward[rk] = k ? reward[g] : 0.f;
+            t.terminal[rk] = term;
+            t.value[rk] = term ? 0.f : value[g];
+            t.visits[rk] = 0;
+            t.wsum[rk] = 0.0;
+            if (k) t.child[((size_t)par * G + g) * A + a] = k;
+            else { t.qmin[g] = INFINITY; t.qmax[g] = -INFINITY; }
+        }
+        leaf = k;
+    } else if (lane == 0) {                                // slot k stays unused
+        t.parent[rk] = -1;
+        t.action[rk] = -1;
+        t.visits[rk] = 0;
+    }
+    if (lane != 0) return;
+    // backup (MuZero's order): from the leaf up to and including the root
+    double ret = (double)t.value[(size_t)leaf * G + g];
+    double qmin = t.qmin[g], qmax = t.qmax[g];
+    for (int c = leaf;;) {
+        const size_t rc = (size_t)c * G + g;
+        const int n = t.visits[rc] + 1;
+        const double w = __dadd_rn(t.wsum[rc], ret);
+        t.visits[rc] = n;
+        t.wsum[rc] = w;
+        if (c == 0) break;
+        const double r = (double)t.reward[rc];
+        const double Q = __dadd_rn(r, __ddiv_rn(w, (double)n));
+        qmin = fmin(qmin, Q);
+        qmax = fmax(qmax, Q);
+        ret = __dadd_rn(r, ret);
+        c = t.parent[rc];
+    }
+    t.qmin[g] = qmin;
+    t.qmax[g] = qmax;
+}
+
+int check_tree(const char *fn, const ge_mcts_tree *t, int k, int kmin) {
+    if (!t) return ge_set_error(GE_ERR_ARG, "%s: null tree", fn);
+    if (t->G < 1 || t->S < 1 || t->A < 1 || t->AW != (t->A + 31) / 32)
+        return ge_set_error(GE_ERR_ARG, "%s: bad tree shape G=%d S=%d A=%d AW=%d", fn, t->G, t->S, t->A, t->AW);
+    if (!isfinite(t->c_puct) || t->c_puct < 0.0) return ge_set_error(GE_ERR_ARG, "%s: c_puct = %g must be finite and >= 0", fn, t->c_puct);
+    if (k < kmin || k > t->S) return ge_set_error(GE_ERR_ARG, "%s: k = %d not in [%d, %d]", fn, k, kmin, t->S);
+    if (!t->parent || !t->action || !t->visits || !t->wsum || !t->reward || !t->value || !t->terminal || !t->child || !t->prior ||
+        !t->mask || !t->qmin || !t->qmax || !t->sel_node || !t->sel_action || !t->load_index || !t->depth)
+        return ge_set_error(GE_ERR_ARG, "%s: null tree array", fn);
+    return GE_OK;
+}
+
 int launched(const char *what) {
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? GE_OK : ge_set_error(GE_ERR_CUDA, "%s launch: %s", what, cudaGetErrorString(e));
@@ -632,6 +791,45 @@ int ge_beam_expand_sampled(const ge_batch *d, int W, const void *logits, int dty
         : ge_launch_step(beam_expand_sampled_kernel<GE_LOGITS_F32>, grid, block, 0, st, *d, W, logits, logp, key, node_key, logp_out,
                          key_out, node_key_out, parent, action, load_index, threshold);
     if (e != cudaSuccess) { (void)cudaGetLastError(); return ge_set_error(GE_ERR_CUDA, "beam_expand_sampled_kernel launch: %s", cudaGetErrorString(e)); }
+    return GE_OK;
+}
+
+int ge_mcts_select(const ge_mcts_tree *tree, int k, void *stream) {
+    GE_NVTX("ge_mcts_select");
+    const int rc = check_tree("ge_mcts_select", tree, k, 1);
+    if (rc) return rc;
+    cudaLaunchConfig_t cfg = {};   // ge_launch_step's launch, with the PDL flag of the tree
+    cfg.gridDim = dim3((unsigned)((tree->G + MCTS_WPB - 1) / MCTS_WPB));
+    cfg.blockDim = dim3(MCTS_WPB * 32);
+    cfg.stream = (cudaStream_t)stream;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = at;
+    cfg.numAttrs = (tree->flags & GE_FLAG_PDL) ? 1 : 0;
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, mcts_select_kernel, *tree, k);
+    if (e != cudaSuccess) { (void)cudaGetLastError(); return ge_set_error(GE_ERR_CUDA, "mcts_select_kernel launch: %s", cudaGetErrorString(e)); }
+    return GE_OK;
+}
+
+int ge_mcts_expand(const ge_mcts_tree *tree, int k, const ge_batch *leaf, const float *reward, const void *logits, int dtype,
+                   const float *value, void *stream) {
+    GE_NVTX("ge_mcts_expand");
+    const char *fn = "ge_mcts_expand";
+    const int rc = check_tree(fn, tree, k, 0);
+    if (rc) return rc;
+    if (!leaf) return ge_set_error(GE_ERR_ARG, "%s: null leaf batch", fn);
+    if (dtype != GE_LOGITS_F32 && dtype != GE_LOGITS_BF16) return ge_set_error(GE_ERR_ARG, "%s: unknown logits dtype %d", fn, dtype);
+    if (leaf->B != tree->G || leaf->A != tree->A || leaf->AW != tree->AW)
+        return ge_set_error(GE_ERR_ARG, "%s: leaf batch B=%d A=%d AW=%d, tree G=%d A=%d AW=%d", fn, leaf->B, leaf->A, leaf->AW, tree->G, tree->A, tree->AW);
+    if (!reward || !logits || !value) return ge_set_error(GE_ERR_ARG, "%s: null reward / logits / value", fn);
+    if (!leaf->mask_bits || !leaf->done) return ge_set_error(GE_ERR_ARG, "%s: null mask_bits / done in the leaf batch", fn);
+    const dim3 grid((unsigned)((tree->G + MCTS_WPB - 1) / MCTS_WPB)), block(MCTS_WPB * 32);
+    cudaStream_t st = (cudaStream_t)stream;
+    const cudaError_t e = dtype == GE_LOGITS_BF16
+        ? ge_launch_step(mcts_expand_kernel<GE_LOGITS_BF16>, grid, block, 0, st, *leaf, *tree, k, reward, logits, value)
+        : ge_launch_step(mcts_expand_kernel<GE_LOGITS_F32>, grid, block, 0, st, *leaf, *tree, k, reward, logits, value);
+    if (e != cudaSuccess) { (void)cudaGetLastError(); return ge_set_error(GE_ERR_CUDA, "mcts_expand_kernel launch: %s", cudaGetErrorString(e)); }
     return GE_OK;
 }
 

@@ -35,6 +35,7 @@
  *   ge_masked_log_prob (+ _backward)  its differentiable log-prob and entropy for the update (ge_policy.cu)
  *   ge_beam_expand    one beam-search step: every beam's valid continuations scored and the W best per instance kept (ge_policy.cu)
  *   ge_beam_expand_sampled  one stochastic-beam-search step: W distinct sequences per instance sampled without replacement
+ *   ge_mcts_select / ge_mcts_expand  Monte Carlo tree search (PUCT): one simulation round's selection and its expansion + backup
  *   ge_state_save / ge_state_load / ge_gather_instances  branching an env, i.e. copy.deepcopy(env) of a gym env: per-env state
  *                     records and instance replication for search decoders (multi-start, beam search, lookahead; ge_state.cu)
  */
@@ -404,6 +405,77 @@ int ge_beam_expand(const ge_batch *batch, int W, const void *logits, int dtype, 
 int ge_beam_expand_sampled(const ge_batch *batch, int W, const void *logits, int dtype, const float *logp, const float *key,
                            const uint64_t *node_key, float *logp_out, float *key_out, uint64_t *node_key_out, int32_t *parent,
                            int32_t *action, int32_t *load_index, float *threshold, void *stream);
+
+/* ---- Monte Carlo tree search with PUCT selection (AlphaZero / MuZero style; csrc/ge_policy.cu) ----
+ *
+ * G instances are searched in parallel, each with S simulations run one after another.  Node 0 of every instance is its root;
+ * simulation k (1 <= k <= S) creates at most node k of every instance, so a tree has S + 1 node slots and node n of instance g
+ * sits at row n * G + g of every per-node array.  The caller keeps one env state record per node, [S + 1, G, R] (ge_state_save),
+ * and a leaf batch of G envs, and runs one simulation round as
+ *   ge_mcts_select(tree, k)                                   -> load_index, sel_action, depth
+ *   ge_state_load(leaf, records, (S + 1) * G, load_index)     the parent node's state (a revisit loads nothing)
+ *   ge_step(leaf, sel_action)                                 -1 for a revisit: GE_STEP_INVALID / AFTER_DONE, state unchanged
+ *   policy(leaf) -> logits [G, A], value [G]
+ *   ge_state_save(leaf, NULL, G, records + k * G * R)
+ *   ge_mcts_expand(tree, k, leaf, step reward, logits, value)
+ * and starts a search with ge_mcts_expand(tree, 0, ...) on the leaf batch holding the root states (and their records in row 0).
+ *
+ * Per node n: parent, action (of the edge into n; -1 at the root), r (float32 step reward on that edge, 0 at the root),
+ * terminal (the leaf's done after that step), v (float32 policy value at expansion, 0 when terminal), N (visits) and Wsum
+ * (float64 sum of backed-up returns), and over the node's VALID actions only -- its packed mask, copied from the leaf's
+ * mask_bits -- the prior P(n, a) = expf(fl32(l_a - lse)) (lse the masked log-sum-exp of ge_masked_log_prob, bit for bit) and
+ * child(n, a) (-1 = unexpanded).  Entries of invalid actions are never written or read.  A node slot k that round k did not
+ * create (the round revisited a node) gets N = 0, parent = action = -1; every created node has N >= 1.
+ * value[g] estimates the undiscounted sum of future rewards from the leaf (discount 1: episodes are finite).
+ *
+ * Arithmetic: float64 with explicitly rounded operations (no FMA contraction), so a plain float64 restatement is exact:
+ *   Q(s, a) = r(c) + Wsum(c) / N(c)                                         for the child c of s by a
+ *   qbar    = (Q - qmin) / (qmax - qmin) when qmax > qmin, else 0;  0 for an unexpanded edge      (MuZero min-max normalization)
+ *   u(s, a) = qbar + ((c_puct * P(s, a)) * sqrt(N(s))) / (1 + N(s, a)),  N(s, a) = N(c), 0 when unexpanded
+ * qmin / qmax (per instance, +inf / -inf at the start) run over every Q computed in a backup.
+ * Select (k >= 1), one warp per instance from the root: at a node s that is terminal, or that has no valid action (a dead end),
+ * stop and REVISIT s; otherwise take the valid action of largest u (ties to the lowest action); an unexpanded edge stops there
+ * (EXPAND s by a), an edge into a terminal child stops there (revisit the child), any other edge descends.  A terminal or done
+ * root is revisited on every simulation.  Outputs per instance: load_index = s * G + g and sel_action = a for an expansion,
+ * -1 and -1 for a revisit; depth = the depth of the new or revisited node (root 0); sel_node = s or the revisited node.
+ * Expand and backup (k >= 0): k = 0 makes node 0 from the leaf's current state (r = 0, terminal = done, v), resets qmin / qmax;
+ * k >= 1 with sel_action[g] = a >= 0 makes node k with parent sel_node[g], action a, r = reward[g], terminal = done[g], v, and
+ * sets child(s, a) = k.  Then from the new (or revisited) node with ret = its v, for each node c up to and including the root:
+ *   N(c) += 1;  Wsum(c) += ret;  if c is not the root: qmin / qmax absorb r(c) + Wsum(c) / N(c), and ret = r(c) + ret.
+ * So the root's expansion is its first visit (N = 1, Wsum = v) and after S simulations N(root) = S + 1.
+ * No atomics and no noise: results depend only on the inputs.  Both kernels touch nothing before pdl_wait(): select launches
+ * with programmatic stream serialization when tree->flags has GE_FLAG_PDL, expand when leaf->flags has it.  No allocation or
+ * synchronisation: a whole search can be captured in a CUDA graph.  GE_ERR_ARG, before any CUDA call, for a NULL pointer,
+ * G < 1, S < 1, A < 1, AW != ceil(A / 32), a non-finite or negative c_puct, k outside [1, S] (select) / [0, S] (expand), an
+ * unknown dtype, leaf->B != G, leaf->A != A, or a NULL leaf->mask_bits / leaf->done.
+ * Memory per node: R + 8 A + 4 AW + 29 bytes (record, child + prior, mask, the scalars), plus 32 bytes per instance. */
+typedef struct ge_mcts_tree {
+    int32_t G, S, A, AW;          /* instances, simulations, mask length and its words */
+    uint32_t flags;               /* GE_FLAG_PDL: ge_mcts_select launches with programmatic stream serialization */
+    double c_puct;                /* >= 0, finite */
+    int32_t *parent;              /* [S + 1, G]     parent node, -1 at the root and in an unused slot */
+    int32_t *action;              /* [S + 1, G]     action of the edge into the node, -1 at the root and in an unused slot */
+    int32_t *visits;              /* [S + 1, G]     N */
+    double *wsum;                 /* [S + 1, G]     Wsum */
+    float *reward;                /* [S + 1, G]     r */
+    float *value;                 /* [S + 1, G]     v */
+    uint8_t *terminal;            /* [S + 1, G] */
+    int32_t *child;               /* [S + 1, G, A]  valid actions only */
+    float *prior;                 /* [S + 1, G, A]  valid actions only */
+    uint32_t *mask;               /* [S + 1, G, AW] packed valid-action mask of the node */
+    double *qmin, *qmax;          /* [G] */
+    int32_t *sel_node;            /* [G] the current simulation's selection (select writes it, expand reads it) */
+    int32_t *sel_action;          /* [G] */
+    int32_t *load_index;          /* [G] */
+    int32_t *depth;               /* [G] */
+} ge_mcts_tree;
+/* Selection of simulation k (1 <= k <= S): writes sel_node, sel_action, load_index and depth of every instance. */
+int ge_mcts_select(const ge_mcts_tree *tree, int k, void *stream);
+/* Expansion and backup of simulation k (0 <= k <= S) from the leaf batch (G envs: leaf->done, leaf->mask_bits), the step's
+ * reward [G] (read for k >= 1 only, but required), the policy's logits [G, A] (layout and dtype of ge_sample_logits) and
+ * value [G] float32. */
+int ge_mcts_expand(const ge_mcts_tree *tree, int k, const ge_batch *leaf, const float *reward, const void *logits, int dtype,
+                   const float *value, void *stream);
 
 /* ---- Branching: per-env state records and instance replication (csrc/ge_state.cu) ----
  *
