@@ -26,6 +26,9 @@ constexpr int LANE_T = 32;
 // __launch_bounds__ of the lane kernels.  It sets their register budget: with a bound of 32 the compiler gives the
 // step kernels 63 instead of 56 registers, a build nobody has measured.
 constexpr int LANE_BOUND = 128;
+// Minimum resident blocks of LANE_BOUND threads the step kernels declare: a cap of 65,536 / (128 x 8) = 64 registers.  The
+// unstaged step kernels run 32 one-warp blocks per SM at 64; left to itself ptxas gives them 56 and spills 12 bytes.
+constexpr int LANE_STEP_MIN_BLOCKS = 8;
 
 namespace {
 
@@ -216,6 +219,23 @@ __device__ __forceinline__ u64 load_bits64(const uint32_t *base, int b, int NW) 
     return (u64)t.x | ((u64)t.y << 32);
 }
 
+// Before pdl_wait() the previous launch may still be writing the dynamic state.  These two touch it without being able to
+// hand a stale value to the loads after the wait: an L2 prefetch moves no data into the SM, and an L2 load (ld.global.cg, no
+// L1 allocation) returns a value that only steers such a prefetch.  L2 is the point of coherence, so the loads after the
+// wait see the previous launch's writes either way.
+__device__ __forceinline__ void prefetch_l2(const void *p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
+__device__ __forceinline__ uint32_t load_l2(const uint32_t *p) {
+    uint32_t v;
+    asm volatile("ld.global.cg.u32 %0, [%1];" : "=r"(v) : "l"(p));
+    return v;
+}
+__device__ __forceinline__ u64 load_l2_bits64(const uint32_t *base, int b, int NW) {
+    if (NW == 1) return (u64)load_l2(base + b);
+    u64 v;
+    asm volatile("ld.global.cg.u64 %0, [%1];" : "=l"(v) : "l"(base + 2 * (size_t)b));
+    return v;
+}
+
 // Stages the adjacency tiles of the block's envs (blockDim.x / 32 tiles of 32 envs, contiguous) with one bulk
 // copy; returns this env's rows.
 template <bool STAGED>
@@ -239,6 +259,14 @@ __device__ __forceinline__ Rows<STAGED> stage_rows(const ge_batch &d, int b0, ui
     return R;
 }
 
+// *p += v as a fire-and-forget reduction (SASS REDG.E.ADD.F64.RN): the SM neither loads the statistics rows nor waits for
+// them.  Every element has one writer per launch and launches are ordered by grid completion, and the fp64 reduction rounds
+// to nearest even like the `*p + v` of a load-add-store, so the rows are bit-identical to one.  Explicit PTX because ptxas
+// keeps an atomicAdd whose result is unused an ATOMG (which returns) when a fence may follow, as signal_progress's does.
+__device__ __forceinline__ void red_add(double *p, double v) {
+    asm volatile("red.relaxed.gpu.global.add.f64 [%0], %1;" ::"l"(p), "d"(v) : "memory");
+}
+
 // r-th set bit of a 64-bit mask, r uniform from the counter RNG (same draw as ge_common.cuh:warp_sample).
 __device__ __forceinline__ int lane_sample(u64 m, uint64_t seed, uint32_t env, uint32_t t) {
     int total = __popcll(m);
@@ -250,25 +278,54 @@ __device__ __forceinline__ int lane_sample(u64 m, uint64_t seed, uint32_t env, u
 }
 
 template <bool STAGED, bool SAMPLED>
-__global__ void __launch_bounds__(LANE_BOUND) lane_step_kernel(ge_batch d, int32_t *__restrict__ actions, ge_step_out out,
+__global__ void __launch_bounds__(LANE_BOUND, LANE_STEP_MIN_BLOCKS) lane_step_kernel(ge_batch d, int32_t *__restrict__ actions, ge_step_out out,
                                                             uint64_t seed, uint32_t t) {
     extern __shared__ __align__(128) uint32_t smem[];
     __shared__ __align__(8) uint64_t bar;
     const int b0 = blockIdx.x * blockDim.x, b = b0 + threadIdx.x;
     // Programmatic dependent launch (ge_common.cuh:pdl_*; no-ops on a plain launch): the next launch in the stream may
-    // become resident now, and everything up to pdl_wait() touches only STATIC instance data (the adjacency tiles), so
-    // it runs under the tail of the previous launch.
+    // become resident now, and everything up to pdl_wait() reads only STATIC instance data (the adjacency tiles, dest, src,
+    // the reset-time mask) or reaches the dynamic state through L2 alone (prefetch_l2 / load_l2), so it runs under the tail
+    // of the previous launch.  A stream that steps other batches in between (sub-batch chains rotating over batches) leaves
+    // this batch's state final while the block waits, and the block's loads after the wait hit L2.
     pdl_launch_dependents();
     Rows<STAGED> R = stage_rows<STAGED>(d, b0, smem, &bar);
     const bool live = b < d.B;
     const int N = d.N, kind = d.kind;
     const u64 full = N == 64 ? ~0ull : ((1ull << N) - 1ull);
+    const bool needs_w = kind == GE_SHORTEST_PATH || kind == GE_LONGEST_PATH || kind == GE_TSP;
+    int dest = 0, src = 0;
+    u64 mask0 = 0;
+    if (live) {
+        if (kind == GE_SHORTEST_PATH || kind == GE_LONGEST_PATH) { dest = d.dest[b]; src = d.src[b]; }
+        if (d.mask0_bits && (d.flags & GE_FLAG_AUTO_RESET)) mask0 = load_bits64(d.mask0_bits, b, d.AW);
+        prefetch_l2(d.node_bits + (size_t)b * d.NW);
+        if (d.node_bits2) prefetch_l2(d.node_bits2 + (size_t)b * d.NW);
+        prefetch_l2(d.cost + b);
+        prefetch_l2(d.done + b);
+        if (d.traj) prefetch_l2(d.traj + b);
+        if (kind == GE_DENSEST_SUBGRAPH) prefetch_l2(d.counters + (size_t)b * 4);
+        if (!SAMPLED) prefetch_l2(actions + b);
+        if (SAMPLED && needs_w) {
+            // Guess this step's draw from the state as it is now and prefetch its edge weight, the step's one dependent
+            // load.  Right whenever the previous launch did not step this batch; a wrong guess costs one wasted line.
+            const u64 m = load_l2_bits64(d.mask_bits, b, d.AW);
+            const uint32_t ns = d.env_steps ? load_l2(d.env_steps + b) : 0u;
+            const int h = min(max((int)load_l2(reinterpret_cast<const uint32_t *>(d.head) + b), 0), N - 1);
+            const int ga = min(max(lane_sample(m, seed, (uint32_t)(d.env_id0 + b), t + ns), 0), N - 1);
+            prefetch_l2(d.wmat + ((size_t)b * N + h) * N + ga);
+        } else {
+            prefetch_l2(d.head + b);
+            prefetch_l2(d.mask_bits + (size_t)b * d.AW);
+            if (d.env_steps) prefetch_l2(d.env_steps + b);
+        }
+    }
     pdl_wait();
     // scalar state (coalesced SoA streams) while the bulk copy is in flight
     LState s;
-    int a = -1, dest = 0, src = 0;
-    u64 oldmask = 0, cs = 0, mask0 = 0;
-    double acc_r = 0.0, w_edge = 0.0;
+    int a = -1;
+    u64 oldmask = 0, cs = 0;
+    double w_edge = 0.0;
     float w_node = 0.f;
     bool was_done = false;
     uint32_t nsteps = 0;
@@ -287,12 +344,8 @@ __global__ void __launch_bounds__(LANE_BOUND) lane_step_kernel(ge_batch d, int32
             actions[b] = a;
         }
         was_done = d.done[b] != 0;
-        if (kind == GE_SHORTEST_PATH || kind == GE_LONGEST_PATH) { dest = d.dest[b]; src = d.src[b]; }
-        acc_r = d.acc[2 * (size_t)d.acc_stride + b];
-        if (d.mask0_bits && (d.flags & GE_FLAG_AUTO_RESET)) mask0 = load_bits64(d.mask0_bits, b, d.AW);
         if (d.traj) cs = d.traj[b];
         // the one dependent load of the step, issued before waiting for the staged rows
-        const bool needs_w = kind == GE_SHORTEST_PATH || kind == GE_LONGEST_PATH || kind == GE_TSP;
         if (needs_w && a >= 0 && a < N) w_edge = lane_edge_weight(d, b, s.head, a);
         if (kind == GE_MAX_INDEPENDENT_SET && a >= 0 && a < N) w_node = d.node_cost[(size_t)b * N + a];
     }
@@ -385,25 +438,12 @@ __global__ void __launch_bounds__(LANE_BOUND) lane_step_kernel(ge_batch d, int32
         d.traj[b] = ((cs << 7) | (cs >> 57)) ^ (u64)(uint32_t)a ^ ((u64)done << 40) ^ ((u64)(solved & 3) << 44) ^ ((u64)status << 48);
     if (status == GE_STEP_OK) {
         if (d.env_steps) d.env_steps[b] = nsteps + 1u;
-        d.acc[2 * (size_t)d.acc_stride + b] = acc_r + reward;
+        const size_t st = (size_t)d.acc_stride;
+        red_add(d.acc + 2 * st + b, reward);
         if (done) {
-            if (STAGED) {
-                d.acc[b] += 1.0;
-                if (solved == 1) d.acc[(size_t)d.acc_stride + b] += 1.0;
-                if (sol == sol) d.acc[3 * (size_t)d.acc_stride + b] += sol;
-            } else {
-                // The unstaged kernels load the three rows before storing any: one memory round trip at the end of the warp
-                // instead of three dependent ones (each `+=` waits for the previous store, which may alias).  cfg1: 9.55 ->
-                // 10.8 G env-steps/s.  The staged kernels keep the `+=`: with the rows loaded together (or at the top of
-                // the kernel) their cfg2 streaming step measured slower (DESIGN §6b).
-                const size_t st = (size_t)d.acc_stride;
-                const double episodes = d.acc[b];
-                const double n_solved = solved == 1 ? d.acc[st + b] : 0.0;
-                const double cost_sum = sol == sol ? d.acc[3 * st + b] : 0.0;
-                d.acc[b] = episodes + 1.0;
-                if (solved == 1) d.acc[st + b] = n_solved + 1.0;
-                if (sol == sol) d.acc[3 * st + b] = cost_sum + sol;
-            }
+            red_add(d.acc + b, 1.0);
+            if (solved == 1) red_add(d.acc + st + b, 1.0);
+            if (sol == sol) red_add(d.acc + 3 * st + b, sol);
         }
     }
     if (done && (d.flags & GE_FLAG_AUTO_RESET)) {                               // tail of reset()

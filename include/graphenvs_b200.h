@@ -77,11 +77,14 @@ typedef enum {
 #define GE_FLAG_UNWEIGHTED 4u   /* ge_generate: weighted=False (all edge weights / MIS costs 1.0) */
 #define GE_FLAG_FORCE_WARP 8u   /* testing: use the warp-per-env kernels even where the lane-per-env ones apply */
 #define GE_FLAG_PDL 16u         /* ge_step / ge_step_sampled launch with programmatic stream serialization: the step kernel may become
-                                   resident -- and prefetch STATIC instance data (adjacency tiles, automaton tables) -- while the previous
-                                   launch of the stream is still running; it waits for that launch (griddepcontrol.wait) before it touches
-                                   any env state.  The caller promises that the preceding work in the stream does not write this batch's
-                                   static arrays (i.e. it is another step or a state save / load, not ge_generate / ge_build_adjacency /
-                                   ge_pool_refill / ge_gather_instances). */
+                                   resident -- and read STATIC instance data (adjacency tiles, automaton tables, src / dest, the
+                                   reset-time mask) -- while the previous launch of the stream is still running; it waits for that launch
+                                   (griddepcontrol.wait) before it uses any env state.  Before the wait it may only prefetch env state
+                                   into L2, or read it through L2 to pick what to prefetch (the lane-per-env step guesses its draw that
+                                   way); such reads are never used as results, and L2 is coherent, so the loads after the wait see the
+                                   previous launch's writes.  The caller promises that the preceding work in the stream does not write
+                                   this batch's static arrays (i.e. it is another step or a state save / load, not ge_generate /
+                                   ge_build_adjacency / ge_pool_refill / ge_gather_instances). */
 
 /* per-env status written by ge_step into flags[b].status */
 #define GE_STEP_OK 0
