@@ -9,6 +9,8 @@ Public surface:
   BeamSearch(venv, width)            beam search / multi-start decoding of a policy on the device (beam.py)
   StochasticBeamSearch(venv, width, seed)   width distinct sequences per instance sampled without replacement (beam.py)
   MCTS(venv, num_simulations, c_puct)   Monte Carlo tree search with PUCT selection on the device (mcts.py)
+  GumbelMCTS(venv, num_simulations, max_considered, ...)   Gumbel MuZero search: sequential halving at the root, improved-policy
+                                     targets (mcts.py)
   utils.vectorize_graph / devectorize_graph / get_env_info   (graph_envs/utils.py layout contract)
 """
 from .spec import ENV_SPECS, get_env_info, get_num_features  # noqa: F401
@@ -30,9 +32,9 @@ def __getattr__(attr):  # lazy: keeps `import graphenvs_b200` cheap and torch-fr
     if attr in ("BeamSearch", "StochasticBeamSearch"):
         from . import beam
         return getattr(beam, attr)
-    if attr == "MCTS":
-        from .mcts import MCTS
-        return MCTS
+    if attr in ("MCTS", "GumbelMCTS"):
+        from . import mcts
+        return getattr(mcts, attr)
     if attr in ("Instance", "generate_instance"):
         from . import instances
         return getattr(instances, attr)

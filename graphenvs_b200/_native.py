@@ -100,12 +100,17 @@ class MctsTree(C.Structure):
     ]
 
 
+class GumbelParams(C.Structure):
+    """Mirror of `struct ge_gumbel_params` (include/graphenvs_b200.h) -- keep field order in sync."""
+    _fields_ = [("m", C.c_int32), ("value_scale", C.c_double), ("maxvisit_init", C.c_double), ("table", _P), ("noise", _P)]
+
+
 EXPORTS = ["ge_abi_version", "ge_last_error", "ge_fill_layout", "ge_step_smem_bytes", "ge_build_adjacency",
            "ge_prepare", "ge_features", "ge_generate", "ge_generate_fallbacks", "ge_pool_refill", "ge_reset", "ge_step", "ge_step_sampled", "ge_sample_actions", "ge_obs_len",
            "ge_obs_flat", "ge_obs_graph", "ge_obs_nodes", "ge_step_kernel_name", "ge_batch_slice", "ge_step_host", "ge_step_host_pipelined", "ge_step_host_compact", "ge_progress_supported",
            "ge_step_host_release", "ge_mask_bytes_current", "ge_mask_bytes", "ge_stats",
            "ge_sample_logits", "ge_masked_log_prob", "ge_masked_log_prob_backward", "ge_beam_expand", "ge_beam_expand_sampled",
-           "ge_mcts_select", "ge_mcts_expand",
+           "ge_mcts_select", "ge_mcts_expand", "ge_gumbel_root", "ge_gumbel_select", "ge_gumbel_result",
            "ge_state_record_bytes", "ge_state_save", "ge_state_load", "ge_gather_instances"]
 
 LOGITS_F32, LOGITS_BF16 = 0, 1   # GE_LOGITS_*
@@ -164,6 +169,10 @@ def lib():
     TP = C.POINTER(MctsTree)
     L.ge_mcts_select.argtypes = [TP, C.c_int, _P]
     L.ge_mcts_expand.argtypes = [TP, C.c_int, BP, _P, _P, C.c_int, _P, _P]
+    GP = C.POINTER(GumbelParams)
+    L.ge_gumbel_root.argtypes = [TP, GP, C.c_uint64, C.c_uint32, C.c_int32, _P]
+    L.ge_gumbel_select.argtypes = [TP, GP, C.c_int, _P]
+    L.ge_gumbel_result.argtypes = [TP, GP, _P, _P, _P, _P]
     L.ge_state_record_bytes.argtypes = [BP]
     L.ge_state_save.argtypes = [BP, _P, C.c_int, _P, _P]
     L.ge_state_load.argtypes = [BP, _P, C.c_int, _P, C.c_uint, _P]

@@ -1,5 +1,5 @@
 // ge_policy.cu -- masked categorical over policy logits (sm_100a): ge_sample_logits, ge_masked_log_prob and its backward, and the
-// search kernels built on it (beam search, stochastic beam search, Monte Carlo tree search).
+// search kernels built on it (beam search, stochastic beam search, Monte Carlo tree search with PUCT and with Gumbel MuZero selection).
 //
 // One device routine, masked_row(), is the whole reduction: for one row of logits it walks the packed valid-action mask
 // and reads ONLY the logits of set bits.  Lane l of the warp owns actions 32w + l; per nonzero mask word it loads its
@@ -11,6 +11,7 @@
 // merged across the warp by a shuffle butterfly in a fixed order.  Then lse = mx + log(se) and H = log(se) - st / se
 // (= lse - sum p l without the cancellation of two large terms).  Every kernel calls the same routine with the same
 // arithmetic, so the sampler's log_prob / entropy equal the forward kernel's bit for bit; there are no atomics.
+#include <cfloat>
 #include <climits>
 #include <cstdio>
 #include <cuda_bf16.h>
@@ -575,7 +576,7 @@ __global__ void __launch_bounds__(MCTS_WPB * 32) mcts_select_kernel(ge_mcts_tree
     }
 }
 
-template <int DT>
+template <int DT, bool LOG_PRIOR>
 __global__ void __launch_bounds__(MCTS_WPB * 32) mcts_expand_kernel(ge_batch d, ge_mcts_tree t, int k, const float *__restrict__ reward,
                                                                      const void *__restrict__ logits, const float *__restrict__ value) {
     pdl_launch_dependents();   // as the sampler: nothing is touched before pdl_wait()
@@ -607,7 +608,8 @@ __global__ void __launch_bounds__(MCTS_WPB * 32) mcts_expand_kernel(ge_batch d, 
                 const uint32_t word = __shfl_sync(GE_FULL, mw, src);
                 if ((word >> lane) & 1u) {
                     const int i = ((w0 + src) << 5) + lane;
-                    prow[i] = expf(__fsub_rn(load_logit<DT>(row, (size_t)i), lse));
+                    const float lp = __fsub_rn(load_logit<DT>(row, (size_t)i), lse);
+                    prow[i] = LOG_PRIOR ? lp : expf(lp);   // GE_MCTS_LOG_PRIOR: the log-prior of the Gumbel search
                     crow[i] = -1;
                 }
             }
@@ -652,6 +654,227 @@ __global__ void __launch_bounds__(MCTS_WPB * 32) mcts_expand_kernel(ge_batch d, 
     t.qmax[g] = qmax;
 }
 
+// ---- Gumbel MuZero search (ge_gumbel_root / ge_gumbel_select / ge_gumbel_result): one warp per instance over a GE_MCTS_LOG_PRIOR
+// tree, with the arithmetic of include/graphenvs_b200.h (float64, every operation explicitly rounded, fixed reduction order) ----
+
+// f(a) for every valid action a of a node, walked as mcts_select_kernel walks it: lane l takes the actions a = l mod 32, ascending.
+// f runs on the lanes that own a valid action only, so it must not use warp collectives.
+template <class F>
+__device__ __forceinline__ void for_valid(const uint32_t *mrow, int A, int AW, int lane, F f) {
+    for (int w0 = 0; w0 < AW; w0 += 32) {
+        const int wl = w0 + lane;
+        const uint32_t mw = wl < AW ? (mrow[wl] & tail_mask(A, wl)) : 0u;
+        unsigned nz = __ballot_sync(GE_FULL, mw != 0u);
+        while (nz) {
+            const int src = __ffs((int)nz) - 1;
+            nz &= nz - 1u;
+            const uint32_t word = __shfl_sync(GE_FULL, mw, src);
+            if ((word >> lane) & 1u) f(((w0 + src) << 5) + lane);
+        }
+    }
+}
+
+// Node s of instance g with the statistics of its completed Q (warp-uniform).
+struct GNode {
+    const uint32_t *mrow;
+    const float *lrow;     // log-priors l(s, a)
+    const int32_t *crow;
+    double vmix, lo, den, cs;   // q~ = (q^ - lo) / den, sigma = cs * q~
+    int M, maxn, nvalid;
+};
+
+// N(s, a) of the edge (c = its child, -1 when unexpanded) and q^(a), which is Q(s, a) when N > 0 and vmix otherwise.
+__device__ __forceinline__ double edge_q(const ge_mcts_tree &t, const int32_t *crow, int a, int g, double vmix, int &n, int &c) {
+    c = crow[a];
+    n = 0;
+    if (c >= 0) {
+        const size_t rc = (size_t)c * t.G + g;
+        n = t.visits[rc];
+        if (n > 0) return __dadd_rn((double)t.reward[rc], __ddiv_rn(t.wsum[rc], (double)n));
+    }
+    return vmix;
+}
+
+__device__ __forceinline__ double gnode_sigma(const GNode &nd, double qh) {
+    return __dmul_rn(nd.cs, __ddiv_rn(__dsub_rn(qh, nd.lo), nd.den));
+}
+
+// Pass 1 over the node's valid actions: M, max N, the mixed value and the range of q^.
+__device__ __forceinline__ GNode gumbel_node(const ge_mcts_tree &t, const ge_gumbel_params &p, int s, int g, int lane) {
+    const size_t row = (size_t)s * t.G + g;
+    GNode nd;
+    nd.mrow = t.mask + row * t.AW;
+    nd.lrow = t.prior + row * t.A;
+    nd.crow = t.child + row * t.A;
+    double sp = 0.0, spq = 0.0, qlo = INFINITY, qhi = -INFINITY;
+    int M = 0, maxn = 0, nvalid = 0;
+    bool unvisited = false;
+    for_valid(nd.mrow, t.A, t.AW, lane, [&](int a) {
+        int n, c;
+        const double Q = edge_q(t, nd.crow, a, g, 0.0, n, c);
+        ++nvalid;
+        if (n > 0) {
+            const double P = fmax(exp((double)nd.lrow[a]), DBL_MIN);
+            sp = __dadd_rn(sp, P);
+            spq = __dadd_rn(spq, __dmul_rn(P, Q));
+            qlo = fmin(qlo, Q);
+            qhi = fmax(qhi, Q);
+            M += n;
+            maxn = max(maxn, n);
+        } else {
+            unvisited = true;
+        }
+    });
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+        sp = __dadd_rn(sp, __shfl_xor_sync(GE_FULL, sp, o));
+        spq = __dadd_rn(spq, __shfl_xor_sync(GE_FULL, spq, o));
+        qlo = fmin(qlo, __shfl_xor_sync(GE_FULL, qlo, o));
+        qhi = fmax(qhi, __shfl_xor_sync(GE_FULL, qhi, o));
+        M += __shfl_xor_sync(GE_FULL, M, o);
+        maxn = max(maxn, __shfl_xor_sync(GE_FULL, maxn, o));
+        nvalid += __shfl_xor_sync(GE_FULL, nvalid, o);
+    }
+    unvisited = __any_sync(GE_FULL, unvisited);
+    const double v = (double)t.value[row];
+    nd.vmix = M ? __ddiv_rn(__dadd_rn(v, __dmul_rn((double)M, __ddiv_rn(spq, sp))), (double)(M + 1)) : v;
+    if (unvisited) { qlo = fmin(qlo, nd.vmix); qhi = fmax(qhi, nd.vmix); }
+    nd.lo = qlo;
+    nd.den = fmax(__dsub_rn(qhi, qlo), 1e-8);
+    nd.cs = __dmul_rn(__dadd_rn(p.maxvisit_init, (double)maxn), p.value_scale);
+    nd.M = M; nd.maxn = maxn; nd.nvalid = nvalid;
+    return nd;
+}
+
+// Pass 2: the softmax normaliser of z = l + sigma over the valid actions, online per lane, merged in the butterfly order.
+__device__ __forceinline__ void gumbel_norm(const ge_mcts_tree &t, const GNode &nd, int g, int lane, double &zm, double &zs) {
+    zm = -INFINITY; zs = 0.0;
+    for_valid(nd.mrow, t.A, t.AW, lane, [&](int a) {
+        int n, c;
+        const double z = __dadd_rn((double)nd.lrow[a], gnode_sigma(nd, edge_q(t, nd.crow, a, g, nd.vmix, n, c)));
+        if (z > zm) { zs = __dadd_rn(__dmul_rn(zs, exp(__dsub_rn(zm, z))), 1.0); zm = z; }
+        else zs = __dadd_rn(zs, exp(__dsub_rn(z, zm)));
+    });
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+        const double zm2 = __shfl_xor_sync(GE_FULL, zm, o), zs2 = __shfl_xor_sync(GE_FULL, zs, o);
+        const double mx = fmax(zm, zm2);
+        zs = __dadd_rn(zs > 0.0 ? __dmul_rn(zs, exp(__dsub_rn(zm, mx))) : 0.0, zs2 > 0.0 ? __dmul_rn(zs2, exp(__dsub_rn(zm2, mx))) : 0.0);
+        zm = mx;
+    }
+}
+
+// The warp's largest score, ties to the lowest action (ba = INT_MAX when no lane has a candidate).
+__device__ __forceinline__ void warp_best(double &best, int &ba, int &bc) {
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+        const double u2 = __shfl_xor_sync(GE_FULL, best, o);
+        const int a2 = __shfl_xor_sync(GE_FULL, ba, o);
+        const int c2 = __shfl_xor_sync(GE_FULL, bc, o);
+        if (u2 > best || (u2 == best && a2 < ba)) { best = u2; ba = a2; bc = c2; }
+    }
+}
+
+// The root's score (g + l) + sigma over its valid actions with N = vstar: the best one (pass 2 at the root, and the readout).
+__device__ __forceinline__ void gumbel_root_best(const ge_mcts_tree &t, const ge_gumbel_params &p, const GNode &nd, int g, int lane,
+                                                 int vstar, int &ba, int &bc) {
+    const float *nrow = p.noise + (size_t)g * t.A;
+    double best = -INFINITY;
+    ba = INT_MAX; bc = -1;
+    for_valid(nd.mrow, t.A, t.AW, lane, [&](int a) {
+        int n, c;
+        const double qh = edge_q(t, nd.crow, a, g, nd.vmix, n, c);
+        if (n != vstar) return;
+        const double u = __dadd_rn(__dadd_rn((double)nrow[a], (double)nd.lrow[a]), gnode_sigma(nd, qh));
+        if (u > best) { best = u; ba = a; bc = c; }   // strictly greater: a lane visits its actions in order
+    });
+    warp_best(best, ba, bc);
+}
+
+__global__ void __launch_bounds__(MCTS_WPB * 32) gumbel_root_kernel(ge_mcts_tree t, ge_gumbel_params p, uint64_t seed, uint32_t step,
+                                                                     int env_id0) {
+    pdl_launch_dependents();   // as the sampler: nothing is touched before pdl_wait()
+    pdl_wait();
+    const int lane = threadIdx.x & 31;
+    const int g = blockIdx.x * MCTS_WPB + (threadIdx.x >> 5);
+    if (g >= t.G) return;
+    const uint64_t key = row_key(seed, (uint32_t)(env_id0 + g), step);
+    float *nrow = p.noise + (size_t)g * t.A;
+    for_valid(t.mask + (size_t)g * t.AW, t.A, t.AW, lane, [&](int a) { nrow[a] = node_gumbel(key, a); });
+}
+
+__global__ void __launch_bounds__(MCTS_WPB * 32) gumbel_select_kernel(ge_mcts_tree t, ge_gumbel_params p, int k) {
+    pdl_launch_dependents();   // as the sampler: nothing is touched before pdl_wait()
+    pdl_wait();
+    const int lane = threadIdx.x & 31;
+    const int g = blockIdx.x * MCTS_WPB + (threadIdx.x >> 5);
+    if (g >= t.G) return;
+    const int G = t.G;
+    int s = 0, depth = 0, load = -1, act = -1;
+    while (!t.terminal[(size_t)s * G + g]) {   // a terminal node is revisited
+        const size_t row = (size_t)s * G + g;
+        const GNode nd = gumbel_node(t, p, s, g, lane);
+        if (nd.nvalid == 0) break;                         // a dead end: revisit s
+        int ba, bc;
+        if (s == 0) {                                      // sequential halving over the considered actions
+            const int vstar = p.table[(size_t)min(p.m, nd.nvalid) * t.S + min(nd.M, t.S - 1)];
+            gumbel_root_best(t, p, nd, g, lane, vstar, ba, bc);
+        } else {                                           // pi'(a) - N(s, a) / (1 + M)
+            double zm, zs;
+            gumbel_norm(t, nd, g, lane, zm, zs);
+            const double vden = (double)(1 + nd.M);
+            double best = -INFINITY;
+            ba = INT_MAX; bc = -1;
+            for_valid(nd.mrow, t.A, t.AW, lane, [&](int a) {
+                int n, c;
+                const double z = __dadd_rn((double)nd.lrow[a], gnode_sigma(nd, edge_q(t, nd.crow, a, g, nd.vmix, n, c)));
+                const double u = __dsub_rn(__ddiv_rn(exp(__dsub_rn(z, zm)), zs), __ddiv_rn((double)n, vden));
+                if (u > best) { best = u; ba = a; bc = c; }
+            });
+            warp_best(best, ba, bc);
+        }
+        if (ba == INT_MAX) break;                          // no considered action: revisit s
+        ++depth;
+        if (bc < 0) { load = (int)row; act = ba; break; }  // an unexpanded edge: expand s by ba
+        s = bc;
+    }
+    if (lane == 0) {
+        t.sel_node[g] = s;
+        t.sel_action[g] = act;
+        t.load_index[g] = load;
+        t.depth[g] = depth;
+    }
+}
+
+__global__ void __launch_bounds__(MCTS_WPB * 32) gumbel_result_kernel(ge_mcts_tree t, ge_gumbel_params p, int32_t *__restrict__ action,
+                                                                       float *__restrict__ policy, double *__restrict__ completed_q) {
+    pdl_launch_dependents();   // as the sampler: nothing is touched before pdl_wait()
+    pdl_wait();
+    const int lane = threadIdx.x & 31;
+    const int g = blockIdx.x * MCTS_WPB + (threadIdx.x >> 5);
+    if (g >= t.G) return;
+    const int A = t.A;
+    const GNode nd = gumbel_node(t, p, 0, g, lane);
+    double zm, zs;
+    gumbel_norm(t, nd, g, lane, zm, zs);
+    int ba, bc;
+    gumbel_root_best(t, p, nd, g, lane, nd.maxn, ba, bc);
+    float *prow = policy + (size_t)g * A;
+    double *qrow = completed_q + (size_t)g * A;
+    for (int a = lane; a < A; a += 32) {
+        float pa = 0.f;
+        double q = NAN;
+        if ((nd.mrow[a >> 5] >> (a & 31)) & 1u) {
+            int n, c;
+            q = edge_q(t, nd.crow, a, g, nd.vmix, n, c);
+            pa = __double2float_rn(__ddiv_rn(exp(__dsub_rn(__dadd_rn((double)nd.lrow[a], gnode_sigma(nd, q)), zm)), zs));
+        }
+        prow[a] = pa;
+        qrow[a] = q;
+    }
+    if (lane == 0) action[g] = (t.terminal[g] || ba == INT_MAX) ? -1 : ba;
+}
+
 int check_tree(const char *fn, const ge_mcts_tree *t, int k, int kmin) {
     if (!t) return ge_set_error(GE_ERR_ARG, "%s: null tree", fn);
     if (t->G < 1 || t->S < 1 || t->A < 1 || t->AW != (t->A + 31) / 32)
@@ -661,6 +884,37 @@ int check_tree(const char *fn, const ge_mcts_tree *t, int k, int kmin) {
     if (!t->parent || !t->action || !t->visits || !t->wsum || !t->reward || !t->value || !t->terminal || !t->child || !t->prior ||
         !t->mask || !t->qmin || !t->qmax || !t->sel_node || !t->sel_action || !t->load_index || !t->depth)
         return ge_set_error(GE_ERR_ARG, "%s: null tree array", fn);
+    return GE_OK;
+}
+
+int check_gumbel(const char *fn, const ge_mcts_tree *t, const ge_gumbel_params *p, int k, int kmin) {
+    const int rc = check_tree(fn, t, k, kmin);
+    if (rc) return rc;
+    if (!(t->flags & GE_MCTS_LOG_PRIOR)) return ge_set_error(GE_ERR_ARG, "%s: the tree lacks GE_MCTS_LOG_PRIOR", fn);
+    if (!p) return ge_set_error(GE_ERR_ARG, "%s: null params", fn);
+    if (p->m < 1) return ge_set_error(GE_ERR_ARG, "%s: m = %d must be >= 1", fn, p->m);
+    if (!isfinite(p->value_scale) || p->value_scale < 0.0)
+        return ge_set_error(GE_ERR_ARG, "%s: value_scale = %g must be finite and >= 0", fn, p->value_scale);
+    if (!isfinite(p->maxvisit_init) || p->maxvisit_init < 0.0)
+        return ge_set_error(GE_ERR_ARG, "%s: maxvisit_init = %g must be finite and >= 0", fn, p->maxvisit_init);
+    if (!p->table || !p->noise) return ge_set_error(GE_ERR_ARG, "%s: null table / noise", fn);
+    return GE_OK;
+}
+
+// A warp-per-instance tree kernel, launched with programmatic stream serialization when the tree's flags have GE_FLAG_PDL.
+template <class... KArgs, class... Args>
+int launch_tree(const char *what, void (*kernel)(KArgs...), const ge_mcts_tree *tree, void *stream, Args... args) {
+    cudaLaunchConfig_t cfg = {};   // ge_launch_step's launch, with the PDL flag of the tree
+    cfg.gridDim = dim3((unsigned)((tree->G + MCTS_WPB - 1) / MCTS_WPB));
+    cfg.blockDim = dim3(MCTS_WPB * 32);
+    cfg.stream = (cudaStream_t)stream;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = at;
+    cfg.numAttrs = (tree->flags & GE_FLAG_PDL) ? 1 : 0;
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, args...);
+    if (e != cudaSuccess) { (void)cudaGetLastError(); return ge_set_error(GE_ERR_CUDA, "%s launch: %s", what, cudaGetErrorString(e)); }
     return GE_OK;
 }
 
@@ -798,18 +1052,9 @@ int ge_mcts_select(const ge_mcts_tree *tree, int k, void *stream) {
     GE_NVTX("ge_mcts_select");
     const int rc = check_tree("ge_mcts_select", tree, k, 1);
     if (rc) return rc;
-    cudaLaunchConfig_t cfg = {};   // ge_launch_step's launch, with the PDL flag of the tree
-    cfg.gridDim = dim3((unsigned)((tree->G + MCTS_WPB - 1) / MCTS_WPB));
-    cfg.blockDim = dim3(MCTS_WPB * 32);
-    cfg.stream = (cudaStream_t)stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = (tree->flags & GE_FLAG_PDL) ? 1 : 0;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, mcts_select_kernel, *tree, k);
-    if (e != cudaSuccess) { (void)cudaGetLastError(); return ge_set_error(GE_ERR_CUDA, "mcts_select_kernel launch: %s", cudaGetErrorString(e)); }
-    return GE_OK;
+    if (tree->flags & GE_MCTS_LOG_PRIOR)
+        return ge_set_error(GE_ERR_ARG, "ge_mcts_select: the tree has GE_MCTS_LOG_PRIOR (log-priors: use ge_gumbel_select)");
+    return launch_tree("mcts_select_kernel", mcts_select_kernel, tree, stream, *tree, k);
 }
 
 int ge_mcts_expand(const ge_mcts_tree *tree, int k, const ge_batch *leaf, const float *reward, const void *logits, int dtype,
@@ -826,11 +1071,38 @@ int ge_mcts_expand(const ge_mcts_tree *tree, int k, const ge_batch *leaf, const 
     if (!leaf->mask_bits || !leaf->done) return ge_set_error(GE_ERR_ARG, "%s: null mask_bits / done in the leaf batch", fn);
     const dim3 grid((unsigned)((tree->G + MCTS_WPB - 1) / MCTS_WPB)), block(MCTS_WPB * 32);
     cudaStream_t st = (cudaStream_t)stream;
+    const bool lp = (tree->flags & GE_MCTS_LOG_PRIOR) != 0;
     const cudaError_t e = dtype == GE_LOGITS_BF16
-        ? ge_launch_step(mcts_expand_kernel<GE_LOGITS_BF16>, grid, block, 0, st, *leaf, *tree, k, reward, logits, value)
-        : ge_launch_step(mcts_expand_kernel<GE_LOGITS_F32>, grid, block, 0, st, *leaf, *tree, k, reward, logits, value);
+        ? (lp ? ge_launch_step(mcts_expand_kernel<GE_LOGITS_BF16, true>, grid, block, 0, st, *leaf, *tree, k, reward, logits, value)
+              : ge_launch_step(mcts_expand_kernel<GE_LOGITS_BF16, false>, grid, block, 0, st, *leaf, *tree, k, reward, logits, value))
+        : (lp ? ge_launch_step(mcts_expand_kernel<GE_LOGITS_F32, true>, grid, block, 0, st, *leaf, *tree, k, reward, logits, value)
+              : ge_launch_step(mcts_expand_kernel<GE_LOGITS_F32, false>, grid, block, 0, st, *leaf, *tree, k, reward, logits, value));
     if (e != cudaSuccess) { (void)cudaGetLastError(); return ge_set_error(GE_ERR_CUDA, "mcts_expand_kernel launch: %s", cudaGetErrorString(e)); }
     return GE_OK;
+}
+
+int ge_gumbel_root(const ge_mcts_tree *tree, const ge_gumbel_params *params, uint64_t seed, uint32_t t, int32_t env_id0, void *stream) {
+    GE_NVTX("ge_gumbel_root");
+    const int rc = check_gumbel("ge_gumbel_root", tree, params, 0, 0);
+    if (rc) return rc;
+    return launch_tree("gumbel_root_kernel", gumbel_root_kernel, tree, stream, *tree, *params, seed, t, (int)env_id0);
+}
+
+int ge_gumbel_select(const ge_mcts_tree *tree, const ge_gumbel_params *params, int k, void *stream) {
+    GE_NVTX("ge_gumbel_select");
+    const int rc = check_gumbel("ge_gumbel_select", tree, params, k, 1);
+    if (rc) return rc;
+    return launch_tree("gumbel_select_kernel", gumbel_select_kernel, tree, stream, *tree, *params, k);
+}
+
+int ge_gumbel_result(const ge_mcts_tree *tree, const ge_gumbel_params *params, int32_t *action, float *policy, double *completed_q,
+                     void *stream) {
+    GE_NVTX("ge_gumbel_result");
+    const char *fn = "ge_gumbel_result";
+    const int rc = check_gumbel(fn, tree, params, 0, 0);
+    if (rc) return rc;
+    if (!action || !policy || !completed_q) return ge_set_error(GE_ERR_ARG, "%s: null action / policy / completed_q", fn);
+    return launch_tree("gumbel_result_kernel", gumbel_result_kernel, tree, stream, *tree, *params, action, policy, completed_q);
 }
 
 }  // extern "C"

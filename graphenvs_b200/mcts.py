@@ -7,6 +7,9 @@ through csrc/ge_state.cu).
     res = mcts.run(policy)        # whole episodes: one search per move, then the most-visited action is stepped
     res.actions, res.ret, res.solution_cost, res.solved, res.found, res.steps, res.root_value
 
+    gm = GumbelMCTS(venv, num_simulations=16, max_considered=16)   # Gumbel MuZero: few simulations, improved-policy targets
+    out = gm.search(policy, t=0)  # + out.policy (softmax(l + sigma(completed Q))), out.completed_q, out.considered
+
 Every instance g of venv is searched in parallel with num_simulations simulations, AlphaZero / MuZero style (the semantics,
 bit for bit, are in include/graphenvs_b200.h).  Node k of every instance is created in simulation k, so the env state
 records are laid out [S + 1, G, R] and a simulation round is: select; load every instance's parent node record into the
@@ -14,6 +17,7 @@ leaf batch (G envs); step it with the selected actions; ask the policy; save the
 and back up.  The leaf batch is stepped only through these forks, so the searched env itself is never touched.
 """
 import ctypes as C
+import math
 from types import SimpleNamespace
 
 import torch
@@ -21,7 +25,8 @@ import torch
 from . import _native
 from .policy import _DTYPES
 
-_PDL = 16   # GE_FLAG_PDL
+_PDL = 16          # GE_FLAG_PDL
+_LOG_PRIOR = 32    # GE_MCTS_LOG_PRIOR
 
 
 def _ptr(t):
@@ -44,6 +49,8 @@ class MCTS:
     one) are allocated here and reused by every search.  `sel_action` and `depth` (int32 [G]) hold the current simulation's
     selection -- the action that led to the leaf and the leaf's depth -- for policies keyed on them (-1 and 0 while the
     roots are evaluated)."""
+
+    _tree_flags = 0
 
     def __init__(self, venv, num_simulations, c_puct=1.25):
         from .batch import BatchedGraphEnv, EnvStates
@@ -146,8 +153,8 @@ class MCTS:
         if not 1 <= k <= self.S:
             raise RuntimeError("MCTS: simulate() needs start() first and runs at most %d simulations" % self.S)
         leaf = self.leaf
-        self.tree.flags = leaf.desc.flags & _PDL
-        _native.check(leaf.lib.ge_mcts_select(C.byref(self.tree), k, leaf._stream()))
+        self.tree.flags = (leaf.desc.flags & _PDL) | self._tree_flags
+        self._select(k)
         leaf.load_states(self.records, self.load_index)
         leaf.step_async(self.sel_action)
         logits, value = self._policy_out(policy(leaf))
@@ -155,6 +162,13 @@ class MCTS:
         _native.check(leaf.lib.ge_mcts_expand(C.byref(self.tree), k, C.byref(leaf.desc), _ptr(leaf.reward), _ptr(logits),
                                               _DTYPES[logits.dtype], _ptr(value), leaf._stream()))
         self.k = k
+
+    def _select(self, k):
+        _native.check(self.leaf.lib.ge_mcts_select(C.byref(self.tree), k, self.leaf._stream()))
+
+    def _move(self, policy, game, t):
+        """The search of move t of run()."""
+        return self.search(policy, game)
 
     def result(self):
         """The roots' statistics after the simulations so far:
@@ -184,7 +198,7 @@ class MCTS:
     def run(self, policy, max_steps=None, from_current=False):
         """Decodes every instance of venv on a copy (a G-env batch, auto-reset off): from reset() or (from_current=True) from
         venv's current state, one search per move, then the most-visited action is stepped, until every episode has ended
-        (checked on the host after every move) or after max_steps moves (default 4 * N).  venv is left untouched.  Returns
+        (checked on the host after every move) or after max_steps moves (default 4 * N); GumbelMCTS steps its Gumbel action.  venv is left untouched.  Returns
           actions        int32 [G, T] the moves, -1 after the episode ended (T = moves made)
           ret            float64 [G] the return (sum of rewards), NaN when the episode did not end
           solution_cost  float64 [G] the final solution_cost (0 when the last step reported none), NaN when it did not end
@@ -214,7 +228,7 @@ class MCTS:
             live = game.t["done"] == 0
             if not bool(live.any()):
                 break
-            out = self.search(policy, game)
+            out = self._move(policy, game, t)
             actions[:, t] = torch.where(live, out.action, -1)
             root_value[:, t] = torch.where(live, out.value, float("nan"))
             game.step_async(out.action)       # a done env gets -1: GE_STEP_AFTER_DONE, state and statistics unchanged
@@ -225,3 +239,106 @@ class MCTS:
         return SimpleNamespace(actions=actions[:, :t].clone(), ret=torch.where(found, acc[2], nan),
                                solution_cost=torch.where(found, acc[3], nan), solved=found & (acc[1] > 0), found=found,
                                steps=t, root_value=root_value[:, :t].clone())
+
+
+def considered_visits_table(m, S):
+    """mctx's get_table_of_considered_visits(m, S): int list [m + 1][S], row n the sequential-halving visit counts of n considered
+    actions over S simulations (include/graphenvs_b200.h, ge_gumbel_params.table)."""
+    rows = []
+    for n in range(m + 1):
+        if n <= 1:
+            rows.append(list(range(S)))
+            continue
+        log2max = int(math.ceil(math.log2(n)))
+        seq, visits, c = [], [0] * n, n
+        while len(seq) < S:
+            for _ in range(max(1, int(S / (log2max * c)))):
+                seq.extend(visits[:c])
+                for i in range(c):
+                    visits[i] += 1
+            c = max(2, c // 2)
+        rows.append(seq[:S])
+    return rows
+
+
+def _finite_nonneg(name, x):
+    if isinstance(x, bool) or not isinstance(x, (int, float)) or not 0.0 <= float(x) < float("inf"):
+        raise ValueError("GumbelMCTS: %s must be a finite number >= 0, got %r" % (name, x))
+    return float(x)
+
+
+class GumbelMCTS(MCTS):
+    """Gumbel MuZero search (Danihelka et al., ICLR 2022; mctx's gumbel_muzero_policy) over every instance of `venv`: at the
+    root, up to `max_considered` actions sampled without replacement by Gumbel-top-k and `num_simulations` split over them by
+    sequential halving; inside the tree, deterministic selection against the improved policy; completed Q scaled by
+    (maxvisit_init + max N) * value_scale.  The root noise is keyed by (seed, global instance id, t, action).
+
+    The tree, records, leaf batch, start / simulate and expansion + backup are MCTS's; the tree keeps log-priors
+    (GE_MCTS_LOG_PRIOR) and selection is ge_gumbel_select (include/graphenvs_b200.h).  `noise` (float32 [G, A]) holds the
+    current search's root noise under the root masks."""
+
+    _tree_flags = _LOG_PRIOR
+
+    def __init__(self, venv, num_simulations, max_considered=16, value_scale=0.1, maxvisit_init=50.0, seed=0):
+        if isinstance(max_considered, bool) or not isinstance(max_considered, int) or max_considered < 1:
+            raise ValueError("GumbelMCTS: max_considered must be an integer >= 1, got %r" % (max_considered,))
+        value_scale = _finite_nonneg("value_scale", value_scale)
+        maxvisit_init = _finite_nonneg("maxvisit_init", maxvisit_init)
+        if isinstance(seed, bool) or not isinstance(seed, int) or not 0 <= seed < 1 << 64:
+            raise ValueError("GumbelMCTS: seed must be an integer in [0, 2^64), got %r" % (seed,))
+        super().__init__(venv, num_simulations)
+        self.max_considered, self.value_scale, self.maxvisit_init, self.seed = max_considered, value_scale, maxvisit_init, seed
+        G, A, dev = self.G, self.A, self.leaf.device
+        self.table = torch.tensor(considered_visits_table(max_considered, self.S), dtype=torch.int32, device=dev)
+        self.noise = torch.zeros((G, A), dtype=torch.float32, device=dev)
+        self._action = torch.full((G,), -1, dtype=torch.int32, device=dev)
+        self._policy = torch.zeros((G, A), dtype=torch.float32, device=dev)
+        self._completed_q = torch.zeros((G, A), dtype=torch.float64, device=dev)
+        p = _native.GumbelParams()
+        p.m, p.value_scale, p.maxvisit_init = max_considered, value_scale, maxvisit_init
+        p.table, p.noise = self.table.data_ptr(), self.noise.data_ptr()
+        self.params = p
+        self.tree.flags = self._tree_flags
+
+    def memory_bytes(self):
+        ts = (self.table, self.noise, self._action, self._policy, self._completed_q)
+        return super().memory_bytes() + sum(x.numel() * x.element_size() for x in ts)
+
+    def start(self, policy, env=None, t=0):
+        """MCTS.start, then the root noise of move t: node_gumbel(row_key(seed, env_id0 + g, t), a) over each root's valid actions."""
+        if isinstance(t, bool) or not isinstance(t, int) or not 0 <= t < 1 << 32:
+            raise ValueError("GumbelMCTS: t must be an integer in [0, 2^32), got %r" % (t,))
+        env = self.venv if env is None else env
+        self.tree.flags = (self.leaf.desc.flags & _PDL) | self._tree_flags
+        super().start(policy, env)
+        _native.check(self.leaf.lib.ge_gumbel_root(C.byref(self.tree), C.byref(self.params), self.seed, t, env.desc.env_id0,
+                                                   self.leaf._stream()))
+
+    def _select(self, k):
+        _native.check(self.leaf.lib.ge_gumbel_select(C.byref(self.tree), C.byref(self.params), k, self.leaf._stream()))
+
+    def _move(self, policy, game, t):
+        return self.search(policy, game, t)
+
+    def result(self):
+        """MCTS.result's visits, q and value, and
+          action       int32 [G]       the Gumbel action: among the most-visited root actions, the largest g + l + sigma; -1 for a
+                                       done root or one without valid actions
+          policy       float32 [G, A]  the improved policy softmax(l + sigma) over the root's valid actions, 0 off the mask
+          completed_q  float64 [G, A]  the completed Q of the root's valid actions, NaN off the mask
+          considered   int32 [G]       m' = min(max_considered, number of valid root actions)"""
+        out = MCTS.result(self)
+        _native.check(self.leaf.lib.ge_gumbel_result(C.byref(self.tree), C.byref(self.params), _ptr(self._action), _ptr(self._policy),
+                                                     _ptr(self._completed_q), self.leaf._stream()))
+        out.action = self._action.clone()
+        out.policy = self._policy.clone()
+        out.completed_q = self._completed_q.clone()
+        out.considered = unpack_mask(self.mask[0], self.A).sum(dim=1).clamp(max=self.max_considered).int()
+        return out
+
+    def search(self, policy, env=None, t=0):
+        """start(policy, env, t), then num_simulations simulate(policy); returns result()."""
+        self.start(policy, env, t)
+        for _ in range(self.S):
+            self.simulate(policy)
+        return self.result()

@@ -36,6 +36,8 @@
  *   ge_beam_expand    one beam-search step: every beam's valid continuations scored and the W best per instance kept (ge_policy.cu)
  *   ge_beam_expand_sampled  one stochastic-beam-search step: W distinct sequences per instance sampled without replacement
  *   ge_mcts_select / ge_mcts_expand  Monte Carlo tree search (PUCT): one simulation round's selection and its expansion + backup
+ *   ge_gumbel_root / ge_gumbel_select / ge_gumbel_result  Gumbel MuZero search over the same tree: root noise, sequential-halving
+ *                     selection and the improved-policy readout
  *   ge_state_save / ge_state_load / ge_gather_instances  branching an env, i.e. copy.deepcopy(env) of a gym env: per-env state
  *                     records and instance replication for search decoders (multi-start, beam search, lookahead; ge_state.cu)
  */
@@ -450,11 +452,15 @@ int ge_beam_expand_sampled(const ge_batch *batch, int W, const void *logits, int
  * with programmatic stream serialization when tree->flags has GE_FLAG_PDL, expand when leaf->flags has it.  No allocation or
  * synchronisation: a whole search can be captured in a CUDA graph.  GE_ERR_ARG, before any CUDA call, for a NULL pointer,
  * G < 1, S < 1, A < 1, AW != ceil(A / 32), a non-finite or negative c_puct, k outside [1, S] (select) / [0, S] (expand), an
- * unknown dtype, leaf->B != G, leaf->A != A, or a NULL leaf->mask_bits / leaf->done.
+ * unknown dtype, leaf->B != G, leaf->A != A, or a NULL leaf->mask_bits / leaf->done; select also for a tree with
+ * GE_MCTS_LOG_PRIOR (its priors are log-priors: the Gumbel search below).
  * Memory per node: R + 8 A + 4 AW + 29 bytes (record, child + prior, mask, the scalars), plus 32 bytes per instance. */
+#define GE_MCTS_LOG_PRIOR 32u   /* ge_mcts_tree.flags: ge_mcts_expand stores the log-prior fl32(l_a - lse) in `prior` instead of its
+                                   expf (the trees of ge_gumbel_select); ge_mcts_select refuses such a tree */
 typedef struct ge_mcts_tree {
     int32_t G, S, A, AW;          /* instances, simulations, mask length and its words */
-    uint32_t flags;               /* GE_FLAG_PDL: ge_mcts_select launches with programmatic stream serialization */
+    uint32_t flags;               /* GE_FLAG_PDL: ge_mcts_select / ge_gumbel_* launch with programmatic stream serialization;
+                                     GE_MCTS_LOG_PRIOR */
     double c_puct;                /* >= 0, finite */
     int32_t *parent;              /* [S + 1, G]     parent node, -1 at the root and in an unused slot */
     int32_t *action;              /* [S + 1, G]     action of the edge into the node, -1 at the root and in an unused slot */
@@ -479,6 +485,62 @@ int ge_mcts_select(const ge_mcts_tree *tree, int k, void *stream);
  * value [G] float32. */
 int ge_mcts_expand(const ge_mcts_tree *tree, int k, const ge_batch *leaf, const float *reward, const void *logits, int dtype,
                    const float *value, void *stream);
+
+/* ---- Gumbel MuZero search (Danihelka, Guez, Schrittwieser, Silver, ICLR 2022; mctx's gumbel_muzero_policy; csrc/ge_policy.cu) ----
+ *
+ * The tree, the records, the simulation round and the expansion + backup are those of the PUCT block above, with
+ * GE_MCTS_LOG_PRIOR set in tree->flags (so `prior` holds l(s, a) = fl32(l_a - lse), the value ge_masked_log_prob gives, bit for
+ * bit) and ge_gumbel_select in place of ge_mcts_select.  A search is
+ *   ge_mcts_expand(tree, 0, ...);  ge_gumbel_root(tree, params, seed, t, env_id0)
+ *   for k = 1 .. S: ge_gumbel_select(tree, params, k), then the fork, step, policy, save and ge_mcts_expand(tree, k, ...) of PUCT
+ *   ge_gumbel_result(tree, params, action, policy, completed_q)
+ * Notation of the PUCT block: node s, its valid actions a (its packed mask), child c(s, a), N(s, a) = N(c) (0 when unexpanded),
+ * Q(s, a) = r(c) + Wsum(c) / N(c) for an expanded child, v(s) the node's value (0 at a terminal node).  All tree arithmetic is
+ * float64 with explicitly rounded operations; exp is the float64 exp.
+ * Sums over the valid actions of a node are taken per lane (lane l of the warp owns the actions a = l mod 32, in ascending
+ * order) and the 32 partial sums combined by the butterfly x_l + x_(l xor o), o = 16, 8, 4, 2, 1 (a fixed order, no atomics).
+ * Completed Q at node s, with M = sum_a N(s, a) and P(a) = max(exp(l(s, a)), DBL_MIN):
+ *   v_mix = (v(s) + M * (sum_{N(a)>0} P(a) * Q(s, a) / sum_{N(a)>0} P(a))) / (M + 1),   v_mix = v(s) when M = 0
+ *   q^(a) = Q(s, a) when N(s, a) > 0, else v_mix
+ *   q~(a) = (q^(a) - lo) / max(hi - lo, 1e-8),  lo / hi = min / max of q^ over the valid actions of s
+ *   sigma(a) = ((maxvisit_init + max_a N(s, a)) * value_scale) * q~(a)
+ * Interior selection (s not the root): z(a) = l(s, a) + sigma(a), pi'(a) = exp(z(a) - zmax) / sum_a exp(z(a) - zmax) (zmax and
+ * the sum taken online per lane: a larger z rescales the lane's sum, and lanes merge as max and rescaled sums); take the valid
+ * action of largest pi'(a) - N(s, a) / (1 + M), ties to the lowest action.
+ * Root selection: m' = min(m, valid actions of the root), j = min(M, S - 1) (j = k - 1 for a live root), v* = table[m'][j];
+ * take the valid action of largest (g(a) + l(root, a)) + sigma(a) among those with N(root, a) = v*, ties to the lowest action
+ * (sequential halving keeps at least one; were there none, the root would be revisited).
+ * Termination is PUCT's: a terminal node or one without valid actions is revisited, an unexpanded edge is expanded, an edge into a
+ * terminal child revisits the child, a terminal root is revisited on every simulation; outputs sel_node, sel_action,
+ * load_index and depth as ge_mcts_select writes them.
+ * Root noise: g(a) = node_gumbel(row_key(seed, env_id0 + g, t), a) in float32, the clamped, finite noise of ge_beam_expand_sampled
+ * with the row key of ge_sample_logits: h = mix32(key, a, 0x85EBCA6B), u = min(fl32((h >> 8) + 0.5) / 2^24, 1 - 2^-24),
+ * g = -logf(-logf(u)), key = (uint64) mix32(seed, i, t) << 32 | mix32(seed ^ 0xD1B54A32D192ED03, i, t), i = env_id0 + g.  It
+ * depends on (seed, global instance i, t, a) only, so a rank slice draws what the full batch draws.
+ * Readout: action = the valid action of largest (g(a) + l(root, a)) + sigma(a) among those with N(root, a) = max_a N(root, a),
+ * ties to the lowest, -1 for a terminal root or one without valid actions; policy [G, A] float32 = fl32 of softmax over the
+ * valid actions of z = l + sigma (the online normaliser above), 0 off the mask; completed_q [G, A] float64 = q^, NaN off the mask.
+ * table is mctx's get_table_of_considered_visits(m, S), int32 [m + 1, S] (row m', column j): row 0 and row 1 are 0, 1, .., S - 1;
+ * row n >= 2 repeats, while shorter than S, a phase over the first c actions (c = n, then max(2, c / 2) each phase): it appends
+ * the visit counts of those c actions, max(1, floor(S / (ceil(log2 n) * c))) times, each time raising each by one.
+ * Every kernel is a warp per instance, launches with programmatic stream serialization when tree->flags has GE_FLAG_PDL and
+ * touches nothing before pdl_wait(); no allocation or synchronisation, so a whole search can be captured in a CUDA graph.
+ * GE_ERR_ARG, before any CUDA call, for everything ge_mcts_select refuses, a tree without GE_MCTS_LOG_PRIOR, a NULL params, table,
+ * noise or output, m < 1, or a non-finite or negative value_scale or maxvisit_init. */
+typedef struct ge_gumbel_params {
+    int32_t m;                    /* maximum number of considered root actions, >= 1 (mctx's max_num_considered_actions) */
+    double value_scale;           /* >= 0, finite (mctx's default 0.1) */
+    double maxvisit_init;         /* >= 0, finite (mctx's default 50) */
+    const int32_t *table;         /* [m + 1, S] considered visit counts */
+    float *noise;                 /* [G, A] root noise g, written by ge_gumbel_root under the root's mask only */
+} ge_gumbel_params;
+/* The root noise of every instance, after ge_mcts_expand(tree, 0, ...) (it reads the root's mask). */
+int ge_gumbel_root(const ge_mcts_tree *tree, const ge_gumbel_params *params, uint64_t seed, uint32_t t, int32_t env_id0, void *stream);
+/* Selection of simulation k (1 <= k <= S), with ge_mcts_select's outputs. */
+int ge_gumbel_select(const ge_mcts_tree *tree, const ge_gumbel_params *params, int k, void *stream);
+/* The readout: action int32 [G], policy float32 [G, A], completed_q float64 [G, A]. */
+int ge_gumbel_result(const ge_mcts_tree *tree, const ge_gumbel_params *params, int32_t *action, float *policy, double *completed_q,
+                     void *stream);
 
 /* ---- Branching: per-env state records and instance replication (csrc/ge_state.cu) ----
  *
