@@ -21,8 +21,8 @@
 //     popcount(row_i & row_j) over the bit-matrix (the first version expanded N x M edges).
 // The first version (one warp per env, N serial sources, CSR expansion with shared fp64 atomics:
 // 190 us/env at TSP N=200 dense, 73 us/env at N=500) is kept as features_warp_kernel for N > 1024.
-// Sums are reassociated relative to networkx (sigma sums are integers < 2^53 => exact; delta and
-// pagerank differ by fp64 rounding, ~1e-16 relative; the tests compare at 1e-5 in float32).
+// Sums are reassociated relative to networkx (sigma sums are exact while path counts stay below 2^53; delta
+// and pagerank differ by fp64 rounding, ~1e-15 relative => within 1 float32 ulp; the other columns are exact).
 #include "ge_common.cuh"
 
 using namespace ge;
